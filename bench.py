@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of the registration hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Headline (BASELINE.json metric "frames/sec FPFH+SAC-IA+ICP @640x480 scene", configs[4] "C5"): batched localisation of 1 024
 independent synthetic 640x480 frames — the model the reference ships (157 825 points) under a random pose at 0.6-1.6 m, table,
@@ -23,6 +23,9 @@ device time.
 
 --impl reference times the CPU oracle on all host cores on the same frames (one frame per core at a time, full iteration
 budget: the same configuration), a bounded sample per step.
+
+--dump-outputs DIR writes what the headline's last timed step returned (see dump_outputs) for comparing two builds: with the same
+arguments every run feeds the same frames and the same libc rand() stream.
 """
 import argparse
 import os
@@ -279,12 +282,14 @@ def run_ours(args):
     # measured 60 % slower than every later one)
     timed(targets, 2)
     # ---- value: clusters resident in HBM ----
-    total_ms, launches, clocks, _ = timed(targets)
+    total_ms, launches, clocks, outputs = timed(targets)
     value = N_FRAMES * args.steps / (total_ms / 1e3)
     # ---- e2e: host buffers in (H2D of every cluster), results out (D2H of every ope_pose_result) ----
     step(clusters)   # untimed: the pinned staging buffers of the host path grow to this batch
     e2e_ms, _, _, last = timed(clusters)
     e2e_value = N_FRAMES * args.steps / (e2e_ms / 1e3)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, mine, outputs, cuda_lib.T, dist)
     h2d = int(sum(len(c) for c in clusters)) * 16 + len(model) * 12
     d2h = len(clusters) * ctypes.sizeof(cuda_lib.T.PoseResult)
     if dist is not None:
@@ -328,6 +333,32 @@ def run_ours(args):
     if dist is not None:
         dist.destroy_process_group()
     return 0
+
+
+def dump_outputs(out_dir, frames, results, T, dist):
+    """the ope_pose_result of every frame as DIR/<field>.npy, row f = frame f of the 1024: the poses as float32 (N, 16) in the
+    ABI's column-major order, every other field as float64 (N,); ranks send their frames to rank 0, which writes"""
+    import ctypes
+    cols = {}
+    for name, ctype in T.PoseResult._fields_:
+        if name == "reserved":
+            continue
+        if issubclass(ctype, ctypes.Array):
+            cols[name] = np.array([list(getattr(r, name)) for r in results], np.float32)
+        else:
+            cols[name] = np.array([getattr(r, name) for r in results], np.float64)
+    order = np.asarray(frames)
+    if dist is not None:
+        parts = [None] * dist.get_world_size()
+        dist.all_gather_object(parts, (order, cols))
+        if dist.get_rank() != 0:
+            return
+        order = np.concatenate([p[0] for p in parts])
+        cols = {k: np.concatenate([p[1][k] for p in parts]) for k in cols}
+    perm = np.argsort(order)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in cols.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v[perm])
 
 
 def sharded_sacia_numbers(ctx, cuda_lib, model, clusters, stream, torch, dist, rank, world, pool=131072):
@@ -639,7 +670,12 @@ def main():
     ap.add_argument("--steps", type=int, default=20)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last timed step as DIR/<name>.npy (--impl ours)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what --impl ours computes")
     if args.impl == "reference":
         return run_reference(args)
     return run_ours(args)

@@ -3,29 +3,24 @@
 oracle/_ref holds the reference's VENDORED registration sources (VP = DetectAndLocalize/include/pcl/registration: the ICP loop,
 Registration::align / getFitnessScore, CorrespondenceEstimation incl. reciprocal and fixed correspondences, the normal-shooting
 loop, the rejector scores, the self-occluded-normal rejector, getAlignStrength, the convergence-criteria wiring), compiled
-UNMODIFIED where they lie under /root/reference against the mock PCL of oracle/refstub (recipe: oracle/Makefile, target `ref`;
-harness: oracle/ref_harness.cpp). The un-vendored PCL pieces ([UPSTREAM]: kd-tree, Umeyama/SVD, point-to-plane solvers,
+UNMODIFIED where they lie in the reference's source tree against the mock PCL of oracle/refstub (recipe: oracle/Makefile, target
+`ref`; harness: oracle/ref_harness.cpp). The un-vendored PCL pieces ([UPSTREAM]: kd-tree, Umeyama/SVD, point-to-plane solvers,
 transformPointCloud, hasConverged) are the oracle's own restatements on both sides and stay unpinned.
 
 Both sides share the exact kd-tree and solvers, so every comparison is BIT-exact: transform, state, iteration count, the
-last correspondence set, the fitness score, the align strength."""
-import os
+last correspondence set, the fitness score, the align strength.
 
+The reference's sources are not part of this repository: where oracle/_ref is not built, the same calls are answered from what
+it returned, recorded in tests/golden/ref_registration.json (arrays as digests, so the comparisons stay bit-exact)."""
 import numpy as np
 import pytest
 
 import ref_py
 
-HAVE_REFERENCE = os.path.isdir("/root/reference/DetectAndLocalize/include/pcl/registration")
-
 
 @pytest.fixture(scope="module")
 def ref(orc):
-    if HAVE_REFERENCE:
-        ref_py.build()          # the build container: compile from the sources where they lie
-    if not ref_py.available():
-        pytest.skip("oracle/_ref is not built and /root/reference is absent")
-    return ref_py
+    return ref_py if ref_py.available() else ref_py.Recorded()
 
 
 @pytest.fixture(scope="module")
@@ -38,7 +33,7 @@ def _same(o, r, oc=None):
     assert (o.converged, o.state, o.iterations, o.n_correspondences) == \
            (r["res"].converged, r["res"].state, r["res"].iterations, r["res"].n_correspondences)
     if oc is not None:
-        assert all(np.array_equal(a, b) for a, b in zip(oc, r["corr"]))
+        assert all(ref_py.same_values(a, b) for a, b in zip(oc, r["corr"]))
 
 
 def test_point_to_point_icp_c2(ref, orc, synth, drill):
@@ -54,7 +49,7 @@ def test_point_to_point_icp_c2(ref, orc, synth, drill):
         _same(o, r, oc)
         assert orc.fitness(src, tgt, T.mat4(o.T)) == r["fitness"]                       # Registration::getFitnessScore
         assert o.n_correspondences / (len(src) + len(tgt)) == r["align_strength"]       # getAlignStrength
-        assert np.array_equal(orc.transform(src, T.mat4(o.T)), r["aligned"])            # `output`
+        assert ref_py.same_values(orc.transform(src, T.mat4(o.T)), r["aligned"])        # `output`
 
 
 def test_icp_with_guess_and_without_correspondences(ref, orc, synth, drill):
@@ -118,7 +113,7 @@ def test_reciprocal_correspondences(ref, orc, synth, drill):
         prm = orc.icp_params(max_correspondence_distance=d, use_reciprocal=1)
         oc = orc.correspondences_fixed(src, tgt, prm)
         rc = ref.correspondences(src, tgt, d, reciprocal=True)
-        assert len(oc[0]) > 100 and all(np.array_equal(a, b) for a, b in zip(oc, rc))
+        assert len(oc[0]) > 100 and all(ref_py.same_values(a, b) for a, b in zip(oc, rc))
         plain = orc.correspondences_fixed(src, tgt, orc.icp_params(max_correspondence_distance=d))
         assert len(oc[0]) < len(plain[0])
     kw = dict(max_iterations=25, max_correspondence_distance=0.05, transformation_epsilon=1e-8, euclidean_fitness_epsilon=1e-8,
@@ -140,7 +135,7 @@ def test_fixed_correspondences(ref, orc, synth, drill):
     prm = orc.icp_params(max_correspondence_distance=0.02)
     oc = orc.correspondences_fixed(src, tgt, prm, fixed)
     rc = ref.correspondences(src, tgt, 0.02, fixed=fixed)
-    assert all(np.array_equal(a, b) for a, b in zip(oc, rc)) and np.array_equal(oc[0][:6], fq) and (oc[2][:6] > 1e3).all()
+    assert all(ref_py.same_values(a, b) for a, b in zip(oc, rc)) and np.array_equal(oc[0][:6], fq) and (oc[2][:6] > 1e3).all()
     kw = dict(max_iterations=20, max_correspondence_distance=0.05, transformation_epsilon=1e-10, euclidean_fitness_epsilon=1e-12)
     o, oc, od = orc.icp(src, tgt, orc.icp_params(**kw), want_corr=True, fixed=fixed)
     r = ref.icp(src, tgt, orc.icp_params(**kw), fixed=fixed)
