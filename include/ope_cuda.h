@@ -112,6 +112,31 @@ int ope_segment_objects_on_plane(ope_ctx* ctx, const ope_cloud* cloud, const ope
                                  float plane2[4], int32_t iters[2], int32_t* n_clusters);
 void ope_segment_params_default(ope_segment_params* p);
 
+/* ---- depth images -> segmented scenes -> poses, many frames per call -------------------------------------------------------------- */
+/* The reference's online loop for every Kinect frame (D&L/src/rosinterface.cpp:212-250): rgbd2Pcl -> getPassThrough ->
+ * getSegmentedObjectsOnPlane -> estimateFinalPose on a cluster, here for a stack of frames at once. */
+typedef struct ope_scene_batch ope_scene_batch;   /* opaque; holds its ope_ctx and must be destroyed before it */
+void ope_scene_params_default(ope_scene_params* p);
+/* depth: frames x rows x cols uint16, host OR device memory. For every frame: ope_depth_to_cloud -> ope_pass_through ->
+ * ope_segment_objects_on_plane (DataGrabber::rgbd2Pcl, D&L/src/datagrabber.cpp:9-62; ProcessingPcd::getPassThrough,
+ * D&L/src/processingpcd.cpp:8-41; ObjectSegmentationPlane::getSegmentedObjectsOnPlane, D&L/src/objectsegmentationplane.cpp:122-282),
+ * each frame's result equal to those calls' bit for bit. The cropped clouds and their labels stay on the device in *out.
+ * info / status: one entry per frame (status may be NULL); a degenerate RANSAC sample fails only its frame (OPE_ERR_UNSUPPORTED).
+ * Returns OPE_OK when every frame succeeded, else the first failing frame's code (*out is then still valid). */
+int ope_scene_batch_create(ope_ctx* ctx, const ope_scene_params* prm, const uint16_t* depth, int frames, int rows, int cols,
+                           ope_scene_batch** out, ope_scene_frame* info, int32_t* status);
+/* host copies of one frame: xyz (n_cropped x 3) and/or labels (n_cropped), either may be NULL; info may be NULL.
+ * labels are exactly ope_segment_objects_on_plane's. */
+int ope_scene_batch_frame(const ope_scene_batch* s, size_t frame, float* xyz, int32_t* labels, ope_scene_frame* info);
+void ope_scene_batch_destroy(ope_scene_batch* s);
+/* ope_pose_batch on the segmented frames. Frame f's target is cluster cluster[f] (NULL: 0 for every frame) = the points of the
+ * cropped cloud labelled with that number, in ascending index order (what pcl::ExtractIndices returns for the cluster's sorted
+ * indices). n_clusters == -1: the whole cropped cloud (the reference hands it on, D&L/src/objectsegmentationplane.cpp:149-152).
+ * A rank >= n_clusters, or a frame whose scene status is an error: an empty target. Results, tables, workers, status: as
+ * ope_pose_batch (tables == NULL draws from libc rand() in frame order, empty targets included). */
+int ope_scene_pose_batch(const ope_scene_batch* s, const ope_pose_params* prm, const float* model_xyz, size_t n_model,
+                         const int32_t* cluster, const ope_rng_table* tables, int workers, ope_pose_result* results, int32_t* status);
+
 /* ---- spatial search: replaces pcl::search::KdTree / KdTreeFLANN (SURVEY A.3) -------------------------- */
 /* nearestKSearch for nq host queries; out_idx/out_d2 are nq*k, padded with -1 / +inf. k <= 32. */
 int ope_knn(ope_ctx* ctx, const ope_cloud* tgt, const void* qry, size_t nq, size_t stride, size_t offset, int k,

@@ -181,6 +181,24 @@ typedef struct ope_segment_params {
 /* per-point labels of ope_segment_objects_on_plane */
 enum { OPE_SEG_OUTSIDE_PRISM = -3, OPE_SEG_PLANE = -2, OPE_SEG_NO_CLUSTER = -1 };
 
+/* Camera, crop and segmentation of ope_scene_batch_create; ope_scene_params_default gives the values below. */
+typedef struct ope_scene_params {
+  float fx, fy, cx, cy, scale, z_max;  /* DataGrabber::rgbd2Pcl: 525, 525, 319.5, 239.5, 1000, 2.0 (D&L/src/datagrabber.cpp:34,146-150) */
+  float limits[6];                     /* ProcessingPcd::getPassThrough x_min, x_max, y_min, y_max, z_min, z_max:
+                                          -0.5, 0.5, -0.5, 0.3, 0.5, 1.6 (ObjectSegmentationPlane::getFiltered, D&L/src/objectsegmentationplane.cpp:17-18) */
+  ope_segment_params seg;              /* ope_segment_params_default */
+} ope_scene_params;
+
+/* One frame of ope_scene_batch_create. */
+typedef struct ope_scene_frame {
+  int32_t n_points;                    /* after depth -> cloud */
+  int32_t n_cropped;                   /* after the pass-through; the length of the frame's labels */
+  float plane1[4], plane2[4];          /* table plane, second plane (zero when n_clusters == -1) */
+  int32_t iterations[2];               /* RANSAC iterations of the two plane fits */
+  int32_t n_clusters;                  /* as ope_segment_objects_on_plane: -1 = a plane fit failed */
+  int32_t reserved;
+} ope_scene_frame;
+
 /* One frame of a batch (ope_pose_batch): the segmented scene cluster either as host points (stride/offset in BYTES as in
  * ope_cloud_upload) or, when points == NULL, as a device-resident cloud that no other call touches during the batch. */
 typedef struct ope_frame_input {

@@ -123,6 +123,16 @@ class SegmentParams(C.Structure):
 SEG_OUTSIDE_PRISM, SEG_PLANE, SEG_NO_CLUSTER = -3, -2, -1
 
 
+class SceneParams(C.Structure):
+    _fields_ = [("fx", C.c_float), ("fy", C.c_float), ("cx", C.c_float), ("cy", C.c_float), ("scale", C.c_float), ("z_max", C.c_float),
+                ("limits", C.c_float * 6), ("seg", SegmentParams)]
+
+
+class SceneFrame(C.Structure):
+    _fields_ = [("n_points", C.c_int32), ("n_cropped", C.c_int32), ("plane1", C.c_float * 4), ("plane2", C.c_float * 4),
+                ("iterations", C.c_int32 * 2), ("n_clusters", C.c_int32), ("reserved", C.c_int32)]
+
+
 class FrameInput(C.Structure):
     _fields_ = [("points", C.c_void_p), ("n", C.c_size_t), ("stride", C.c_size_t), ("offset", C.c_size_t), ("cloud", C.c_void_p)]
 

@@ -31,6 +31,7 @@ EXPORTS = [
     "ope_comm_unique_id", "ope_comm_nccl_version", "ope_comm_create", "ope_comm_destroy", "ope_comm_rank", "ope_comm_world", "ope_sacia_draw",
     "ope_pose_tracker_create", "ope_pose_tracker_destroy", "ope_pose_estimate_final", "ope_pose_estimate_final_device", "ope_pose_batch",
     "ope_pose_stage_ms", "ope_pose_batch_stage_ms", "ope_icp_params_default", "ope_sacia_params_default", "ope_pose_params_default",
+    "ope_scene_params_default", "ope_scene_batch_create", "ope_scene_batch_frame", "ope_scene_batch_destroy", "ope_scene_pose_batch",
 ]
 
 
@@ -312,6 +313,39 @@ class Context:
         self._chk(lib().ope_segment_objects_on_plane(self.h, cloud.h, C.byref(prm), labels.ctypes.data_as(i32p), p1, p2, it, C.byref(k)))
         return labels[:len(cloud)].copy(), k.value, np.array(list(p1), np.float32), np.array(list(p2), np.float32), (it[0], it[1])
 
+    def scene_batch(self, depth, **params):
+        """Depth images -> cropped, segmented scenes, many frames per call (ope_scene_batch_create). depth: (frames, rows, cols)
+        uint16 on the host (numpy) or a CUDA tensor of uint16 / int16 bits. params: fx, fy, cx, cy, scale, z_max, limits (x_min,
+        x_max, y_min, y_max, z_min, z_max) and any ope_segment_params field. Returns a SceneBatch."""
+        prm = T.SceneParams()
+        lib().ope_scene_params_default(C.byref(prm))
+        for k, v in params.items():
+            if k == "limits":
+                prm.limits = (C.c_float * 6)(*[float(x) for x in v])
+            elif hasattr(prm, k) and k != "seg":
+                setattr(prm, k, v)
+            else:
+                setattr(prm.seg, k, v)
+        if hasattr(depth, "data_ptr"):
+            import torch
+            assert depth.is_cuda and depth.is_contiguous() and depth.element_size() == 2 and depth.dim() == 3
+            torch.cuda.synchronize(depth.device)
+            keep, ptr, shape = depth, C.c_void_p(depth.data_ptr()), tuple(depth.shape)
+        else:
+            keep = np.ascontiguousarray(depth, np.uint16)
+            assert keep.ndim == 3
+            ptr, shape = keep.ctypes.data_as(C.c_void_p), keep.shape
+        n = shape[0]
+        info = (T.SceneFrame * max(n, 1))()
+        status = (C.c_int32 * max(n, 1))()
+        h = C.c_void_p()
+        rc = lib().ope_scene_batch_create(self.h, C.byref(prm), ptr, int(n), int(shape[1]), int(shape[2]), C.byref(h), info, status)
+        del keep
+        st = np.array(list(status)[:n], np.int32)
+        if not h.value:
+            self._chk(rc)
+        return SceneBatch(self, h, [info[i] for i in range(n)], st)
+
     # ---- search ----
     def knn(self, tgt, qry, k):
         """tgt: Cloud; qry: Cloud or (N,>=3) array."""
@@ -476,6 +510,52 @@ class Context:
                                         None if table is None else C.byref(table), C.byref(res),
                                         None if errs is None else errs.ctypes.data_as(f32p)))
         return (res, errs) if want_errors else res
+
+
+class SceneBatch:
+    """ope_scene_batch: the cropped clouds and labels of a stack of depth images, resident on the device. .info: one SceneFrame
+    per frame; .status: per-frame return codes (OPE_ERR_UNSUPPORTED where a RANSAC sample was degenerate)."""
+
+    def __init__(self, ctx, handle, info, status):
+        self.ctx, self.h, self.info, self.status = ctx, handle, info, status
+
+    def __len__(self):
+        return len(self.info)
+
+    def frame(self, f):
+        """(xyz (n_cropped, 3) float32, labels (n_cropped,) int32) of frame f, as ope_pass_through + ope_segment_objects_on_plane"""
+        n = self.info[f].n_cropped
+        xyz = np.empty((max(n, 1), 3), np.float32)
+        labels = np.empty(max(n, 1), np.int32)
+        self.ctx._chk(lib().ope_scene_batch_frame(self.h, C.c_size_t(f), xyz.ctypes.data_as(f32p), labels.ctypes.data_as(i32p), None))
+        return xyz[:n].copy(), labels[:n].copy()
+
+    def pose(self, model, cluster=None, tables=None, workers=8, prm=None):
+        """ope_scene_pose_batch: frame f localised on cluster rank cluster[f] (None: 0 everywhere). Returns (PoseResults, status)."""
+        m = np.ascontiguousarray(model[:, :3], np.float32)
+        n = len(self.info)
+        cl = None if cluster is None else np.ascontiguousarray(cluster, np.int32)
+        assert cl is None or len(cl) == n
+        res = (T.PoseResult * max(n, 1))()
+        status = (C.c_int32 * max(n, 1))()
+        tb = None if tables is None else (T.RngTable * n)(*tables)
+        rc = lib().ope_scene_pose_batch(self.h, None if prm is None else C.byref(prm), m.ctypes.data_as(f32p), C.c_size_t(len(m)),
+                                        None if cl is None else cl.ctypes.data_as(i32p), tb, int(workers), res, status)
+        st = np.array(list(status)[:n], np.int32)
+        self.ctx._chk(rc)
+        return [res[i] for i in range(n)], st
+
+    def close(self):
+        # the handle holds device memory of its context: destroyed before the context is
+        if self.h and self.ctx.h:
+            lib().ope_scene_batch_destroy(self.h)
+        self.h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
 
 
 def comm_unique_id():
