@@ -198,9 +198,12 @@ int ope_correspondences(ope_ctx* ctx, const ope_cloud* src, const ope_cloud* tgt
 int ope_icp_align(ope_ctx* ctx, const ope_cloud* src, const ope_cloud* tgt, const ope_icp_params* prm,
                   const float guess[16], ope_reg_result* res, ope_correspondence* out_corr, ope_cloud** out_aligned);
 /* The same with the reference's own extension of ICP, fixed correspondences (IterativeClosestPoint::setFixedCorrespondences,
- * VP/icp_mod.h:267-281; VP/impl/icp_mod.hpp:150-151,209-225; VP/impl/correspondence_estimation_mod.hpp:134-161): pairs the caller
- * pins enter every iteration's list in front with distance = squared distance * 1e10 and, when rejectors exist, a second time at
- * the end after rejector 0 alone. `fixed` is in/out (the loop rewrites its distances); out_corr must hold ns + 2 * n_fixed entries.
+ * VP/icp_mod.h:267-281; VP/impl/icp_mod.hpp:150-151,209-225; VP/impl/correspondence_estimation_mod.hpp:134-161): with the
+ * nearest-neighbour estimator, pairs the caller pins enter every iteration's list in front with distance = squared distance * 1e10
+ * (written back into `fixed`). Whatever the estimator, when rejectors exist they enter a second time at the end after rejector 0
+ * alone, with the distances `fixed` holds. The reciprocal and the normal-shooting estimators omit the front entries but keep that
+ * tail, with the caller's distances unchanged. The MODCORR variant ignores the list. `fixed` is in/out; out_corr must hold
+ * ns + 2 * n_fixed entries. A pair whose source or target point is not finite is refused (OPE_ERR_INVALID).
  * prm->use_reciprocal (either entry point) selects determineReciprocalCorrespondences (VP/impl/correspondence_estimation_mod.hpp:
  * 216-303) for the nearest-neighbour estimator. */
 int ope_icp_align_fixed(ope_ctx* ctx, const ope_cloud* src, const ope_cloud* tgt, const ope_icp_params* prm, const float guess[16],

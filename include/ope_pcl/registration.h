@@ -444,7 +444,8 @@ class IterativeClosestPoint : public Registration<PointSource, PointTarget, Scal
   }
   void setUseReciprocalCorrespondences(bool use) { use_reciprocal_correspondence_ = use; }
   bool getUseReciprocalCorrespondences() const { return use_reciprocal_correspondence_; }
-  // the vendored class's fixed correspondences, VP/icp_mod.h:267-281: the caller keeps ownership, align() rewrites the distances
+  // the vendored class's fixed correspondences, VP/icp_mod.h:267-281: the caller keeps ownership; align() rewrites the distances
+  // when the nearest-neighbour estimator puts the pairs in front (see ope_icp_align_fixed)
   void setFixedCorrespondences(Correspondences* correspondences) { corres_fixed_ = correspondences; }
   Correspondences& getFixedCorrespondences() { return *corres_fixed_; }
   void clearCorrespondences() { if (corres_fixed_) corres_fixed_->clear(); }

@@ -1359,6 +1359,15 @@ __global__ void fixed_pairs_kernel(IcpDev a, const int* __restrict__ fq, const i
   }
 }
 
+// the first fixed pair (index into the list) whose source or target point is not finite, via atomicMin on *first_bad
+__global__ void fixed_finite_kernel(const float4* __restrict__ src, const float4* __restrict__ tgt, const int* __restrict__ fq,
+                                    const int* __restrict__ fm, int n_fixed, int* __restrict__ first_bad) {
+  for (int j = threadIdx.x; j < n_fixed; j += blockDim.x) {
+    const float4 s = __ldg(src + fq[j]), t = __ldg(tgt + fm[j]);
+    if (!finite3(s.x, s.y, s.z) || !finite3(t.x, t.y, t.z)) atomicMin(first_bad, j);
+  }
+}
+
 // raw Umeyama moments (+ pair count and the sum of the correspondence distances) of the pairs (src[is[i]], tgt[it[i]]), it[i] >= 0
 static constexpr int kPairAcc = kMomentAcc + 1;
 __global__ void pairs_moments_kernel(const float4* __restrict__ src, const float4* __restrict__ tgt, const int* __restrict__ is,
@@ -2214,9 +2223,10 @@ static int icp_stepwise_device(ope_ctx* ctx, const ope_cloud* src, const ope_clo
   OPE_TRY(icp_fill(ctx, src, tgt, prm, &a));
   const size_t n = src->n;
   const bool shooting = prm.estimator == OPE_EST_NORMAL_SHOOTING;
-  // icp_modCorr.h has no setFixedCorrespondences; normal shooting leaves the list out of its result (VP/impl/correspondence_
-  // estimation_normal_shooting_weighted.hpp:81-100)
-  if (prm.variant != OPE_ICP_VARIANT_MOD || shooting) n_fixed = 0;
+  // icp_modCorr.h has no setFixedCorrespondences. Normal shooting never puts the fixed pairs in front of its result (VP/impl/
+  // correspondence_estimation_normal_shooting_weighted.hpp:81-100), but the loop still appends them after rejector 0 with the
+  // caller's distances (VP/impl/icp_mod.hpp:209-225), as for the reciprocal estimator; without rejectors nothing is appended.
+  if (prm.variant != OPE_ICP_VARIANT_MOD || (shooting && prm.n_rejectors == 0)) n_fixed = 0;
   const size_t F = n_fixed;
   for (size_t j = 0; j < F; ++j)
     if (fixed[j].index_query < 0 || (size_t)fixed[j].index_query >= n || fixed[j].index_match < 0 || (size_t)fixed[j].index_match >= tgt->n)
@@ -2244,7 +2254,16 @@ static int icp_stepwise_device(ope_ctx* ctx, const ope_cloud* src, const ope_clo
     OPE_CUDA_TRY(ctx, cudaMemcpyAsync(fq.p, h_fq.data(), F * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
     OPE_CUDA_TRY(ctx, cudaMemcpyAsync(fm.p, h_fm.data(), F * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
     OPE_CUDA_TRY(ctx, cudaMemcpyAsync(d2.p, h_fd.data(), 2 * F * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
-    OPE_CUDA_TRY(ctx, ope::stream_sync(ctx));
+    // a pair naming a NaN / inf point has no defined result (its 1e10-scaled distance and the moments turn NaN): refused
+    Scratch<int> bad(ctx);
+    OPE_TRY(bad.alloc(1));
+    OPE_CUDA_TRY(ctx, cudaMemsetAsync(bad.p, 0x7f, sizeof(int), ctx->stream));
+    fixed_finite_kernel<<<1, 128, 0, ctx->stream>>>(src->pts, tgt->pts, fq.p, fm.p, (int)F, bad.p);
+    OPE_TRY(check_launch(ctx, "fixed_finite_kernel"));
+    void* h;
+    OPE_TRY(read_back(ctx, bad.p, sizeof(int), &h));
+    const int first_bad = *(const int*)h;
+    if ((size_t)first_bad < F) return fail(ctx, OPE_ERR_INVALID, "fixed correspondence %d names a non-finite point", first_bad);
   }
   a.corr_match = match.p + 2 * F; a.corr_d2 = d2.p + 2 * F; a.seed = seed.p;
   OPE_TRY(dyn_smem(ctx, (const void*)correspond_once_kernel, sizeof(IcpSmem)));
@@ -2279,7 +2298,8 @@ static int icp_stepwise_device(ope_ctx* ctx, const ope_cloud* src, const ope_clo
       OPE_TRY(check_launch(ctx, "reciprocal_filter_kernel"));
     }
     if (F) {
-      fixed_pairs_kernel<<<1, 128, 0, ctx->stream>>>(a, fq.p, fm.p, (int)F, prm.use_reciprocal ? 0 : 1, is.p, match.p, d2.p);
+      // front = 0 (reciprocal, shooting): slots [0, F) stay -1, the tail keeps the caller's distances
+      fixed_pairs_kernel<<<1, 128, 0, ctx->stream>>>(a, fq.p, fm.p, (int)F, (prm.use_reciprocal || shooting) ? 0 : 1, is.p, match.p, d2.p);
       OPE_TRY(check_launch(ctx, "fixed_pairs_kernel"));
     }
     Mat4 T = mat4_identity();

@@ -238,7 +238,10 @@ void estimateCorrespondences(const CloudView& src, const CloudView& tgt, const K
       out.push_back(fixed[f]);
     }
     for (size_t i = 0; i < src.n; ++i) {
-      if (tgt_tree.knn(src.p(i), 1, &nn) == 0) continue;  // (non-finite query in FLANN would assert; skipped)
+      // a non-finite query is skipped (FLANN would assert); the tree's answer to a NaN query has d2 = NaN, which the
+      // `d2 > max` gate below would let through
+      if (!orc::finite3(src.p(i))) continue;
+      if (tgt_tree.knn(src.p(i), 1, &nn) == 0) continue;
       if (nn.d2 > max_dist_sqr) continue;
       out.push_back(ope_correspondence{(int32_t)i, nn.idx, nn.d2});
     }
