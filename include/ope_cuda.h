@@ -39,8 +39,8 @@ int ope_ctx_synchronize(ope_ctx* ctx);
 /* number of kernels this context has launched so far (bench.py's gpu_launches) */
 int64_t ope_ctx_launch_count(const ope_ctx* ctx);
 /* device time (ms, CUDA events on the context's stream) of the last launch of the named dominant kernel:
- * which = 0: icp_kernel (the fused ICP loop), 1: sacia_kernel (hypothesis pool), 2: featgemm_kernel (tcgen05 feature-distance
- * GEMM). Negative if it never ran. */
+ * which = 0: icp_kernel (the fused ICP loop), 1: the SAC-IA scorer (sacia_score_batch_kernel or sacia_kernel), 2: featgemm_kernel
+ * (tcgen05 feature-distance GEMM). Negative if it never ran. */
 double ope_ctx_last_kernel_ms(ope_ctx* ctx, int which);
 /* feature-space k-NN bookkeeping: queries answered through the tcgen05 distance GEMM so far, and how many of them the exact
  * float32 kernel re-answered because the candidate set could not be proven complete */

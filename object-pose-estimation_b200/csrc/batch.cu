@@ -7,16 +7,17 @@
 //   target UniformSampling 1 cm + 8 mm     bsample_kernel<false>      grid (frames, 2)        cluster -> tp1, tp2 (voxel-key order)
 //   normals k = 30 of tp1, tp2             normals_smem_batch_kernel  grid (<=8, 2 frames)
 //   SPFH + FPFH of tp1                     spfh_/fpfh_batch_kernel    grid (n/8, frames)
-//   5 nearest target features per model    feature_knn_batch_kernel (+ merge)                 the model's descriptors are shared
-//   SAC-IA 400 x 5                         sacia_smem_batch_kernel    grid (400, frames)      + select: coarse pose per frame
+//   5 nearest target features per model    feature_knn_kernel (+ merge) grid (nq/128, <=4, frames)   the model's descriptors are shared
+//   SAC-IA 400 x 5                         sacia_transform_/seed_/score_batch_kernel         + select: coarse pose per frame
+//                                                                     score grid (frames, 400/16)
 //   model under the coarse pose, 8 mm      bsample_kernel<true>       grid (frames)           157 825 points, never materialised
 //   normals k = 30 of sp2                  normals_smem_batch_kernel
 //   removeNaNNormalsFromPointCloud x 2     compact_normals_batch_kernel
 //   ICP-with-normals <= 100 iterations     icp_small_batch_kernel     ticketed blocks of all frames
 //   getFitnessScore                        fitness_smem_batch_kernel  grid (frames)
 //
-// The kernels are the single-frame kernels' bodies (features.cu, registration.cu) behind a frame index, so a frame's result is
-// what ope_pose_estimate_final returns for it — bit for bit, tests/test_gpu_parity.py. Frames outside the fast path's envelope
+// The kernels are the single-frame kernels, or their bodies (features.cu, registration.cu), behind a frame index, so a frame's
+// result is what ope_pose_estimate_final returns for it — bit for bit, tests/test_gpu_parity.py. Frames outside the fast path's envelope
 // (empty or tiny clusters, clouds beyond the shared-memory capacities, voxel tables that overflow) are finished by the per-frame
 // path in pipeline.cu. The frame-invariant model side (1 cm sample, normals, FPFH; dense Umeyama of the model onto itself) is
 // computed once per call (SURVEY 8f-3).
@@ -507,6 +508,7 @@ int pose_batch_chunk(ope_ctx* ctx, const ope_pose_params& P, const ope_cloud* d_
   std::memset(&sb, 0, sizeof(sb));
   sb.src = sp->pts; sb.ns = ns; sb.tgt = sampled.p; sb.counts = d_counts.p; sb.stride = kBCap;
   sb.nr_samples = S; sb.k_corr = K; sb.H = H; sb.samples = d_samples.p; sb.picks = d_picks.p; sb.knn_idx = d_knn.p; sb.active = d_active.p;
+  sb.h_begin = 0; sb.h_end = H; sb.early_exit = 1;
   sb.threshold = (float)P.sacia.max_correspondence_distance; sb.errors = errors.p; sb.transforms = transforms.p;
   {
     const char* me = std::getenv("OPE_BATCH_MORTON");
@@ -516,16 +518,7 @@ int pose_batch_chunk(ope_ctx* ctx, const ope_pose_params& P, const ope_cloud* d_
       sb.tgt_scan = compacted.p;
     }
   }
-  Scratch<unsigned> d_best(ctx);
-  OPE_TRY(d_best.alloc(B));
-  {
-    std::vector<unsigned> inf((size_t)B, 0x7f800000u);
-    OPE_CUDA_TRY(ctx, cudaMemcpyAsync(d_best.p, inf.data(), (size_t)B * sizeof(unsigned), cudaMemcpyHostToDevice, ctx->stream));
-    OPE_CUDA_TRY(ctx, stream_sync(ctx));
-  }
-  sb.best_bits = d_best.p;
-  { const char* e = std::getenv("OPE_SACIA_EARLY_EXIT"); sb.early_exit = !(e && std::atoi(e) == 0); }
-  OPE_TRY(sacia_batch_device(ctx, sb, B, max_tp1, d_coarse.p));
+  OPE_TRY(sacia_batch_device(ctx, sb, B, max_tp1, nullptr, d_coarse.p));
   tm.mark();   // [5] SAC-IA
   // ---- estimateFinePose (:161-379): the model under the coarse pose sampled at the fine leaf, never materialised ----
   std::memset(&sa, 0, sizeof(sa));

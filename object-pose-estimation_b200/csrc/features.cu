@@ -304,59 +304,22 @@ static constexpr int kFkTile = 64;       // targets per shared-memory tile
 static constexpr int kFkMaxDim = 64;
 static constexpr int kFkMaxK = 16;
 
-__global__ void feature_knn_kernel(const float* __restrict__ ftgt, int nt, const float* __restrict__ fqry, int nq, int dim,
-                                   int k, int t_per_split, const int* __restrict__ qlist, int* __restrict__ part_idx,
-                                   float* __restrict__ part_d2) {
+// blockIdx.z = frame: targets ftgt + z * stride * dim, counts[z] rows (counts null: nt rows); every frame answers the same nq
+// queries (the rows qlist lists, null: 0 .. nq-1). Partial lists at ((z * nq + qi) * splits + y) * k; splits past a frame's end
+// produce empty lists.
+__global__ void feature_knn_kernel(const float* __restrict__ ftgt, int nt, const int* __restrict__ counts, int stride,
+                                   const float* __restrict__ fqry, int nq, int dim, int k, int t_per_split, const int* __restrict__ qlist,
+                                   int* __restrict__ part_idx, float* __restrict__ part_d2) {
   extern __shared__ float tile[];  // kFkTile * dim
+  const int frame = blockIdx.z;
+  if (counts) nt = counts[frame];
+  const float* ft = ftgt + (size_t)frame * stride * dim;
   const int qi = blockIdx.x * kFkQueries + threadIdx.x;   // position in the work list (nq entries)
   const int qsrc = (qi < nq && qlist) ? qlist[qi] : qi;    // row of fqry
   const int t_begin = blockIdx.y * t_per_split, t_end = min(nt, t_begin + t_per_split);
   float q[kFkMaxDim];
   if (qi < nq)
     for (int c = 0; c < dim; ++c) q[c] = __ldg(fqry + (size_t)qsrc * dim + c);
-  float bd[kFkMaxK];
-  int bi[kFkMaxK];
-  int cnt = 0;
-  for (int t0 = t_begin; t0 < t_end; t0 += kFkTile) {
-    const int tn = min(kFkTile, t_end - t0);
-    __syncthreads();
-    for (int e = threadIdx.x; e < tn * dim; e += blockDim.x) tile[e] = __ldg(ftgt + (size_t)t0 * dim + e);
-    __syncthreads();
-    if (qi < nq) {
-      for (int t = 0; t < tn; ++t) {
-        const float* f = tile + t * dim;
-        float d = 0.0f;
-        for (int c = 0; c < dim; ++c) { float df = q[c] - f[c]; d += df * df; }
-        if (!isfinite(d)) continue;
-        const int idx = t0 + t;
-        if (cnt == k && !nb_less(d, idx, bd[k - 1], bi[k - 1])) continue;
-        int j = cnt < k ? cnt : k - 1;
-        while (j > 0 && nb_less(d, idx, bd[j - 1], bi[j - 1])) { bd[j] = bd[j - 1]; bi[j] = bi[j - 1]; --j; }
-        bd[j] = d; bi[j] = idx;
-        if (cnt < k) ++cnt;
-      }
-    }
-  }
-  if (qi < nq) {
-    const size_t o = ((size_t)qi * gridDim.y + blockIdx.y) * k;
-    for (int j = 0; j < k; ++j) { part_idx[o + j] = j < cnt ? bi[j] : -1; part_d2[o + j] = j < cnt ? bd[j] : INFINITY; }
-  }
-}
-// frame-spanning launch: blockIdx.z = frame; targets ftgt + z * stride * dim (nt = counts[z]), the SAME nq queries for every frame
-// (the model's descriptors); partial lists at ((z * nq + qi) * splits + y) * k. t_per_split is fixed for the launch; splits past
-// a frame's end produce empty lists.
-__global__ void feature_knn_batch_kernel(const float* __restrict__ ftgt, const int* __restrict__ counts, int stride,
-                                         const float* __restrict__ fqry, int nq, int dim, int k, int t_per_split, int* __restrict__ part_idx,
-                                         float* __restrict__ part_d2) {
-  extern __shared__ float tile[];  // kFkTile * dim
-  const int frame = blockIdx.z;
-  const int nt = counts[frame];
-  const float* ft = ftgt + (size_t)frame * stride * dim;
-  const int qi = blockIdx.x * kFkQueries + threadIdx.x;
-  const int t_begin = blockIdx.y * t_per_split, t_end = min(nt, t_begin + t_per_split);
-  float q[kFkMaxDim];
-  if (qi < nq)
-    for (int c = 0; c < dim; ++c) q[c] = __ldg(fqry + (size_t)qi * dim + c);
   float bd[kFkMaxK];
   int bi[kFkMaxK];
   int cnt = 0;
@@ -385,12 +348,15 @@ __global__ void feature_knn_batch_kernel(const float* __restrict__ ftgt, const i
     for (int j = 0; j < k; ++j) { part_idx[o + j] = j < cnt ? bi[j] : -1; part_d2[o + j] = j < cnt ? bd[j] : INFINITY; }
   }
 }
-// merge of the batched partial lists: one thread per (frame, query); out_idx at (frame * nq + qi) * k
-__global__ void feature_knn_batch_merge_kernel(const int* __restrict__ part_idx, const float* __restrict__ part_d2, int nq, int splits, int k,
-                                               int* __restrict__ out_idx) {
+// one thread per (frame = blockIdx.y, query): the splits' lists merged into out_idx / out_d2 (optional) at row
+// frame * nq + qlist[qi] (qlist null: qi)
+__global__ void feature_knn_merge_kernel(const int* __restrict__ part_idx, const float* __restrict__ part_d2, int nq,
+                                         int splits, int k, const int* __restrict__ qlist, int* __restrict__ out_idx,
+                                         float* __restrict__ out_d2) {
   const int qi = blockIdx.x * blockDim.x + threadIdx.x;
   if (qi >= nq) return;
   const size_t row = (size_t)blockIdx.y * nq + qi;
+  const size_t dst = (size_t)blockIdx.y * nq + (qlist ? qlist[qi] : qi);
   float bd[kFkMaxK];
   int bi[kFkMaxK];
   int cnt = 0;
@@ -406,32 +372,9 @@ __global__ void feature_knn_batch_merge_kernel(const int* __restrict__ part_idx,
       bd[j] = d; bi[j] = idx;
       if (cnt < k) ++cnt;
     }
-  for (int j = 0; j < k; ++j) out_idx[row * k + j] = j < cnt ? bi[j] : -1;
-}
-__global__ void feature_knn_merge_kernel(const int* __restrict__ part_idx, const float* __restrict__ part_d2, int nq,
-                                         int splits, int k, const int* __restrict__ qlist, int* __restrict__ out_idx,
-                                         float* __restrict__ out_d2) {
-  const int qi = blockIdx.x * blockDim.x + threadIdx.x;
-  if (qi >= nq) return;
-  const int qdst = qlist ? qlist[qi] : qi;
-  float bd[kFkMaxK];
-  int bi[kFkMaxK];
-  int cnt = 0;
-  for (int s = 0; s < splits; ++s)
-    for (int e = 0; e < k; ++e) {
-      const size_t o = ((size_t)qi * splits + s) * k + e;
-      const int idx = part_idx[o];
-      if (idx < 0) break;
-      const float d = part_d2[o];
-      if (cnt == k && !nb_less(d, idx, bd[k - 1], bi[k - 1])) continue;
-      int j = cnt < k ? cnt : k - 1;
-      while (j > 0 && nb_less(d, idx, bd[j - 1], bi[j - 1])) { bd[j] = bd[j - 1]; bi[j] = bi[j - 1]; --j; }
-      bd[j] = d; bi[j] = idx;
-      if (cnt < k) ++cnt;
-    }
   for (int j = 0; j < k; ++j) {
-    out_idx[(size_t)qdst * k + j] = j < cnt ? bi[j] : -1;
-    if (out_d2) out_d2[(size_t)qdst * k + j] = j < cnt ? bd[j] : INFINITY;
+    out_idx[dst * k + j] = j < cnt ? bi[j] : -1;
+    if (out_d2) out_d2[dst * k + j] = j < cnt ? bd[j] : INFINITY;
   }
 }
 
@@ -532,8 +475,8 @@ int feature_knn_exact_device(ope_ctx* ctx, const float* d_ftgt, size_t nt, const
   OPE_TRY(pi.alloc(nq * splits * k));
   OPE_TRY(pd.alloc(nq * splits * k));
   dim3 grid(qblocks, splits);
-  feature_knn_kernel<<<grid, kFkQueries, kFkTile * dim * sizeof(float), ctx->stream>>>(d_ftgt, (int)nt, d_fqry, (int)nq, dim,
-                                                                                        k, t_per_split, d_qlist, pi.p, pd.p);
+  feature_knn_kernel<<<grid, kFkQueries, kFkTile * dim * sizeof(float), ctx->stream>>>(d_ftgt, (int)nt, nullptr, 0, d_fqry, (int)nq,
+                                                                                        dim, k, t_per_split, d_qlist, pi.p, pd.p);
   OPE_TRY(check_launch(ctx, "feature_knn_kernel"));
   feature_knn_merge_kernel<<<div_up(nq, 128), 128, 0, ctx->stream>>>(pi.p, pd.p, (int)nq, splits, k, d_qlist, d_idx, d_d2);
   return check_launch(ctx, "feature_knn_merge_kernel");
@@ -591,11 +534,12 @@ int feature_knn_batch(ope_ctx* ctx, const float* ftgt, const int* d_counts, int 
   Scratch<float> pd(ctx);
   OPE_TRY(pi.alloc((size_t)frames * nq * splits * k));
   OPE_TRY(pd.alloc((size_t)frames * nq * splits * k));
-  feature_knn_batch_kernel<<<dim3(qblocks, splits, frames), kFkQueries, kFkTile * dim * sizeof(float), ctx->stream>>>(
-      ftgt, d_counts, stride, fqry, nq, dim, k, t_per_split, pi.p, pd.p);
-  OPE_TRY(check_launch(ctx, "feature_knn_batch_kernel"));
-  feature_knn_batch_merge_kernel<<<dim3(div_up((size_t)nq, 128), frames), 128, 0, ctx->stream>>>(pi.p, pd.p, nq, splits, k, out_idx);
-  return check_launch(ctx, "feature_knn_batch_merge_kernel");
+  feature_knn_kernel<<<dim3(qblocks, splits, frames), kFkQueries, kFkTile * dim * sizeof(float), ctx->stream>>>(
+      ftgt, 0, d_counts, stride, fqry, nq, dim, k, t_per_split, nullptr, pi.p, pd.p);
+  OPE_TRY(check_launch(ctx, "feature_knn_kernel"));
+  feature_knn_merge_kernel<<<dim3(div_up((size_t)nq, 128), frames), 128, 0, ctx->stream>>>(pi.p, pd.p, nq, splits, k, nullptr, out_idx,
+                                                                                          nullptr);
+  return check_launch(ctx, "feature_knn_merge_kernel");
 }
 
 int remove_nan_normals_device(ope_ctx* ctx, ope_cloud** cloud) {

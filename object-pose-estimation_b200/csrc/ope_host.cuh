@@ -278,14 +278,16 @@ struct SaciaBatch {
   const float4* tgt; const int* counts; int stride;        // frame f: tgt + f * stride, counts[f] points
   const float4* tgt_scan;                                  // the same points in any order (null: tgt): what the distance scan reads
   int nr_samples, k_corr, H;
+  int h_begin, h_end;                                      // the hypotheses scored: [h_begin, h_end) of 0 .. H-1
   const int* samples; const int* picks;                    // frame f: + f * H * nr_samples
   const int* knn_idx;                                      // frame f: + f * ns * k_corr
   const int* active;                                       // per frame: 0 = skip
   float threshold;
   float* errors;                                           // frames * H (+inf: stopped early, cannot be the winner)
   float* transforms;                                       // frames * H * 16
-  unsigned* best_bits;                                     // per frame: float bits of the lowest complete error so far (init 0x7f800000)
-  int early_exit;                                          // 1: stop a hypothesis whose partial error already exceeds that
+  int early_exit;                                          // 1: the shared-memory scorer may stop a hypothesis whose partial error
+                                                           // already exceeds the frame's lowest complete one (OPE_SACIA_EARLY_EXIT=0: never)
+  unsigned* best_bits;                                     // set by sacia_batch_device: per frame, float bits of the lowest complete error
   unsigned short* seed_tab; float4* seed_geo;              // set by sacia_batch_device: per frame, the seed grid of the distance search
   const float4* src_scan;                                  // set by sacia_batch_device: the source in scoring order, .w = original index
 };
@@ -296,7 +298,9 @@ int fpfh_smem_batch(ope_ctx* ctx, const float4* pts, const float4* nrm, const in
                     float* spfh, float* fpfh);
 int feature_knn_batch(ope_ctx* ctx, const float* ftgt, const int* d_counts, int stride, int frames, int max_nt, const float* fqry, int nq,
                       int dim, int k, int* out_idx);
-int sacia_batch_device(ope_ctx* ctx, const SaciaBatch& a, int frames, int max_nt, ope_reg_result* d_results);
+// scores hypotheses [h_begin, h_end) of every frame and writes each frame's winner to d_results: from shared memory (grid null,
+// every target <= max_nt <= 8 192 points) or, for one frame, through the target's grid index
+int sacia_batch_device(ope_ctx* ctx, const SaciaBatch& a, int frames, int max_nt, const GridView* grid, ope_reg_result* d_results);
 int fitness_batch_device(ope_ctx* ctx, const float4* tgt, const int* tgt_counts, const float4* src, const int* src_counts, int stride, int frames,
                          int max_nt, const ope_reg_result* d_icp, const int* d_active, double* d_out);
 bool icp_small_batch_applicable(const ope_icp_params& prm, size_t n_src, size_t n_tgt);

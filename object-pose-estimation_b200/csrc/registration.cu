@@ -1395,56 +1395,33 @@ __global__ void pairs_moments_kernel(const float4* __restrict__ src, const float
 }
 
 // ============================================================================================ SAC-IA ====
-struct SaciaDev {
-  GridView grid;
-  const float4* src;      // ns
-  const float4* tgt;      // original order
-  int ns;
-  int nr_samples, k_corr;
-  const int* samples;     // H * nr_samples
-  const int* picks;       // H * nr_samples
-  const int* knn_idx;     // ns * k_corr: feature-space neighbours of every source point
-  int h_begin;
-  float threshold;        // TruncatedError threshold (applied to squared distances)
-  float* terms;           // scratch: gridDim * ns floats
-  float* errors;          // H
-  float* transforms;      // H * 16
-};
-
+// Every hypothesis is scored by the same stages, for a whole batch of frames (ope_pose_batch) or for the one frame of
+// ope_sacia_align / ope_pose_estimate_final:
+//   sacia_transform_batch_kernel  one THREAD per (frame, hypothesis): the 5-point Umeyama (double moments, as everywhere)
+//   sacia_seed_batch_kernel       blockIdx.x = frame, blockIdx.y = a share of the cells: a kSeedG^3 grid around the frame's target;
+//                                 every cell remembers the target point nearest to its centre. A query looks up its (clamped) cell and starts its search from that
+//                                 point's distance: a bound within a cell size of the answer, so the box tests prune from the start
+//   sacia_score_batch_kernel      blockIdx.x = frame, blockIdx.y = a few consecutive hypotheses: the frame's target (at most
+//                                 kSaciaSmemMaxTargets points), its group boxes and the seed grid are staged in shared memory once
+//                                 per block
+//   sacia_kernel                  one frame whose target does not fit: one block per hypothesis, block_nn1 through the grid index
+//   sacia_select_batch_kernel     first strictly-lower error wins, per frame
+// Both scorers sum a hypothesis' terms as floats in point order in one thread (bit-exact with the reference's serial
+// `error += ...`, so the first-lowest-error hypothesis is the same one), and only the DISTANCE of the nearest neighbour enters a
+// term: ties need no index order.
 static constexpr int kSaciaThreads = 256;
 static constexpr int kSaciaMaxSamples = 16;
+static constexpr int kSaciaSmemMaxTargets = 8192;   // 128 KB of the 227 KB shared memory
 
-// one block per hypothesis: 5-point Umeyama (double moments, as everywhere), then every source point's
-// truncated NN error in parallel (one point per thread, block_nn1), then the float sum in point order by one thread
-// (bit-exact with the reference's serial `error += ...`, so the first-lowest-error hypothesis is the same one).
-__global__ void __launch_bounds__(kSaciaThreads) sacia_kernel(SaciaDev a) {
+__global__ void __launch_bounds__(kSaciaThreads) sacia_kernel(SaciaBatch a, GridView grid, float* __restrict__ terms_all) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   Nn1Smem<kSaciaThreads>* nn = reinterpret_cast<Nn1Smem<kSaciaThreads>*>(smem_raw);
   __shared__ Mat4 T;
   const int h = a.h_begin + blockIdx.x;
-  if (threadIdx.x == 0) {
-    double acc[16];
-    for (int i = 0; i < 16; ++i) acc[i] = 0.0;
-    for (int j = 0; j < a.nr_samples; ++j) {
-      const int si = a.samples[(size_t)h * a.nr_samples + j];
-      const int pick = a.picks[(size_t)h * a.nr_samples + j];
-      int ti = a.knn_idx[(size_t)si * a.k_corr + pick];
-      if (ti < 0) ti = a.knn_idx[(size_t)si * a.k_corr];  // fewer than k target features
-      const float4 sp = __ldg(a.src + si), tp = __ldg(a.tgt + ti);
-      const double sv[3] = {sp.x, sp.y, sp.z}, tv[3] = {tp.x, tp.y, tp.z};
-      acc[0] += 1.0;
-      for (int k = 0; k < 3; ++k) { acc[1 + k] += sv[k]; acc[4 + k] += tv[k]; }
-      for (int c = 0; c < 3; ++c)
-        for (int r = 0; r < 3; ++r) acc[7 + c * 3 + r] += tv[r] * sv[c];
-    }
-    Mat4 M;
-    umeyama_from_moments(acc, M);
-    T = M;
-    for (int i = 0; i < 16; ++i) a.transforms[(size_t)h * 16 + i] = M.m[i];
-  }
+  if (threadIdx.x < 16) T.m[threadIdx.x] = __ldg(a.transforms + (size_t)h * 16 + threadIdx.x);
   __syncthreads();
   const Mat4 M = T;
-  float* terms = a.terms + (size_t)blockIdx.x * a.ns;
+  float* terms = terms_all + (size_t)blockIdx.x * a.ns;
   for (int base = 0; base < a.ns; base += kSaciaThreads) {
     const int i = base + (int)threadIdx.x;
     float x = 0, y = 0, z = 0;
@@ -1455,7 +1432,7 @@ __global__ void __launch_bounds__(kSaciaThreads) sacia_kernel(SaciaDev a) {
       ok = finite3(x, y, z);
     }
     float d2;
-    const int idx = block_nn1<kSaciaThreads>(a.grid, nn, ok, x, y, z, a.threshold, -1, nullptr, d2);
+    const int idx = block_nn1<kSaciaThreads>(grid, nn, ok, x, y, z, a.threshold, -1, nullptr, d2);
     if (i < a.ns) terms[i] = (ok && idx >= 0 && d2 <= a.threshold) ? d2 / a.threshold : 1.0f;
   }
   __syncthreads();
@@ -1465,81 +1442,15 @@ __global__ void __launch_bounds__(kSaciaThreads) sacia_kernel(SaciaDev a) {
     a.errors[h] = error;
   }
 }
-// Small targets (a segmented cluster after 1 cm sampling: ~1 000 points, 16 KB): the whole target sits in SHARED memory and
-// every transformed source point scans it exhaustively — exact by construction ((d2, index) order), no index, no dependent
-// loads: every thread reads the same target point at the same time (shared-memory broadcast).
-static constexpr int kSaciaSmemMaxTargets = 8192;   // 128 KB of the 227 KB shared memory
-__global__ void __launch_bounds__(kSaciaThreads) sacia_smem_kernel(SaciaDev a, int nt) {
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  float4* tg = reinterpret_cast<float4*>(smem_raw);
-  __shared__ Mat4 T;
-  const int h = a.h_begin + blockIdx.x;
-  for (int j = threadIdx.x; j < nt; j += kSaciaThreads) tg[j] = __ldg(a.tgt + j);
-  if (threadIdx.x == 0) {
-    double acc[16];
-    for (int i = 0; i < 16; ++i) acc[i] = 0.0;
-    for (int j = 0; j < a.nr_samples; ++j) {
-      const int si = a.samples[(size_t)h * a.nr_samples + j];
-      const int pick = a.picks[(size_t)h * a.nr_samples + j];
-      int ti = a.knn_idx[(size_t)si * a.k_corr + pick];
-      if (ti < 0) ti = a.knn_idx[(size_t)si * a.k_corr];  // fewer than k target features
-      const float4 sp = __ldg(a.src + si), tp = __ldg(a.tgt + ti);
-      const double sv[3] = {sp.x, sp.y, sp.z}, tv[3] = {tp.x, tp.y, tp.z};
-      acc[0] += 1.0;
-      for (int k = 0; k < 3; ++k) { acc[1 + k] += sv[k]; acc[4 + k] += tv[k]; }
-      for (int c = 0; c < 3; ++c)
-        for (int r = 0; r < 3; ++r) acc[7 + c * 3 + r] += tv[r] * sv[c];
-    }
-    Mat4 M;
-    umeyama_from_moments(acc, M);
-    T = M;
-    for (int i = 0; i < 16; ++i) a.transforms[(size_t)h * 16 + i] = M.m[i];
-  }
-  __syncthreads();
-  const Mat4 M = T;
-  float* terms = a.terms + (size_t)blockIdx.x * a.ns;
-  for (int i = threadIdx.x; i < a.ns; i += kSaciaThreads) {
-    const float4 p = __ldg(a.src + i);
-    float x, y, z;
-    xform_point(M, p.x, p.y, p.z, x, y, z);
-    float term = 1.0f;
-    if (finite3(x, y, z)) {
-      float best = FLT_MAX;   // only the DISTANCE of the nearest neighbour enters the score: ties need no index order
-#pragma unroll 4
-      for (int j = 0; j < nt; ++j) {
-        const float4 t = tg[j];
-        const float d2 = dist2(x, y, z, t.x, t.y, t.z);   // a NaN target never compares below
-        best = d2 < best ? d2 : best;
-      }
-      if (best <= a.threshold) term = best / a.threshold;
-    }
-    terms[i] = term;
-  }
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    float error = 0.0f;
-    for (int i = 0; i < a.ns; ++i) error += terms[i];
-    a.errors[h] = error;
-  }
-}
-// Frame-spanning SAC-IA scoring. Every frame has its own target (tgt + f * stride, counts[f] points, in shared memory), decision
-// table (samples / picks + f * H * S) and feature neighbours (knn_idx + f * ns * k); the source (the model's coarse sample) is
-// shared. Same arithmetic as sacia_smem_kernel: same errors, bit for bit.
 // squared distance from a query to an axis-aligned box (0 inside); an empty box (lo = +inf, hi = -inf) gives +inf
 __device__ __forceinline__ float box_d2(const float4 lo, const float4 hi, float x, float y, float z) {
   const float ex = fmaxf(fmaxf(lo.x - x, x - hi.x), 0.0f), ey = fmaxf(fmaxf(lo.y - y, y - hi.y), 0.0f), ez = fmaxf(fmaxf(lo.z - z, z - hi.z), 0.0f);
   return ex * ex + ey * ey + ez * ez;
 }
-// The batch scores its hypotheses in three launches:
-//   sacia_transform_batch_kernel  one THREAD per (frame, hypothesis): the 5-point Umeyama (double moments, as everywhere)
-//   sacia_seed_batch_kernel       one block per frame: a kSeedG^3 grid around the frame's target; every cell remembers the target
-//                                 point nearest to its centre. A query looks up its (clamped) cell and starts its search from that
-//                                 point's distance: a bound within a cell size of the answer, so the box tests prune from the start
-//   sacia_score_batch_kernel      blockIdx.x = frame, blockIdx.y = kSaciaHypPerBlock consecutive hypotheses: the target, its group
-//                                 boxes and the seed grid are staged once per block
 static constexpr int kSeedG = 12;
 static constexpr int kSeedCells = kSeedG * kSeedG * kSeedG;
-static constexpr int kSaciaHypPerBlock = 16;
+static_assert(kSaciaSmemMaxTargets <= 65536, "the seed grid stores target indices as unsigned short");
+static constexpr int kSaciaHypPerBlock = 16;     // hypotheses per scoring block while the launch still fills the device
 static constexpr int kSaciaScoreThreads = 128;   // points per early-exit check: most hypotheses are out after the first one
 
 // The scoring kernel's work order of the source: along the Morton curve of its bounding box, so that the 32 points of a warp are
@@ -1610,9 +1521,10 @@ __global__ void __launch_bounds__(kSaciaThreads) sacia_source_order_kernel(const
 }
 
 __global__ void __launch_bounds__(128) sacia_transform_batch_kernel(SaciaBatch a, int frames) {
+  const int nh = a.h_end - a.h_begin;
   const int idx = blockIdx.x * 128 + threadIdx.x;
-  if (idx >= frames * a.H) return;
-  const int f = idx / a.H, h = idx - f * a.H;
+  if (idx >= frames * nh) return;
+  const int f = idx / nh, h = a.h_begin + idx - f * nh;
   if (!a.active[f]) return;
   const float4* tgt = a.tgt + (size_t)f * a.stride;
   double acc[16];
@@ -1673,8 +1585,8 @@ __global__ void __launch_bounds__(kSaciaThreads) sacia_seed_batch_kernel(SaciaBa
   const float cell = 1.5f * ext / (float)kSeedG;
   float org[3];
   for (int d = 0; d < 3; ++d) { org[d] = 0.5f * (box[d] + box[3 + d]) - 0.5f * cell * (float)kSeedG; if (!(fabsf(org[d]) < FLT_MAX)) org[d] = 0.0f; }
-  if (tid == 0) a.seed_geo[f] = make_float4(org[0], org[1], org[2], 1.0f / cell);
-  for (int c = tid; c < kSeedCells; c += kSaciaThreads) {
+  if (tid == 0 && blockIdx.y == 0) { a.seed_geo[f] = make_float4(org[0], org[1], org[2], 1.0f / cell); a.best_bits[f] = 0x7f800000u; }   // +inf
+  for (int c = (int)blockIdx.y * kSaciaThreads + tid; c < kSeedCells; c += (int)gridDim.y * kSaciaThreads) {
     const int cx = c % kSeedG, cy = (c / kSeedG) % kSeedG, cz = c / (kSeedG * kSeedG);
     const float x = org[0] + ((float)cx + 0.5f) * cell, y = org[1] + ((float)cy + 0.5f) * cell, z = org[2] + ((float)cz + 0.5f) * cell;
     float best = FLT_MAX;
@@ -1689,7 +1601,7 @@ __global__ void __launch_bounds__(kSaciaThreads) sacia_seed_batch_kernel(SaciaBa
   }
 }
 
-__global__ void __launch_bounds__(kSaciaScoreThreads) sacia_score_batch_kernel(SaciaBatch a) {
+__global__ void __launch_bounds__(kSaciaScoreThreads) sacia_score_batch_kernel(SaciaBatch a, int hyp_per_block) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   // blockIdx.x = frame (fastest): the hypothesis groups of one frame run one after the other, so the bound below is known early
   const int f = blockIdx.x;
@@ -1723,8 +1635,8 @@ __global__ void __launch_bounds__(kSaciaScoreThreads) sacia_score_batch_kernel(S
     glo[g] = lo; ghi[g] = hi;
   }
   unsigned* frame_best = a.best_bits + f;
-  const int h_end = min(a.H, ((int)blockIdx.y + 1) * kSaciaHypPerBlock);
-  for (int h = (int)blockIdx.y * kSaciaHypPerBlock; h < h_end; ++h) {
+  const int h_begin = a.h_begin + (int)blockIdx.y * hyp_per_block, h_end = min(a.h_end, h_begin + hyp_per_block);
+  for (int h = h_begin; h < h_end; ++h) {
     // (this barrier also closes the previous hypothesis: thread 0's final sum has read the terms)
     if (tid < 16) T.m[tid] = __ldg(a.transforms + ((size_t)f * a.H + h) * 16 + tid);
     __syncthreads();
@@ -1817,20 +1729,19 @@ __global__ void __launch_bounds__(kSaciaScoreThreads) sacia_score_batch_kernel(S
     }
   }
 }
-// first strictly-lower error wins, per frame (one thread per frame)
-__global__ void sacia_select_batch_kernel(const float* __restrict__ errors, const float* __restrict__ transforms, const int* __restrict__ active,
-                                          int H, int frames, ope_reg_result* __restrict__ out) {
+// first strictly-lower error wins, in hypothesis order (SURVEY A.6); one thread per frame
+__global__ void sacia_select_batch_kernel(SaciaBatch a, int frames, ope_reg_result* __restrict__ out) {
   const int f = blockIdx.x * blockDim.x + threadIdx.x;
-  if (f >= frames || !active[f]) return;
+  if (f >= frames || !a.active[f]) return;
   int best = -1;
   float lowest = 0.0f;
-  for (int h = 0; h < H; ++h) {
-    const float e = errors[(size_t)f * H + h];
+  for (int h = a.h_begin; h < a.h_end; ++h) {
+    const float e = a.errors[(size_t)f * a.H + h];
     if (best < 0 || e < lowest) { lowest = e; best = h; }
   }
   ope_reg_result r;
-  for (int i = 0; i < 16; ++i) r.T[i] = (best >= 0) ? transforms[((size_t)f * H + best) * 16 + i] : ((i % 5 == 0) ? 1.0f : 0.0f);
-  r.converged = best >= 0; r.state = 0; r.iterations = H; r.n_correspondences = 0; r.last_mse = 0.0;
+  for (int i = 0; i < 16; ++i) r.T[i] = (best >= 0) ? a.transforms[((size_t)f * a.H + best) * 16 + i] : ((i % 5 == 0) ? 1.0f : 0.0f);
+  r.converged = best >= 0; r.state = 0; r.iterations = a.H; r.n_correspondences = 0; r.last_mse = 0.0;
   r.best_error = lowest; r.best_iteration = best; r.reserved = 0;
   out[f] = r;
 }
@@ -1877,22 +1788,6 @@ __global__ void __launch_bounds__(kNnThreads) fitness_smem_batch_kernel(const fl
   }
   block_reduce_store<2>(acc, smem, fin);
   if (threadIdx.x == 0) out[f] = fin[1] > 0 ? fin[0] / fin[1] : DBL_MAX;
-}
-// first strictly-lower error wins, in hypothesis order (SURVEY A.6)
-__global__ void sacia_select_kernel(const float* __restrict__ errors, const float* __restrict__ transforms, int h_begin,
-                                    int h_end, ope_reg_result* __restrict__ out) {
-  if (blockIdx.x != 0 || threadIdx.x != 0) return;
-  int best = -1;
-  float lowest = 0.0f;
-  for (int h = h_begin; h < h_end; ++h) {
-    const float e = errors[h];
-    if (best < 0 || e < lowest) { lowest = e; best = h; }
-  }
-  ope_reg_result r;
-  for (int i = 0; i < 16; ++i) r.T[i] = (best >= 0) ? transforms[(size_t)best * 16 + i] : ((i % 5 == 0) ? 1.0f : 0.0f);
-  r.converged = best >= 0; r.state = 0; r.iterations = 0; r.n_correspondences = 0; r.last_mse = 0.0;
-  r.best_error = lowest; r.best_iteration = best; r.reserved = 0;
-  *out = r;
 }
 
 // ================================================================================================ host ==
@@ -2532,6 +2427,12 @@ static int draw_samples(LibcRandSession& rng, const float* src, size_t ns, size_
   return OPE_OK;
 }
 
+// dynamic shared memory of sacia_score_batch_kernel: the target padded to groups of 8, the group boxes, the terms, the seed grid
+static size_t sacia_score_bytes(int max_nt, int ns) {
+  const size_t nt8 = ((size_t)max_nt + 7) & ~(size_t)7;
+  return (nt8 + 2 * (nt8 / 8)) * sizeof(float4) + (size_t)ns * sizeof(float) + (size_t)kSeedCells * sizeof(unsigned short);
+}
+
 int sacia_device(ope_ctx* ctx, const ope_cloud* src, const float* d_fsrc, const ope_cloud* tgt, const float* d_ftgt,
                  const ope_sacia_params& prm, const ope_rng_table* table, const float* host_src_xyz3, ope_reg_result* res,
                  float* out_errors_host) {
@@ -2540,7 +2441,7 @@ int sacia_device(ope_ctx* ctx, const ope_cloud* src, const float* d_fsrc, const 
   if (src->n == 0 || tgt->n == 0) return fail(ctx, OPE_ERR_EMPTY, "empty cloud");
   if ((size_t)S > src->n) return fail(ctx, OPE_ERR_INVALID, "The number of samples must not be greater than the number of points");
   int h0 = 0, h1 = H;
-  if (prm.hypothesis_end > prm.hypothesis_begin) { h0 = std::max(0, prm.hypothesis_begin); h1 = std::min(H, prm.hypothesis_end); }
+  if (prm.hypothesis_end > prm.hypothesis_begin) { h0 = std::min(H, std::max(0, prm.hypothesis_begin)); h1 = std::max(h0, std::min(H, prm.hypothesis_end)); }
   float final_msd = prm.min_sample_distance;
   // ---- decision table: replayed or drawn from libc rand() ----
   std::vector<int32_t> hs, hp;
@@ -2569,53 +2470,47 @@ int sacia_device(ope_ctx* ctx, const ope_cloud* src, const float* d_fsrc, const 
   for (size_t i = 0; i < (size_t)H * S; ++i)
     if (samples[i] < 0 || (size_t)samples[i] >= src->n || picks[i] < 0 || picks[i] >= K)
       return fail(ctx, OPE_ERR_INVALID, "rng table entry out of range");
-  // ---- device side ----
+  // ---- device side: a one-frame run of the frame-spanning stages ----
   const size_t ns = src->n;
-  Scratch<int> d_samples(ctx), d_picks(ctx), d_knn(ctx);
-  Scratch<float> d_terms(ctx), d_errors(ctx), d_T(ctx), d_knn_d2(ctx);
+  Scratch<int> d_samples(ctx), d_picks(ctx), d_knn(ctx), d_frame(ctx);
+  Scratch<float> d_errors(ctx), d_T(ctx), d_knn_d2(ctx);
   Scratch<ope_reg_result> d_res(ctx);
   OPE_TRY(d_samples.alloc((size_t)H * S)); OPE_TRY(d_picks.alloc((size_t)H * S));
   OPE_TRY(d_knn.alloc(ns * K)); OPE_TRY(d_knn_d2.alloc(ns * K));
-  const int nh = h1 - h0;
-  OPE_TRY(d_terms.alloc((size_t)std::max(nh, 1) * ns));
-  OPE_TRY(d_errors.alloc(H)); OPE_TRY(d_T.alloc((size_t)H * 16)); OPE_TRY(d_res.alloc(1));
+  OPE_TRY(d_errors.alloc(H)); OPE_TRY(d_T.alloc((size_t)H * 16)); OPE_TRY(d_res.alloc(1)); OPE_TRY(d_frame.alloc(2));
+  const int frame[2] = {(int)tgt->n, 1};   // counts[0], active[0]
   OPE_CUDA_TRY(ctx, cudaMemcpyAsync(d_samples.p, samples, (size_t)H * S * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
   OPE_CUDA_TRY(ctx, cudaMemcpyAsync(d_picks.p, picks, (size_t)H * S * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
+  OPE_CUDA_TRY(ctx, cudaMemcpyAsync(d_frame.p, frame, sizeof(frame), cudaMemcpyHostToDevice, ctx->stream));
   OPE_CUDA_TRY(ctx, cudaMemsetAsync(d_errors.p, 0xff, (size_t)H * sizeof(float), ctx->stream));  // NaN = not evaluated
   // findSimilarFeatures for every source point at once (K6)
   OPE_TRY(feature_knn_device(ctx, d_ftgt, tgt->n, d_fsrc, ns, 33, K, d_knn.p, d_knn_d2.p));
-  SaciaDev a;
+  SaciaBatch a;
   std::memset(&a, 0, sizeof(a));
-  const char* force = std::getenv("OPE_SACIA_PATH");   // "grid" / "smem": force a path (tests); default: by target size
-  const bool use_smem = tgt->n <= (size_t)kSaciaSmemMaxTargets && !(force && std::strcmp(force, "grid") == 0);
-  if (!use_smem) {   // the spatial index is only needed when the target does not fit in shared memory
+  a.src = src->pts; a.ns = (int)ns; a.tgt = tgt->pts; a.counts = d_frame.p; a.active = d_frame.p + 1;
+  a.nr_samples = S; a.k_corr = K; a.H = H; a.h_begin = h0; a.h_end = h1;
+  a.samples = d_samples.p; a.picks = d_picks.p; a.knn_idx = d_knn.p;
+  a.threshold = (float)prm.max_correspondence_distance; a.errors = d_errors.p; a.transforms = d_T.p;
+  a.early_exit = out_errors_host == nullptr;   // a hypothesis that stops early reports +inf: the caller gets every error exactly
+  // the shared-memory scorer where the target and the source's terms fit, the grid index otherwise
+  const char* force = std::getenv("OPE_SACIA_PATH");   // "grid" / "smem": force a path (tests); default: by size
+  bool use_smem = tgt->n <= (size_t)kSaciaSmemMaxTargets && !(force && std::strcmp(force, "grid") == 0);
+  if (use_smem) {
+    int optin = 0;
+    cudaFuncAttributes fa;
+    OPE_CUDA_TRY(ctx, cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, ctx->device));
+    OPE_CUDA_TRY(ctx, cudaFuncGetAttributes(&fa, (const void*)sacia_score_batch_kernel));
+    use_smem = sacia_score_bytes((int)tgt->n, (int)ns) + fa.sharedSizeBytes <= (size_t)optin;
+  }
+  GridView grid;
+  if (!use_smem) {
     OPE_TRY(cloud_bbox(ctx, const_cast<ope_cloud*>(tgt)));
-    OPE_TRY(cloud_grid(ctx, tgt, knn_cell_size(tgt, 1), &a.grid));
+    OPE_TRY(cloud_grid(ctx, tgt, knn_cell_size(tgt, 1), &grid));
   }
-  a.src = src->pts; a.tgt = tgt->pts; a.ns = (int)ns; a.nr_samples = S; a.k_corr = K;
-  a.samples = d_samples.p; a.picks = d_picks.p; a.knn_idx = d_knn.p; a.h_begin = h0;
-  a.threshold = (float)prm.max_correspondence_distance;
-  a.terms = d_terms.p; a.errors = d_errors.p; a.transforms = d_T.p;
-  if (nh > 0) {
-    cudaEventRecord(ctx->kev[1][0], ctx->stream);
-    if (use_smem) {
-      const size_t bytes = tgt->n * sizeof(float4);
-      OPE_TRY(dyn_smem(ctx, (const void*)sacia_smem_kernel, bytes));
-      sacia_smem_kernel<<<nh, kSaciaThreads, bytes, ctx->stream>>>(a, (int)tgt->n);
-    } else {
-      OPE_TRY(dyn_smem(ctx, (const void*)sacia_kernel, sizeof(Nn1Smem<kSaciaThreads>)));
-      sacia_kernel<<<nh, kSaciaThreads, sizeof(Nn1Smem<kSaciaThreads>), ctx->stream>>>(a);
-    }
-    cudaEventRecord(ctx->kev[1][1], ctx->stream);
-    ctx->kev_valid[1] = true;
-    OPE_TRY(check_launch(ctx, use_smem ? "sacia_smem_kernel" : "sacia_kernel"));
-  }
-  sacia_select_kernel<<<1, 32, 0, ctx->stream>>>(d_errors.p, d_T.p, h0, h1, d_res.p);
-  OPE_TRY(check_launch(ctx, "sacia_select_kernel"));
+  OPE_TRY(sacia_batch_device(ctx, a, 1, (int)tgt->n, use_smem ? nullptr : &grid, d_res.p));
   void* h;
   OPE_TRY(read_back(ctx, d_res.p, sizeof(ope_reg_result), &h));
   std::memcpy(res, h, sizeof(ope_reg_result));
-  res->iterations = H;
   res->last_mse = (double)final_msd;   // min_sample_distance_ as selectSamples left it (it halves the member and keeps it halved)
   if (out_errors_host) {
     OPE_CUDA_TRY(ctx, cudaMemcpyAsync(out_errors_host, d_errors.p, (size_t)H * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
@@ -2624,36 +2519,56 @@ int sacia_device(ope_ctx* ctx, const ope_cloud* src, const float* d_fsrc, const 
   return OPE_OK;
 }
 
-// ---- frame-spanning launches for ope_pose_batch (batch.cu) ----------------------------------------------------------------
-int sacia_batch_device(ope_ctx* ctx, const SaciaBatch& a_in, int frames, int max_nt, ope_reg_result* d_results) {
+// ---- the SAC-IA stages, for ope_pose_batch (batch.cu) and, with one frame, sacia_device ----------------------------------
+int sacia_batch_device(ope_ctx* ctx, const SaciaBatch& a_in, int frames, int max_nt, const GridView* grid, ope_reg_result* d_results) {
   SaciaBatch a = a_in;
   if (frames <= 0 || a.H <= 0) return OPE_OK;
   if (a.nr_samples < 1 || a.nr_samples > kSaciaMaxSamples || a.k_corr < 1 || a.k_corr > 16) return fail(ctx, OPE_ERR_INVALID, "bad SAC-IA parameters");
-  if (max_nt > kSaciaSmemMaxTargets) return fail(ctx, OPE_ERR_CAPACITY, "batched SAC-IA: target larger than the shared-memory path");
-  if (max_nt > 65535) return fail(ctx, OPE_ERR_CAPACITY, "batched SAC-IA: target larger than the seed grid's index type");
+  if (a.h_begin < 0 || a.h_end > a.H || a.h_begin > a.h_end) return fail(ctx, OPE_ERR_INVALID, "bad SAC-IA hypothesis range");
+  if (grid && frames != 1) return fail(ctx, OPE_ERR_INVALID, "the grid SAC-IA scorer takes one frame");
+  if (!grid && max_nt > kSaciaSmemMaxTargets) return fail(ctx, OPE_ERR_CAPACITY, "batched SAC-IA: target larger than the shared-memory path");
+  { const char* e = std::getenv("OPE_SACIA_EARLY_EXIT"); if (e && std::atoi(e) == 0) a.early_exit = 0; }
+  const int nh = a.h_end - a.h_begin;
   Scratch<unsigned short> seed_tab(ctx);
-  Scratch<float4> seed_geo(ctx);
-  OPE_TRY(seed_tab.alloc((size_t)frames * kSeedCells)); OPE_TRY(seed_geo.alloc((size_t)frames));
-  a.seed_tab = seed_tab.p; a.seed_geo = seed_geo.p;
-  Scratch<float4> src_scan(ctx);
-  OPE_TRY(src_scan.alloc((size_t)a.ns));
-  sacia_source_order_kernel<<<1, kSaciaThreads, 0, ctx->stream>>>(a.src, a.ns, src_scan.p);
-  OPE_TRY(check_launch(ctx, "sacia_source_order_kernel"));
-  a.src_scan = src_scan.p;
-  const size_t nt8 = ((size_t)max_nt + 7) & ~(size_t)7, ng = nt8 / 8;
-  const size_t bytes = (nt8 + 2 * ng) * sizeof(float4) + (size_t)a.ns * sizeof(float) + (size_t)kSeedCells * sizeof(unsigned short);
-  sacia_transform_batch_kernel<<<div_up((size_t)frames * a.H, 128), 128, 0, ctx->stream>>>(a, frames);
-  OPE_TRY(check_launch(ctx, "sacia_transform_batch_kernel"));
-  OPE_TRY(dyn_smem(ctx, (const void*)sacia_seed_batch_kernel, nt8 * sizeof(float4)));
-  sacia_seed_batch_kernel<<<frames, kSaciaThreads, nt8 * sizeof(float4), ctx->stream>>>(a);
-  OPE_TRY(check_launch(ctx, "sacia_seed_batch_kernel"));
-  OPE_TRY(dyn_smem(ctx, (const void*)sacia_score_batch_kernel, bytes));
-  cudaEventRecord(ctx->kev[1][0], ctx->stream);
-  sacia_score_batch_kernel<<<dim3(frames, (a.H + kSaciaHypPerBlock - 1) / kSaciaHypPerBlock), kSaciaScoreThreads, bytes, ctx->stream>>>(a);
-  cudaEventRecord(ctx->kev[1][1], ctx->stream);
-  ctx->kev_valid[1] = true;
-  OPE_TRY(check_launch(ctx, "sacia_score_batch_kernel"));
-  sacia_select_batch_kernel<<<div_up((size_t)frames, 128), 128, 0, ctx->stream>>>(a.errors, a.transforms, a.active, a.H, frames, d_results);
+  Scratch<float4> seed_geo(ctx), src_scan(ctx);
+  Scratch<unsigned> best_bits(ctx);
+  Scratch<float> terms(ctx);
+  if (nh > 0) {
+    sacia_transform_batch_kernel<<<div_up((size_t)frames * nh, 128), 128, 0, ctx->stream>>>(a, frames);
+    OPE_TRY(check_launch(ctx, "sacia_transform_batch_kernel"));
+  }
+  if (nh > 0 && grid) {
+    OPE_TRY(terms.alloc((size_t)nh * a.ns));
+    OPE_TRY(dyn_smem(ctx, (const void*)sacia_kernel, sizeof(Nn1Smem<kSaciaThreads>)));
+    cudaEventRecord(ctx->kev[1][0], ctx->stream);
+    sacia_kernel<<<nh, kSaciaThreads, sizeof(Nn1Smem<kSaciaThreads>), ctx->stream>>>(a, *grid, terms.p);
+    cudaEventRecord(ctx->kev[1][1], ctx->stream);
+    ctx->kev_valid[1] = true;
+    OPE_TRY(check_launch(ctx, "sacia_kernel"));
+  } else if (nh > 0) {
+    OPE_TRY(seed_tab.alloc((size_t)frames * kSeedCells)); OPE_TRY(seed_geo.alloc((size_t)frames)); OPE_TRY(best_bits.alloc((size_t)frames));
+    OPE_TRY(src_scan.alloc((size_t)a.ns));
+    a.seed_tab = seed_tab.p; a.seed_geo = seed_geo.p; a.best_bits = best_bits.p; a.src_scan = src_scan.p;
+    sacia_source_order_kernel<<<1, kSaciaThreads, 0, ctx->stream>>>(a.src, a.ns, src_scan.p);
+    OPE_TRY(check_launch(ctx, "sacia_source_order_kernel"));
+    const size_t nt8 = ((size_t)max_nt + 7) & ~(size_t)7, bytes = sacia_score_bytes(max_nt, a.ns);
+    // every block of a frame stages its target and finds the same box; a few frames split the cells over more blocks
+    const unsigned seed_blocks = std::max(1u, std::min(div_up(kSeedCells, kSaciaThreads), (unsigned)(2 * ctx->sm_count / frames)));
+    OPE_TRY(dyn_smem(ctx, (const void*)sacia_seed_batch_kernel, nt8 * sizeof(float4)));
+    sacia_seed_batch_kernel<<<dim3(frames, seed_blocks), kSaciaThreads, nt8 * sizeof(float4), ctx->stream>>>(a);
+    OPE_TRY(check_launch(ctx, "sacia_seed_batch_kernel"));
+    // kSaciaHypPerBlock hypotheses per block while that still gives every SM two blocks, fewer for a few frames (the winner, its
+    // error and its transform do not depend on how the hypotheses are grouped)
+    int hyp_per_block = kSaciaHypPerBlock;
+    while (hyp_per_block > 1 && (size_t)frames * div_up(nh, hyp_per_block) < 2 * (size_t)ctx->sm_count) hyp_per_block /= 2;
+    OPE_TRY(dyn_smem(ctx, (const void*)sacia_score_batch_kernel, bytes));
+    cudaEventRecord(ctx->kev[1][0], ctx->stream);
+    sacia_score_batch_kernel<<<dim3(frames, div_up(nh, hyp_per_block)), kSaciaScoreThreads, bytes, ctx->stream>>>(a, hyp_per_block);
+    cudaEventRecord(ctx->kev[1][1], ctx->stream);
+    ctx->kev_valid[1] = true;
+    OPE_TRY(check_launch(ctx, "sacia_score_batch_kernel"));
+  }
+  sacia_select_batch_kernel<<<div_up((size_t)frames, 128), 128, 0, ctx->stream>>>(a, frames, d_results);
   return check_launch(ctx, "sacia_select_batch_kernel");
 }
 

@@ -178,7 +178,7 @@ class Context:
         return int(lib().ope_ctx_launch_count(self.h))
 
     def last_kernel_ms(self, which=0):
-        """device time of the last icp_kernel (0) / sacia_kernel (1) launch, from CUDA events on the ctx stream"""
+        """device time of the last icp_kernel (0) / SAC-IA scorer (1) launch, from CUDA events on the ctx stream"""
         return float(lib().ope_ctx_last_kernel_ms(self.h, int(which)))
 
     def feature_knn_stats(self):
