@@ -270,6 +270,22 @@ int ope_pose_stage_ms(const ope_pose_tracker* t, double out[8]);
 int ope_pose_batch(ope_ctx* ctx, const ope_pose_params* prm, const float* model_xyz, size_t n_model, const ope_frame_input* frames,
                    size_t n_frames, const ope_rng_table* tables, int workers, ope_pose_result* results, int32_t* status);
 
+/* Advance n trackers of this context by one frame each. For every i the result is what
+ *   ope_pose_estimate_final_device(trackers[i], &sources[i], target_i, tables ? &tables[i] : NULL, &results[i])
+ * returns and leaves behind, the calls made in index order: the same results, the same tracker state
+ * (alignedSource, cloudModel, fitnessScoreFine, alignedStrength, firstTimePose), the same *sources[i]
+ * afterwards, and the same consumption of libc rand() when tables == NULL. A tracker draws a table, or
+ * uses tables[i], only if it runs SAC-IA. targets: as ope_pose_batch's frames (host points or device
+ * clouds; n == 0 means an empty target). Trackers and source handles must be distinct and belong to ctx.
+ * Trackers may carry different models. Those whose parameters equal trackers[0]'s run through the frame-spanning launches of
+ * ope_pose_batch with a per-tracker source; the others, and clouds outside those launches' capacities, through the single call.
+ * status: n return codes or NULL; returns OPE_OK when every tracker succeeded, else the first failing tracker's code (a failing
+ * tracker's state changes as the single call would change it). Duplicate or foreign trackers or sources, or a NULL source,
+ * return OPE_ERR_INVALID before anything changes. */
+int ope_pose_tracker_step_batch(ope_ctx* ctx, ope_pose_tracker* const* trackers, ope_cloud** sources,
+                                const ope_frame_input* targets, size_t n, const ope_rng_table* tables,
+                                ope_pose_result* results, int32_t* status);
+
 /* Device time per stage of ope_pose_batch's frame-spanning launches (CUDA events on the context's stream), in milliseconds,
  * accumulated over the calls since the last reset: [0] staging + H2D of the clusters [1] target UniformSampling (1 cm + 8 mm)
  * [2] target normals [3] SPFH + FPFH [4] feature k-NN [5] SAC-IA pool [6] model under the coarse pose, 8 mm sampling [7] source

@@ -34,25 +34,10 @@
 
 namespace ope {
 
-static constexpr int kBCap = 4096;        // capacity of a sampled cloud (normals / ICP shared-memory paths)
-static constexpr int kBFeatCap = 2048;    // capacity of the 1 cm target sample (FPFH shared-memory path)
 static constexpr int kBTable = 8192;      // voxel hash slots per block (load factor <= 0.5 at kBCap voxels)
 static constexpr int kBThreads = 1024;
 static constexpr unsigned long long kEmpty = ~0ull;
 
-struct BSampleArgs {
-  const float4* pts;                // XFORM: the shared model; else the concatenated clusters
-  const int* offsets;               // !XFORM: first point of frame f
-  const int* counts;                // !XFORM: points of frame f
-  int n_model;                      // XFORM
-  const ope_reg_result* xforms;     // XFORM: frame f's coarse pose
-  const int* active;                // frames to process (null: all)
-  float inv_leaf[2];
-  int cap[2];                       // output capacity per leaf
-  float4* out[2];                   // leaf l, frame f: out[l] + f * kBCap
-  int* out_counts[2];               // leaf l: counts[f]
-  int* flags;                       // per frame: |= 1 when a sample overflowed its capacity / the voxel frame is too large
-};
 
 struct SampleSmem {
   unsigned long long keys[kBTable];
@@ -73,20 +58,20 @@ __device__ __forceinline__ unsigned hash_cell(long long c) {
 // pcl::UniformSampling (SURVEY A.1) of one cloud per block: bounding box -> voxel frame -> per voxel the point with the smallest
 // (||p4 - ijk4||^2, index) -> selected points in ascending voxel index. The voxel table is a shared-memory hash (linear probing,
 // 64-bit keys); the result equals uniform_sample_device + gather_cloud (grid.cu) point for point.
-template <bool XFORM>
 __global__ void __launch_bounds__(kBThreads) bsample_kernel(BSampleArgs a) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   SampleSmem* sm = reinterpret_cast<SampleSmem*>(smem_raw);
   const int f = blockIdx.x, leaf = blockIdx.y;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   if (a.active && !a.active[f]) return;
-  const float4* pts = XFORM ? a.pts : a.pts + a.offsets[f];
-  const int n = XFORM ? a.n_model : a.counts[f];
+  const float4* pts = a.src[f];
+  const int n = a.counts[f];
+  const bool xf = a.xforms && (!a.xform_on || a.xform_on[f]);
   Mat4 T;
-  if (XFORM) for (int i = 0; i < 16; ++i) T.m[i] = a.xforms[f].T[i];
+  if (xf) for (int i = 0; i < 16; ++i) T.m[i] = a.xforms[f].T[i];
   auto load = [&](int i) {
     float4 p = __ldg(pts + i);
-    if (XFORM) { float x, y, z; xform_point(T, p.x, p.y, p.z, x, y, z); p.x = x; p.y = y; p.z = z; }
+    if (xf) { float x, y, z; xform_point(T, p.x, p.y, p.z, x, y, z); p.x = x; p.y = y; p.z = z; }
     return p;
   };
   // ---- bounding box of the finite points ----
@@ -208,6 +193,12 @@ __global__ void __launch_bounds__(kBThreads) bsample_kernel(BSampleArgs a) {
     out[j] = p;
   }
   if (tid == 0) *out_count = m;
+}
+
+int bsample_batch(ope_ctx* ctx, const BSampleArgs& a, int frames, int leaves) {
+  OPE_TRY(dyn_smem(ctx, (const void*)bsample_kernel, sizeof(SampleSmem)));
+  bsample_kernel<<<dim3(frames, leaves), kBThreads, sizeof(SampleSmem), ctx->stream>>>(a);
+  return check_launch(ctx, "bsample_kernel");
 }
 
 // pcl::removeNaNNormalsFromPointCloud (D&L/src/poseestimator.cpp:215-216) for one cloud per block: points whose normal is finite,
@@ -336,7 +327,6 @@ __global__ void __launch_bounds__(kBThreads) morton_sort_batch_kernel(const floa
   }
 }
 
-namespace {
 // per-stage device time of the chunk (CUDA events on the context's stream), accumulated into ctx->batch_stage_ms
 struct ChunkTimer {
   ope_ctx* ctx;
@@ -363,6 +353,7 @@ struct ChunkTimer {
     for (auto& e : ev) cudaEventDestroy(e);
   }
 };
+namespace {
 struct DevGuardF { ope_ctx* ctx; float* p = nullptr; explicit DevGuardF(ope_ctx* c) : ctx(c) {} ~DevGuardF() { dfree(ctx, p); } };
 template <typename T>
 int download(ope_ctx* ctx, const T* d, size_t n, std::vector<T>& h) {
@@ -373,6 +364,137 @@ int download(ope_ctx* ctx, const T* d, size_t n, std::vector<T>& h) {
   return OPE_OK;
 }
 }  // namespace
+
+// The fine stage of a chunk (estimateFinePose, :161-379): frame f's source (sa.src / sa.counts, through sa.xforms where set) sampled
+// at the fine leaf into slab [2], its normals, removeNaNNormalsFromPointCloud of tp2 (slab [1], sampled with its normals by the
+// caller) and sp2, the ICP's Morton work order, ICP, getFitnessScore. A frame that leaves the envelope leaves h_active; for the
+// others by_frame (ICP), h_fit and h_cc (compacted counts: [0, B) tp2, [B, 2B) sp2) hold the results.
+int fine_stage(ope_ctx* ctx, const ope_pose_params& P, int B, const BatchClouds& c, BSampleArgs sa, std::vector<int>& h_active,
+               std::vector<ope_reg_result>& by_frame, std::vector<double>& h_fit, std::vector<int>& h_cc, ChunkTimer* tm) {
+  const size_t slab = (size_t)B * kBCap;
+  float4 *sampled = c.sampled, *normals = c.normals, *compacted = c.compacted, *cnormals = c.cnormals;
+  int *d_counts = c.counts, *d_ccounts = c.ccounts, *d_flags = c.flags, *d_active = c.active;
+  const float vp[3] = {0, 0, 0};
+  sa.active = d_active; sa.flags = d_flags;
+  sa.inv_leaf[0] = 1.0f / P.fine_leaf; sa.cap[0] = kBCap; sa.out[0] = sampled + 2 * slab; sa.out_counts[0] = d_counts + 2 * (size_t)B;
+  bsample_kernel<<<dim3(B, 1), kBThreads, sizeof(SampleSmem), ctx->stream>>>(sa);
+  OPE_TRY(check_launch(ctx, "bsample_kernel<source>"));
+  std::vector<int> h_sp2;
+  OPE_TRY(download(ctx, d_counts + 2 * (size_t)B, (size_t)B, h_sp2));
+  std::vector<int> h_flags;
+  OPE_TRY(download(ctx, d_flags, (size_t)B, h_flags));
+  int max_sp2 = 0;
+  for (int i = 0; i < B; ++i) {
+    if (!h_active[(size_t)i]) continue;
+    if (h_flags[(size_t)i] || h_sp2[(size_t)i] <= 0) { h_active[(size_t)i] = 0; continue; }
+    max_sp2 = std::max(max_sp2, h_sp2[(size_t)i]);
+  }
+  OPE_CUDA_TRY(ctx, cudaMemcpyAsync(d_active, h_active.data(), B * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
+  if (tm) tm->mark();   // [6] model sampling
+  OPE_TRY(normals_smem_batch(ctx, sampled + 2 * slab, d_counts + 2 * (size_t)B, kBCap, B, max_sp2, P.normal_k, vp, normals + 2 * slab));
+  if (tm) tm->mark();   // [7] source normals
+  // removeNaNNormalsFromPointCloud on both fine clouds (:215-216): clouds [1] (tp2) and [2] (sp2)
+  compact_normals_batch_kernel<<<2 * B, kBThreads, 0, ctx->stream>>>(sampled + slab, normals + slab, d_counts + B, d_active, B,
+                                                                     compacted + slab, cnormals + slab, d_ccounts + B);
+  OPE_TRY(check_launch(ctx, "compact_normals_batch_kernel"));
+  OPE_TRY(download(ctx, d_ccounts + B, 2 * (size_t)B, h_cc));   // [0..B) tp2, [B..2B) sp2
+  // the ICP's work order: both fine clouds along their Morton curve (the raw samples' arrays are free by now)
+  const char* me = std::getenv("OPE_BATCH_MORTON");
+  const bool morton = !(me && std::atoi(me) == 0);
+  const float4* fine_pts = compacted;
+  const float4* fine_nrm = cnormals;
+  if (morton) {
+    morton_sort_batch_kernel<<<2 * B, kBThreads, 0, ctx->stream>>>(compacted + slab, cnormals + slab, d_ccounts + B, d_active, B,
+                                                                   sampled + slab, normals + slab);
+    OPE_TRY(check_launch(ctx, "morton_sort_batch_kernel"));
+    fine_pts = sampled; fine_nrm = normals;
+  }
+  std::vector<IcpBatchFrame> icp_frames;
+  std::vector<int> icp_of;
+  int max_tgt = 0;
+  for (int i = 0; i < B; ++i) {
+    if (!h_active[(size_t)i]) continue;
+    const int nt = h_cc[(size_t)i], nsrc = h_cc[(size_t)B + i];
+    if (nt < P.min_target_points || !icp_small_batch_applicable(P.icp, (size_t)nsrc, (size_t)nt)) { h_active[(size_t)i] = 0; continue; }
+    IcpBatchFrame fr;
+    fr.tgt_pts = fine_pts + slab + (size_t)i * kBCap; fr.tgt_nrm = fine_nrm + slab + (size_t)i * kBCap; fr.n_tgt = nt;
+    fr.src_pts = fine_pts + 2 * slab + (size_t)i * kBCap; fr.src_nrm = fine_nrm + 2 * slab + (size_t)i * kBCap; fr.n_src = nsrc;
+    icp_frames.push_back(fr);
+    icp_of.push_back(i);
+    max_tgt = std::max(max_tgt, nt);
+  }
+  if (icp_frames.empty()) return OPE_OK;
+  Scratch<ope_reg_result> d_fine(ctx);
+  Scratch<double> d_fit(ctx);
+  OPE_TRY(d_fine.alloc(B));
+  Scratch<ope_reg_result> d_icp(ctx);
+  const int NI = (int)icp_frames.size();
+  OPE_TRY(d_icp.alloc(NI));
+  if (tm) tm->mark();   // [8] NaN-normal compaction
+  OPE_TRY(icp_small_batch_device(ctx, P.icp, icp_frames.data(), NI, d_icp.p));
+  if (tm) tm->mark();   // [9] ICP
+  // ---- getFitnessScore (:354) of every aligned pair; the ICP results are indexed by their position in icp_frames ----
+  OPE_TRY(d_fit.alloc(B));
+  {
+    // scatter the compact ICP results back to frame order so that the fitness kernel can index by frame
+    std::vector<ope_reg_result> h_icp;
+    OPE_TRY(download(ctx, d_icp.p, (size_t)NI, h_icp));
+    by_frame.assign((size_t)B, ope_reg_result());
+    std::memset(by_frame.data(), 0, by_frame.size() * sizeof(ope_reg_result));
+    for (int j = 0; j < NI; ++j) by_frame[(size_t)icp_of[(size_t)j]] = h_icp[(size_t)j];
+    OPE_CUDA_TRY(ctx, cudaMemcpyAsync(d_fine.p, by_frame.data(), (size_t)B * sizeof(ope_reg_result), cudaMemcpyHostToDevice, ctx->stream));
+    OPE_CUDA_TRY(ctx, cudaMemcpyAsync(d_active, h_active.data(), B * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
+    OPE_TRY(fitness_batch_device(ctx, fine_pts + slab, d_ccounts + B, fine_pts + 2 * slab, d_ccounts + 2 * (size_t)B, kBCap, B, max_tgt,
+                                 d_fine.p, d_active, d_fit.p));
+    if (tm) tm->mark();   // [10] fitness
+    OPE_TRY(download(ctx, d_fit.p, (size_t)B, h_fit));   // also orders the host vectors above after their copies
+  }
+  return OPE_OK;
+}
+
+// Stages a chunk's targets in one device array (host points through the pinned arena, device clouds device-to-device) and
+// fills `d_src` with each frame's first point. h_active[i] == 0 on entry excludes frame i; empty frames are excluded here.
+// h_cnt[i]: the points of frame i (0 when excluded); *total == 0: nothing was staged.
+int stage_frames(ope_ctx* ctx, const ope_frame_input* frames, int B, std::vector<int>& h_active, std::vector<int>& h_off,
+                 std::vector<int>& h_cnt, Scratch<float4>& clusters, Scratch<const float4*>& d_src, size_t* total_out) {
+  h_off.assign((size_t)B, 0); h_cnt.assign((size_t)B, 0);
+  size_t total = 0;
+  *total_out = 0;
+  for (int i = 0; i < B; ++i) {
+    const ope_frame_input& in = frames[i];
+    const size_t n = in.points ? in.n : (in.cloud ? ((const ope_cloud*)in.cloud)->n : 0);
+    if (n == 0 || n > 0x3fffffff) h_active[(size_t)i] = 0;
+    h_off[(size_t)i] = (int)total; h_cnt[(size_t)i] = h_active[(size_t)i] ? (int)n : 0;
+    total += (size_t)h_cnt[(size_t)i];
+  }
+  if (total == 0 || total > 0x7fffffffull) return OPE_OK;
+  OPE_TRY(clusters.alloc(total));
+  OPE_TRY(d_src.alloc((size_t)B));
+  void* stage = nullptr;
+  OPE_TRY(stage_reserve(ctx, total * sizeof(float4) + (size_t)B * sizeof(const float4*), &stage));
+  float4* h = (float4*)stage;
+  for (int i = 0; i < B; ++i) {
+    if (!h_active[(size_t)i]) continue;
+    const ope_frame_input& in = frames[i];
+    float4* dst = h + h_off[(size_t)i];
+    if (in.points) {
+      const unsigned char* base = (const unsigned char*)in.points + in.offset;
+      for (size_t j = 0; j < in.n; ++j) { float v[3]; std::memcpy(v, base + j * in.stride, 12); dst[j] = make_float4(v[0], v[1], v[2], 1.0f); }
+    }
+  }
+  const float4** hp = (const float4**)(h + total);
+  for (int i = 0; i < B; ++i) hp[i] = clusters.p + h_off[(size_t)i];
+  OPE_CUDA_TRY(ctx, cudaMemcpyAsync(clusters.p, stage, total * sizeof(float4), cudaMemcpyHostToDevice, ctx->stream));
+  OPE_CUDA_TRY(ctx, cudaMemcpyAsync(d_src.p, hp, (size_t)B * sizeof(const float4*), cudaMemcpyHostToDevice, ctx->stream));
+  for (int i = 0; i < B; ++i) {   // device-resident clusters: device-to-device into their slot
+    const ope_frame_input& in = frames[i];
+    if (h_active[(size_t)i] && !in.points)
+      OPE_CUDA_TRY(ctx, cudaMemcpyAsync(clusters.p + h_off[(size_t)i], ((const ope_cloud*)in.cloud)->pts, (size_t)h_cnt[(size_t)i] * sizeof(float4),
+                                        cudaMemcpyDeviceToDevice, ctx->stream));
+  }
+  *total_out = total;
+  return OPE_OK;
+}
 
 // One chunk of frames through the frame-spanning launches. Returns in `done[i]` whether frame i was finished here (else the
 // caller runs it through the per-frame path). d_model: the full-resolution model; sp / d_fs: its coarse sample (with normals)
@@ -385,68 +507,38 @@ int pose_batch_chunk(ope_ctx* ctx, const ope_pose_params& P, const ope_cloud* d_
   for (int i = 0; i < B; ++i) done[i] = 0;
   if (B == 0) return OPE_OK;
   if (!icp_small_batch_applicable(P.icp, 1, 1) || P.icp.n_rejectors < 0 || (int)sp->n < S || sp->n == 0) return OPE_OK;   // not this path's configuration
-  // ---- stage the clusters: one concatenated float4 array ----
-  std::vector<int> h_off((size_t)B), h_cnt((size_t)B), h_active((size_t)B, 1);
+  std::vector<int> h_off, h_cnt, h_active((size_t)B, 1);
+  Scratch<float4> clusters(ctx);
+  Scratch<const float4*> d_src(ctx);
   size_t total = 0;
-  for (int i = 0; i < B; ++i) {
-    const ope_frame_input& in = frames[i];
-    const size_t n = in.points ? in.n : (in.cloud ? ((const ope_cloud*)in.cloud)->n : 0);
-    if (n == 0 || n > 0x3fffffff) h_active[(size_t)i] = 0;
-    h_off[(size_t)i] = (int)total; h_cnt[(size_t)i] = h_active[(size_t)i] ? (int)n : 0;
-    total += (size_t)h_cnt[(size_t)i];
-  }
-  if (total == 0 || total > 0x7fffffffull) return OPE_OK;
-  Scratch<float4> clusters(ctx), sampled(ctx), normals(ctx), compacted(ctx), cnormals(ctx);
-  Scratch<int> d_off(ctx), d_cnt(ctx), d_active(ctx), d_counts(ctx), d_ccounts(ctx), d_flags(ctx), d_samples(ctx), d_picks(ctx), d_knn(ctx);
+  OPE_TRY(stage_frames(ctx, frames, B, h_active, h_off, h_cnt, clusters, d_src, &total));
+  if (total == 0) return OPE_OK;
+  Scratch<float4> sampled(ctx), normals(ctx), compacted(ctx), cnormals(ctx);
+  Scratch<int> d_cnt(ctx), d_active(ctx), d_counts(ctx), d_ccounts(ctx), d_flags(ctx), d_samples(ctx), d_picks(ctx), d_knn(ctx);
   Scratch<float> spfh(ctx), fpfh(ctx), errors(ctx), transforms(ctx);
-  Scratch<ope_reg_result> d_coarse(ctx), d_fine(ctx);
-  Scratch<double> d_fit(ctx);
-  OPE_TRY(clusters.alloc(total));
-  {
-    void* stage = nullptr;
-    OPE_TRY(stage_reserve(ctx, total * sizeof(float4), &stage));
-    float4* h = (float4*)stage;
-    for (int i = 0; i < B; ++i) {
-      if (!h_active[(size_t)i]) continue;
-      const ope_frame_input& in = frames[i];
-      float4* dst = h + h_off[(size_t)i];
-      if (in.points) {
-        const unsigned char* base = (const unsigned char*)in.points + in.offset;
-        for (size_t j = 0; j < in.n; ++j) { float v[3]; std::memcpy(v, base + j * in.stride, 12); dst[j] = make_float4(v[0], v[1], v[2], 1.0f); }
-      }
-    }
-    OPE_CUDA_TRY(ctx, cudaMemcpyAsync(clusters.p, stage, total * sizeof(float4), cudaMemcpyHostToDevice, ctx->stream));
-    for (int i = 0; i < B; ++i) {   // device-resident clusters: device-to-device into their slot
-      const ope_frame_input& in = frames[i];
-      if (h_active[(size_t)i] && !in.points)
-        OPE_CUDA_TRY(ctx, cudaMemcpyAsync(clusters.p + h_off[(size_t)i], ((const ope_cloud*)in.cloud)->pts, (size_t)h_cnt[(size_t)i] * sizeof(float4),
-                                          cudaMemcpyDeviceToDevice, ctx->stream));
-    }
-  }
+  Scratch<ope_reg_result> d_coarse(ctx);
   // sampled clouds: [0] tp1 (1 cm target), [1] tp2 (8 mm target), [2] sp2 (8 mm source), each B x kBCap
   const size_t slab = (size_t)B * kBCap;
   OPE_TRY(sampled.alloc(3 * slab)); OPE_TRY(normals.alloc(3 * slab)); OPE_TRY(compacted.alloc(3 * slab)); OPE_TRY(cnormals.alloc(3 * slab));
-  OPE_TRY(d_off.alloc(B)); OPE_TRY(d_cnt.alloc(B)); OPE_TRY(d_active.alloc(B)); OPE_TRY(d_counts.alloc(3 * (size_t)B)); OPE_TRY(d_ccounts.alloc(3 * (size_t)B));
+  OPE_TRY(d_cnt.alloc(B)); OPE_TRY(d_active.alloc(B)); OPE_TRY(d_counts.alloc(3 * (size_t)B)); OPE_TRY(d_ccounts.alloc(3 * (size_t)B));
   OPE_TRY(d_flags.alloc(B));
-  OPE_CUDA_TRY(ctx, cudaMemcpyAsync(d_off.p, h_off.data(), B * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
   OPE_CUDA_TRY(ctx, cudaMemcpyAsync(d_cnt.p, h_cnt.data(), B * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
   OPE_CUDA_TRY(ctx, cudaMemcpyAsync(d_active.p, h_active.data(), B * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
   OPE_CUDA_TRY(ctx, cudaMemsetAsync(d_flags.p, 0, B * sizeof(int), ctx->stream));
   OPE_CUDA_TRY(ctx, cudaMemsetAsync(d_counts.p, 0, 3 * (size_t)B * sizeof(int), ctx->stream));
   OPE_CUDA_TRY(ctx, cudaMemsetAsync(d_ccounts.p, 0, 3 * (size_t)B * sizeof(int), ctx->stream));
   ChunkTimer tm(ctx);
-  OPE_TRY(dyn_smem(ctx, (const void*)bsample_kernel<false>, sizeof(SampleSmem)));
-  OPE_TRY(dyn_smem(ctx, (const void*)bsample_kernel<true>, sizeof(SampleSmem)));
+  OPE_TRY(dyn_smem(ctx, (const void*)bsample_kernel, sizeof(SampleSmem)));
   tm.mark();   // [0] staging + H2D of the clusters
   // ---- target UniformSampling at the coarse and the fine leaf (subSampleAndCalculateNormals, :131-158) ----
   BSampleArgs sa;
   std::memset(&sa, 0, sizeof(sa));
-  sa.pts = clusters.p; sa.offsets = d_off.p; sa.counts = d_cnt.p; sa.active = d_active.p; sa.flags = d_flags.p;
+  sa.src = d_src.p; sa.counts = d_cnt.p; sa.active = d_active.p; sa.flags = d_flags.p;
   sa.inv_leaf[0] = 1.0f / P.coarse_leaf; sa.inv_leaf[1] = 1.0f / P.fine_leaf;
   sa.cap[0] = kBFeatCap; sa.cap[1] = kBCap;
   sa.out[0] = sampled.p; sa.out[1] = sampled.p + slab;
   sa.out_counts[0] = d_counts.p; sa.out_counts[1] = d_counts.p + B;
-  bsample_kernel<false><<<dim3(B, 2), kBThreads, sizeof(SampleSmem), ctx->stream>>>(sa);
+  bsample_kernel<<<dim3(B, 2), kBThreads, sizeof(SampleSmem), ctx->stream>>>(sa);
   OPE_TRY(check_launch(ctx, "bsample_kernel<target>"));
   std::vector<int> h_counts, h_flags;
   OPE_TRY(download(ctx, d_counts.p, 2 * (size_t)B, h_counts));
@@ -475,7 +567,7 @@ int pose_batch_chunk(ope_ctx* ctx, const ope_pose_params& P, const ope_cloud* d_
   // ---- findSimilarFeatures for every model point at once, SAC-IA pool, first strictly-lower error wins (:50-64) ----
   const int ns = (int)sp->n;
   OPE_TRY(d_knn.alloc((size_t)B * ns * K));
-  OPE_TRY(feature_knn_batch(ctx, fpfh.p, d_counts.p, kBCap, B, max_tp1, d_fs, ns, 33, K, d_knn.p));
+  OPE_TRY(feature_knn_batch(ctx, fpfh.p, d_counts.p, kBCap, B, max_tp1, d_fs, ns, 0, nullptr, 33, K, d_knn.p));
   tm.mark();   // [4] feature k-NN
   OPE_TRY(d_samples.alloc((size_t)B * H * S)); OPE_TRY(d_picks.alloc((size_t)B * H * S));
   {
@@ -503,7 +595,7 @@ int pose_batch_chunk(ope_ctx* ctx, const ope_pose_params& P, const ope_cloud* d_
     OPE_CUDA_TRY(ctx, cudaMemcpyAsync(d_samples.p, hs, tb * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
     OPE_CUDA_TRY(ctx, cudaMemcpyAsync(d_picks.p, hp, tb * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
   }
-  OPE_TRY(errors.alloc((size_t)B * H)); OPE_TRY(transforms.alloc((size_t)B * H * 16)); OPE_TRY(d_coarse.alloc(B)); OPE_TRY(d_fine.alloc(B));
+  OPE_TRY(errors.alloc((size_t)B * H)); OPE_TRY(transforms.alloc((size_t)B * H * 16)); OPE_TRY(d_coarse.alloc(B));
   SaciaBatch sb;
   std::memset(&sb, 0, sizeof(sb));
   sb.src = sp->pts; sb.ns = ns; sb.tgt = sampled.p; sb.counts = d_counts.p; sb.stride = kBCap;
@@ -521,81 +613,21 @@ int pose_batch_chunk(ope_ctx* ctx, const ope_pose_params& P, const ope_cloud* d_
   OPE_TRY(sacia_batch_device(ctx, sb, B, max_tp1, nullptr, d_coarse.p));
   tm.mark();   // [5] SAC-IA
   // ---- estimateFinePose (:161-379): the model under the coarse pose sampled at the fine leaf, never materialised ----
-  std::memset(&sa, 0, sizeof(sa));
-  sa.pts = d_model->pts; sa.n_model = (int)d_model->n; sa.xforms = d_coarse.p; sa.active = d_active.p; sa.flags = d_flags.p;
-  sa.inv_leaf[0] = 1.0f / P.fine_leaf; sa.cap[0] = kBCap; sa.out[0] = sampled.p + 2 * slab; sa.out_counts[0] = d_counts.p + 2 * (size_t)B;
-  bsample_kernel<true><<<dim3(B, 1), kBThreads, sizeof(SampleSmem), ctx->stream>>>(sa);
-  OPE_TRY(check_launch(ctx, "bsample_kernel<model>"));
-  std::vector<int> h_sp2;
-  OPE_TRY(download(ctx, d_counts.p + 2 * (size_t)B, (size_t)B, h_sp2));
-  OPE_TRY(download(ctx, d_flags.p, (size_t)B, h_flags));
-  int max_sp2 = 0;
-  for (int i = 0; i < B; ++i) {
-    if (!h_active[(size_t)i]) continue;
-    if (h_flags[(size_t)i] || h_sp2[(size_t)i] <= 0) { h_active[(size_t)i] = 0; continue; }
-    max_sp2 = std::max(max_sp2, h_sp2[(size_t)i]);
+  {   // every frame's source is the model
+    std::vector<const float4*> h_src((size_t)B, d_model->pts);
+    std::vector<int> h_n((size_t)B, (int)d_model->n);
+    OPE_CUDA_TRY(ctx, cudaMemcpyAsync(d_src.p, h_src.data(), B * sizeof(const float4*), cudaMemcpyHostToDevice, ctx->stream));
+    OPE_CUDA_TRY(ctx, cudaMemcpyAsync(d_cnt.p, h_n.data(), B * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
   }
-  OPE_CUDA_TRY(ctx, cudaMemcpyAsync(d_active.p, h_active.data(), B * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
-  tm.mark();   // [6] model sampling
-  OPE_TRY(normals_smem_batch(ctx, sampled.p + 2 * slab, d_counts.p + 2 * (size_t)B, kBCap, B, max_sp2, P.normal_k, vp, normals.p + 2 * slab));
-  tm.mark();   // [7] source normals
-  // removeNaNNormalsFromPointCloud on both fine clouds (:215-216): clouds [1] (tp2) and [2] (sp2)
-  compact_normals_batch_kernel<<<2 * B, kBThreads, 0, ctx->stream>>>(sampled.p + slab, normals.p + slab, d_counts.p + B, d_active.p, B,
-                                                                     compacted.p + slab, cnormals.p + slab, d_ccounts.p + B);
-  OPE_TRY(check_launch(ctx, "compact_normals_batch_kernel"));
+  sa.xforms = d_coarse.p; sa.xform_on = nullptr;   // the rest of sa still names the model
+  BatchClouds bc{sampled.p, normals.p, compacted.p, cnormals.p, d_counts.p, d_ccounts.p, d_flags.p, d_active.p};
+  std::vector<ope_reg_result> by_frame;
+  std::vector<double> h_fit;
   std::vector<int> h_cc;
-  OPE_TRY(download(ctx, d_ccounts.p + B, 2 * (size_t)B, h_cc));   // [0..B) tp2, [B..2B) sp2
-  // the ICP's work order: both fine clouds along their Morton curve (the raw samples' arrays are free by now)
-  const char* me = std::getenv("OPE_BATCH_MORTON");
-  const bool morton = !(me && std::atoi(me) == 0);
-  const float4* fine_pts = compacted.p;
-  const float4* fine_nrm = cnormals.p;
-  if (morton) {
-    morton_sort_batch_kernel<<<2 * B, kBThreads, 0, ctx->stream>>>(compacted.p + slab, cnormals.p + slab, d_ccounts.p + B, d_active.p, B,
-                                                                   sampled.p + slab, normals.p + slab);
-    OPE_TRY(check_launch(ctx, "morton_sort_batch_kernel"));
-    fine_pts = sampled.p; fine_nrm = normals.p;
-  }
-  std::vector<IcpBatchFrame> icp_frames;
-  std::vector<int> icp_of;
-  int max_tgt = 0;
-  for (int i = 0; i < B; ++i) {
-    if (!h_active[(size_t)i]) continue;
-    const int nt = h_cc[(size_t)i], nsrc = h_cc[(size_t)B + i];
-    if (nt < P.min_target_points || !icp_small_batch_applicable(P.icp, (size_t)nsrc, (size_t)nt)) { h_active[(size_t)i] = 0; continue; }
-    IcpBatchFrame fr;
-    fr.tgt_pts = fine_pts + slab + (size_t)i * kBCap; fr.tgt_nrm = fine_nrm + slab + (size_t)i * kBCap; fr.n_tgt = nt;
-    fr.src_pts = fine_pts + 2 * slab + (size_t)i * kBCap; fr.src_nrm = fine_nrm + 2 * slab + (size_t)i * kBCap; fr.n_src = nsrc;
-    icp_frames.push_back(fr);
-    icp_of.push_back(i);
-    max_tgt = std::max(max_tgt, nt);
-  }
-  if (icp_frames.empty()) return OPE_OK;
-  Scratch<ope_reg_result> d_icp(ctx);
-  Scratch<int> d_icp_active(ctx), d_tc(ctx), d_sc(ctx);
-  const int NI = (int)icp_frames.size();
-  OPE_TRY(d_icp.alloc(NI));
-  tm.mark();   // [8] NaN-normal compaction
-  OPE_TRY(icp_small_batch_device(ctx, P.icp, icp_frames.data(), NI, d_icp.p));
-  tm.mark();   // [9] ICP
-  // ---- getFitnessScore (:354) of every aligned pair; the ICP results are indexed by their position in icp_frames ----
-  OPE_TRY(d_fit.alloc(B));
+  OPE_TRY(fine_stage(ctx, P, B, bc, sa, h_active, by_frame, h_fit, h_cc, &tm));
   {
-    // scatter the compact ICP results back to frame order so that the fitness kernel can index by frame
-    std::vector<ope_reg_result> h_icp;
-    OPE_TRY(download(ctx, d_icp.p, (size_t)NI, h_icp));
-    std::vector<ope_reg_result> by_frame((size_t)B);
-    std::memset(by_frame.data(), 0, by_frame.size() * sizeof(ope_reg_result));
-    for (int j = 0; j < NI; ++j) by_frame[(size_t)icp_of[(size_t)j]] = h_icp[(size_t)j];
-    OPE_CUDA_TRY(ctx, cudaMemcpyAsync(d_fine.p, by_frame.data(), (size_t)B * sizeof(ope_reg_result), cudaMemcpyHostToDevice, ctx->stream));
-    OPE_CUDA_TRY(ctx, cudaMemcpyAsync(d_active.p, h_active.data(), B * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
-    OPE_TRY(fitness_batch_device(ctx, fine_pts + slab, d_ccounts.p + B, fine_pts + 2 * slab, d_ccounts.p + 2 * (size_t)B, kBCap, B, max_tgt,
-                                 d_fine.p, d_active.p, d_fit.p));
-    tm.mark();   // [10] fitness
     std::vector<ope_reg_result> h_coarse;
-    std::vector<double> h_fit;
     OPE_TRY(download(ctx, d_coarse.p, (size_t)B, h_coarse));
-    OPE_TRY(download(ctx, d_fit.p, (size_t)B, h_fit));   // also orders the stack vectors above after their copies
     // ---- estimateFinalPose (:383-448): finalPose = rigidmodelPose * (coarse * fine) ----
     for (int i = 0; i < B; ++i) {
       if (!h_active[(size_t)i]) continue;

@@ -307,19 +307,23 @@ static constexpr int kFkMaxK = 16;
 // blockIdx.z = frame: targets ftgt + z * stride * dim, counts[z] rows (counts null: nt rows); every frame answers the same nq
 // queries (the rows qlist lists, null: 0 .. nq-1). Partial lists at ((z * nq + qi) * splits + y) * k; splits past a frame's end
 // produce empty lists.
+// frame f (blockIdx.z): targets ftgt + f * stride * dim (counts[f] rows, or nt), queries fqry + f * qstride * dim (qcounts[f] rows,
+// or nq); qstride 0: every frame asks the same queries
 __global__ void feature_knn_kernel(const float* __restrict__ ftgt, int nt, const int* __restrict__ counts, int stride,
-                                   const float* __restrict__ fqry, int nq, int dim, int k, int t_per_split, const int* __restrict__ qlist,
-                                   int* __restrict__ part_idx, float* __restrict__ part_d2) {
+                                   const float* __restrict__ fqry, int nq, int qstride, const int* __restrict__ qcounts, int dim, int k,
+                                   int t_per_split, const int* __restrict__ qlist, int* __restrict__ part_idx, float* __restrict__ part_d2) {
   extern __shared__ float tile[];  // kFkTile * dim
   const int frame = blockIdx.z;
   if (counts) nt = counts[frame];
   const float* ft = ftgt + (size_t)frame * stride * dim;
+  const float* fq = fqry + (size_t)frame * qstride * dim;
+  const int nqf = qcounts ? qcounts[frame] : nq;
   const int qi = blockIdx.x * kFkQueries + threadIdx.x;   // position in the work list (nq entries)
-  const int qsrc = (qi < nq && qlist) ? qlist[qi] : qi;    // row of fqry
+  const int qsrc = (qi < nqf && qlist) ? qlist[qi] : qi;   // row of fq
   const int t_begin = blockIdx.y * t_per_split, t_end = min(nt, t_begin + t_per_split);
   float q[kFkMaxDim];
-  if (qi < nq)
-    for (int c = 0; c < dim; ++c) q[c] = __ldg(fqry + (size_t)qsrc * dim + c);
+  if (qi < nqf)
+    for (int c = 0; c < dim; ++c) q[c] = __ldg(fq + (size_t)qsrc * dim + c);
   float bd[kFkMaxK];
   int bi[kFkMaxK];
   int cnt = 0;
@@ -328,7 +332,7 @@ __global__ void feature_knn_kernel(const float* __restrict__ ftgt, int nt, const
     __syncthreads();
     for (int e = threadIdx.x; e < tn * dim; e += blockDim.x) tile[e] = __ldg(ft + (size_t)t0 * dim + e);
     __syncthreads();
-    if (qi < nq) {
+    if (qi < nqf) {
       for (int t = 0; t < tn; ++t) {
         const float* f = tile + t * dim;
         float d = 0.0f;
@@ -343,7 +347,7 @@ __global__ void feature_knn_kernel(const float* __restrict__ ftgt, int nt, const
       }
     }
   }
-  if (qi < nq) {
+  if (qi < nqf) {
     const size_t o = (((size_t)frame * nq + qi) * gridDim.y + blockIdx.y) * k;
     for (int j = 0; j < k; ++j) { part_idx[o + j] = j < cnt ? bi[j] : -1; part_d2[o + j] = j < cnt ? bd[j] : INFINITY; }
   }
@@ -351,10 +355,10 @@ __global__ void feature_knn_kernel(const float* __restrict__ ftgt, int nt, const
 // one thread per (frame = blockIdx.y, query): the splits' lists merged into out_idx / out_d2 (optional) at row
 // frame * nq + qlist[qi] (qlist null: qi)
 __global__ void feature_knn_merge_kernel(const int* __restrict__ part_idx, const float* __restrict__ part_d2, int nq,
-                                         int splits, int k, const int* __restrict__ qlist, int* __restrict__ out_idx,
-                                         float* __restrict__ out_d2) {
+                                         const int* __restrict__ qcounts, int splits, int k, const int* __restrict__ qlist,
+                                         int* __restrict__ out_idx, float* __restrict__ out_d2) {
   const int qi = blockIdx.x * blockDim.x + threadIdx.x;
-  if (qi >= nq) return;
+  if (qi >= (qcounts ? qcounts[blockIdx.y] : nq)) return;
   const size_t row = (size_t)blockIdx.y * nq + qi;
   const size_t dst = (size_t)blockIdx.y * nq + (qlist ? qlist[qi] : qi);
   float bd[kFkMaxK];
@@ -475,10 +479,10 @@ int feature_knn_exact_device(ope_ctx* ctx, const float* d_ftgt, size_t nt, const
   OPE_TRY(pi.alloc(nq * splits * k));
   OPE_TRY(pd.alloc(nq * splits * k));
   dim3 grid(qblocks, splits);
-  feature_knn_kernel<<<grid, kFkQueries, kFkTile * dim * sizeof(float), ctx->stream>>>(d_ftgt, (int)nt, nullptr, 0, d_fqry, (int)nq,
-                                                                                        dim, k, t_per_split, d_qlist, pi.p, pd.p);
+  feature_knn_kernel<<<grid, kFkQueries, kFkTile * dim * sizeof(float), ctx->stream>>>(d_ftgt, (int)nt, nullptr, 0, d_fqry, (int)nq, 0,
+                                                                                        nullptr, dim, k, t_per_split, d_qlist, pi.p, pd.p);
   OPE_TRY(check_launch(ctx, "feature_knn_kernel"));
-  feature_knn_merge_kernel<<<div_up(nq, 128), 128, 0, ctx->stream>>>(pi.p, pd.p, (int)nq, splits, k, d_qlist, d_idx, d_d2);
+  feature_knn_merge_kernel<<<div_up(nq, 128), 128, 0, ctx->stream>>>(pi.p, pd.p, (int)nq, nullptr, splits, k, d_qlist, d_idx, d_d2);
   return check_launch(ctx, "feature_knn_merge_kernel");
 }
 
@@ -519,9 +523,11 @@ int fpfh_smem_batch(ope_ctx* ctx, const float4* pts, const float4* nrm, const in
   fpfh_batch_kernel<<<grid, kWarpsPerBlock * 32, (size_t)max_n * sizeof(float4), ctx->stream>>>(pts, d_counts, stride, r2, spfh, fpfh);
   return check_launch(ctx, "fpfh_batch_kernel");
 }
-// k nearest target descriptors (frame f: ftgt + f * stride * dim, counts[f] rows) of each of the nq shared query descriptors
+// k nearest target descriptors (frame f: ftgt + f * stride * dim, counts[f] rows) of each query descriptor of the frame
+// (fqry + f * qstride * dim, d_qcounts[f] <= nq rows; qstride 0 and d_qcounts null: the same nq queries in every frame);
+// frame f's answers at out_idx + f * nq * k
 int feature_knn_batch(ope_ctx* ctx, const float* ftgt, const int* d_counts, int stride, int frames, int max_nt, const float* fqry, int nq,
-                      int dim, int k, int* out_idx) {
+                      int qstride, const int* d_qcounts, int dim, int k, int* out_idx) {
   if (dim < 1 || dim > kFkMaxDim) return fail(ctx, OPE_ERR_INVALID, "feature dimension must be in [1, %d]", kFkMaxDim);
   if (k < 1 || k > kFkMaxK) return fail(ctx, OPE_ERR_INVALID, "feature k must be in [1, %d]", kFkMaxK);
   if (frames <= 0 || nq <= 0) return OPE_OK;
@@ -535,10 +541,10 @@ int feature_knn_batch(ope_ctx* ctx, const float* ftgt, const int* d_counts, int 
   OPE_TRY(pi.alloc((size_t)frames * nq * splits * k));
   OPE_TRY(pd.alloc((size_t)frames * nq * splits * k));
   feature_knn_kernel<<<dim3(qblocks, splits, frames), kFkQueries, kFkTile * dim * sizeof(float), ctx->stream>>>(
-      ftgt, 0, d_counts, stride, fqry, nq, dim, k, t_per_split, nullptr, pi.p, pd.p);
+      ftgt, 0, d_counts, stride, fqry, nq, qstride, d_qcounts, dim, k, t_per_split, nullptr, pi.p, pd.p);
   OPE_TRY(check_launch(ctx, "feature_knn_kernel"));
-  feature_knn_merge_kernel<<<dim3(div_up((size_t)nq, 128), frames), 128, 0, ctx->stream>>>(pi.p, pd.p, nq, splits, k, nullptr, out_idx,
-                                                                                          nullptr);
+  feature_knn_merge_kernel<<<dim3(div_up((size_t)nq, 128), frames), 128, 0, ctx->stream>>>(pi.p, pd.p, nq, d_qcounts, splits, k, nullptr,
+                                                                                          out_idx, nullptr);
   return check_launch(ctx, "feature_knn_merge_kernel");
 }
 

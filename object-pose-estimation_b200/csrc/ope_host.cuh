@@ -7,6 +7,7 @@
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
+#include <functional>
 #include <map>
 #include <mutex>
 #include <string>
@@ -71,6 +72,25 @@ struct ope_ctx {
   std::vector<ModelCacheEntry> model_cache;   // at most 4 entries, least recently used replaced (pipeline.cu)
   unsigned long long model_cache_clock = 0;
   int64_t model_cache_hits = 0, model_cache_misses = 0;
+};
+
+// PoseEstimator (D&L/include/poseestimator.h): the state one tracker carries from frame to frame
+struct ope_pose_tracker {
+  ope_ctx* ctx = nullptr;
+  ope_pose_params prm;
+  int firstTimePose = 0;           // D&L/include/poseestimator.h:50-53
+  double fitnessScoreFine = 10;
+  double alignedStrength = 0.0;
+  ope_cloud* alignedSource = nullptr;
+  ope_cloud* cloudModel = nullptr;
+  double stage_ms[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+  bool timing = true;              // per-stage CUDA-event laps (each lap synchronises); the batch path turns them off
+  // frame-invariant model side of the coarse stage (SURVEY 8f-3): the 1 cm sample of the pristine model with its normals,
+  // and its FPFH descriptors. Not owned. Used by the first call of this tracker only (the source IS the model then).
+  const ope_cloud* cache_sp = nullptr;
+  const float* cache_fs = nullptr;
+  size_t cache_model_n = 0;
+  cudaEvent_t ev0 = nullptr, ev1 = nullptr, evt0 = nullptr, evt1 = nullptr;
 };
 
 // How points are binned into cells: c = (int)floorf((p - o) * inv) - min_b, per axis.
@@ -274,7 +294,8 @@ int sacia_device(ope_ctx* ctx, const ope_cloud* src, const float* d_fsrc, const 
 
 // ---- frame-spanning launches (ope_pose_batch, batch.cu): clouds of counts[c] points at c * stride ----
 struct SaciaBatch {
-  const float4* src; int ns;                               // the shared source (the model's coarse sample)
+  const float4* src; int ns;                               // frame f's source: src + f * src_stride, src_counts[f] <= ns points
+  int src_stride; const int* src_counts;                   // (src_stride 0, src_counts null: one source of ns points for every frame)
   const float4* tgt; const int* counts; int stride;        // frame f: tgt + f * stride, counts[f] points
   const float4* tgt_scan;                                  // the same points in any order (null: tgt): what the distance scan reads
   int nr_samples, k_corr, H;
@@ -297,7 +318,7 @@ int normals_smem_batch(ope_ctx* ctx, const float4* pts, const int* d_counts, int
 int fpfh_smem_batch(ope_ctx* ctx, const float4* pts, const float4* nrm, const int* d_counts, int stride, int clouds, int max_n, float radius,
                     float* spfh, float* fpfh);
 int feature_knn_batch(ope_ctx* ctx, const float* ftgt, const int* d_counts, int stride, int frames, int max_nt, const float* fqry, int nq,
-                      int dim, int k, int* out_idx);
+                      int qstride, const int* d_qcounts, int dim, int k, int* out_idx);
 // scores hypotheses [h_begin, h_end) of every frame and writes each frame's winner to d_results: from shared memory (grid null,
 // every target <= max_nt <= 8 192 points) or, for one frame, through the target's grid index
 int sacia_batch_device(ope_ctx* ctx, const SaciaBatch& a, int frames, int max_nt, const GridView* grid, ope_reg_result* d_results);
@@ -306,10 +327,56 @@ int fitness_batch_device(ope_ctx* ctx, const float4* tgt, const int* tgt_counts,
 bool icp_small_batch_applicable(const ope_icp_params& prm, size_t n_src, size_t n_tgt);
 int icp_small_batch_device(ope_ctx* ctx, const ope_icp_params& prm, const IcpBatchFrame* frames, int n_frames, ope_reg_result* d_results);
 
+// one tracker's state commit (track_commit_kernel): the new alignedSource and the copy that replaces the source, and the dense
+// Umeyama of the model onto the source
+struct TrackCommit {
+  const float4* in; int n_in; int pre;          // points to move: through coarse first (pre = 1), then through fine
+  float coarse[16], fine[16];
+  float4* out_aligned; float4* out_source;      // n_in points each
+  const float4* model; const float4* src; int n_model;   // moments of model[i] -> src[i], i < n_model (0: no Umeyama)
+  int nb;                                       // blocks: umeyama_blocks(n_model), or of n_in when there is no Umeyama
+};
+// the block count of umeyama_device for n pairs
+int umeyama_blocks(ope_ctx* ctx, size_t n);
+// n commits (device and host copies of the same array); d_rigid: n x 16 floats, written where n_model > 0
+int track_commit_device(ope_ctx* ctx, const TrackCommit* d_commits, const TrackCommit* h_commits, int n, float* d_rigid);
+
+// ---- batch.cu: the stages of a chunk of frames ----
+static constexpr int kBCap = 4096;        // capacity of a sampled cloud (normals / ICP shared-memory paths)
+static constexpr int kBFeatCap = 2048;    // capacity of a 1 cm sample (FPFH shared-memory path)
+struct BSampleArgs {
+  const float4* const* src;         // frame f's cloud (a shared source is the same pointer in every frame)
+  const int* counts;                // its points
+  const ope_reg_result* xforms;     // null: points as they are; else frame f's points go through xforms[f] (an identity matrix is not
+                                    // the same thing: it turns -0 into +0)
+  const int* xform_on;              // with xforms: the frames whose points are transformed (null: all)
+  const int* active;                // frames to process (null: all)
+  float inv_leaf[2];
+  int cap[2];                       // output capacity per leaf
+  float4* out[2];                   // leaf l, frame f: out[l] + f * kBCap
+  int* out_counts[2];               // leaf l: counts[f]
+  int* flags;                       // per frame: |= 1 when a sample overflowed its capacity / the voxel frame is too large
+};
+// UniformSampling of every frame's cloud at each leaf, one block per (frame, leaf): grid (frames, leaves)
+int bsample_batch(ope_ctx* ctx, const BSampleArgs& a, int frames, int leaves);
+// a chunk's sampled clouds: [0] 1 cm target, [1] 8 mm target, [2] source, each frames x kBCap points (and their normals, their
+// NaN-normal compactions); counts / ccounts: 3 x frames; flags, active: per frame
+struct BatchClouds { float4 *sampled, *normals, *compacted, *cnormals; int *counts, *ccounts, *flags, *active; };
+struct ChunkTimer;
+int fine_stage(ope_ctx* ctx, const ope_pose_params& P, int B, const BatchClouds& c, BSampleArgs sa, std::vector<int>& h_active,
+               std::vector<ope_reg_result>& by_frame, std::vector<double>& h_fit, std::vector<int>& h_cc, ChunkTimer* tm);
+// ---- batch.cu: stages a chunk's targets in one device array (see there) ----
+int stage_frames(ope_ctx* ctx, const ope_frame_input* frames, int B, std::vector<int>& h_active, std::vector<int>& h_off,
+                 std::vector<int>& h_cnt, Scratch<float4>& clusters, Scratch<const float4*>& d_src, size_t* total_out);
+
 // ---- batch.cu: one chunk of frames of ope_pose_batch through the frame-spanning launches; done[i] = 1 where frame i was finished ----
 int pose_batch_chunk(ope_ctx* ctx, const ope_pose_params& P, const ope_cloud* d_model, const ope_cloud* sp, const float* d_fs, const Mat4& rigid,
                      const ope_frame_input* frames, size_t n_frames, const ope_rng_table* tables, ope_pose_result* results, char* done,
                      const std::atomic<size_t>* tables_ready, size_t tables_needed);
+
+// ---- pipeline.cu: the lanes of the frame-spanning batches (see there) ----
+int run_chunks_on_lanes(ope_ctx* ctx, size_t n, const std::atomic<int>* stop,
+                        const std::function<int(ope_ctx*, size_t, size_t, size_t)>& run_chunk);
 
 // ---- p2plane.cu: TransformationEstimationPointToPlaneLLS / ...PointToPlane (Levenberg-Marquardt) ----
 int point_to_plane_device(ope_ctx* ctx, const float4* src, const float4* tgt, const float4* tgt_n, const int* d_is, const int* d_it,

@@ -88,8 +88,7 @@ __global__ void moments_kernel(const float4* __restrict__ src, const float4* __r
   block_reduce_store<kMomentAcc>(acc, smem, partials + (size_t)blockIdx.x * kMomentAcc);
 }
 // one warp per accumulator (lanes stride over the blocks, fixed shuffle tree), then one thread runs the 3x3 Umeyama
-__global__ void umeyama_final_kernel(const double* __restrict__ partials, int nblocks, float* __restrict__ out16,
-                                     const float4* __restrict__ tgt) {
+__device__ __forceinline__ void umeyama_final(const double* __restrict__ partials, int nblocks, float* __restrict__ out16, const float4* __restrict__ tgt) {
   __shared__ double acc[kMomentAcc];
   const int a = threadIdx.x >> 5, lane = threadIdx.x & 31;
   if (a < kMomentAcc) {
@@ -107,6 +106,55 @@ __global__ void umeyama_final_kernel(const double* __restrict__ partials, int nb
     umeyama_from_moments(acc, T, o[0], o[1], o[2]);
     for (int i = 0; i < 16; ++i) out16[i] = T.m[i];
   }
+}
+__global__ void umeyama_final_kernel(const double* __restrict__ partials, int nblocks, float* __restrict__ out16,
+                                     const float4* __restrict__ tgt) {
+  umeyama_final(partials, nblocks, out16, tgt);
+}
+
+// The state commit of a tracker step (ope_pose_tracker_step_batch), blockIdx.y = tracker, one read of its big clouds:
+//   out_aligned = out_source = fine(coarse(in)) (re-coarse; rounded to float after each transform, as two transform_kernel
+//                              passes) or fine(in) (tracking)
+//   the moments of the dense Umeyama model -> source with umeyama_device's shape: c.nb blocks, the same grid-stride loop, the
+//   same block reduction, so that track_umeyama_final_kernel returns its bits
+__global__ void __launch_bounds__(kRedThreads) track_commit_kernel(const TrackCommit* __restrict__ commits, double* __restrict__ partials) {
+  __shared__ double smem[(kRedThreads / 32) * kMomentAcc];
+  const TrackCommit& c = commits[blockIdx.y];
+  if ((int)blockIdx.x >= c.nb) return;
+  const int stride = c.nb * kRedThreads;
+  Mat4 C, F;
+  for (int i = 0; i < 16; ++i) { C.m[i] = c.coarse[i]; F.m[i] = c.fine[i]; }
+  for (int i = blockIdx.x * kRedThreads + threadIdx.x; i < c.n_in; i += stride) {
+    float4 p = __ldg(c.in + i);
+    if (c.pre) { float4 q = p; xform_point(C, p.x, p.y, p.z, q.x, q.y, q.z); p = q; }
+    float4 o = p;
+    xform_point(F, p.x, p.y, p.z, o.x, o.y, o.z);
+    c.out_aligned[i] = o;
+    c.out_source[i] = o;
+  }
+  if (c.n_model == 0) return;
+  double acc[kMomentAcc];
+  for (int a = 0; a < kMomentAcc; ++a) acc[a] = 0.0;
+  double o[3];
+  { const float4 t0 = __ldg(c.src); moment_origin(t0.x, t0.y, t0.z, o[0], o[1], o[2]); }
+  for (int i = blockIdx.x * kRedThreads + threadIdx.x; i < c.n_model; i += stride) {
+    const float4 s = __ldg(c.model + i);
+    const float4 t = __ldg(c.src + i);
+    const double sv[3] = {(double)s.x - o[0], (double)s.y - o[1], (double)s.z - o[2]};
+    const double tv[3] = {(double)t.x - o[0], (double)t.y - o[1], (double)t.z - o[2]};
+    acc[0] += 1.0;
+    acc[1] += sv[0]; acc[2] += sv[1]; acc[3] += sv[2];
+    acc[4] += tv[0]; acc[5] += tv[1]; acc[6] += tv[2];
+    for (int cc = 0; cc < 3; ++cc)
+      for (int r = 0; r < 3; ++r) acc[7 + cc * 3 + r] += tv[r] * sv[cc];
+  }
+  block_reduce_store<kMomentAcc>(acc, smem, partials + ((size_t)blockIdx.y * gridDim.x + blockIdx.x) * kMomentAcc);
+}
+__global__ void track_umeyama_final_kernel(const TrackCommit* __restrict__ commits, const double* __restrict__ partials, int max_nb,
+                                           float* __restrict__ out16) {
+  const TrackCommit& c = commits[blockIdx.x];
+  if (c.n_model == 0) return;
+  umeyama_final(partials + (size_t)blockIdx.x * max_nb * kMomentAcc, c.nb, out16 + (size_t)blockIdx.x * 16, c.src);
 }
 
 // fitness: sum of NN-1 squared distances <= max_range of the transformed source (double), plus the count.
@@ -1455,12 +1503,18 @@ static constexpr int kSaciaScoreThreads = 128;   // points per early-exit check:
 
 // The scoring kernel's work order of the source: along the Morton curve of its bounding box, so that the 32 points of a warp are
 // neighbours (the coarse sample arrives in voxel-key order: rows across the whole model). .w carries the original index: the terms
-// are stored — and finally summed — in the original order. One block; more than kSaciaOrderMax points keep their order.
+// are stored — and finally summed — in the original order. One block per source (frame f's at out + f * out_stride); more than
+// kSaciaOrderMax points keep their order.
 static constexpr int kSaciaOrderMax = 4096;
-__global__ void __launch_bounds__(kSaciaThreads) sacia_source_order_kernel(const float4* __restrict__ src, int n, float4* __restrict__ out) {
+__global__ void __launch_bounds__(kSaciaThreads) sacia_source_order_kernel(SaciaBatch a, int out_stride, float4* __restrict__ out_all) {
   __shared__ unsigned long long keys[kSaciaOrderMax];
   __shared__ float red[6][kSaciaThreads / 32];
   __shared__ float box[6];
+  const int f = blockIdx.x;
+  if (a.src_stride && !a.active[f]) return;
+  const float4* src = a.src + (size_t)f * a.src_stride;
+  const int n = a.src_counts ? a.src_counts[f] : a.ns;
+  float4* out = out_all + (size_t)f * out_stride;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   if (n > kSaciaOrderMax) {
     for (int i = tid; i < n; i += kSaciaThreads) { float4 p = __ldg(src + i); p.w = __int_as_float(i); out[i] = p; }
@@ -1532,11 +1586,12 @@ __global__ void __launch_bounds__(128) sacia_transform_batch_kernel(SaciaBatch a
   const int* samples = a.samples + ((size_t)f * a.H + h) * a.nr_samples;
   const int* picks = a.picks + ((size_t)f * a.H + h) * a.nr_samples;
   const int* knn = a.knn_idx + (size_t)f * a.ns * a.k_corr;
+  const float4* src = a.src + (size_t)f * a.src_stride;
   for (int j = 0; j < a.nr_samples; ++j) {
     const int si = samples[j];
     int ti = knn[(size_t)si * a.k_corr + picks[j]];
     if (ti < 0) ti = knn[(size_t)si * a.k_corr];  // fewer than k target features
-    const float4 sp = __ldg(a.src + si), tp = __ldg(tgt + ti);
+    const float4 sp = __ldg(src + si), tp = __ldg(tgt + ti);
     const double sv[3] = {sp.x, sp.y, sp.z}, tv[3] = {tp.x, tp.y, tp.z};
     acc[0] += 1.0;
     for (int k = 0; k < 3; ++k) { acc[1 + k] += sv[k]; acc[4 + k] += tv[k]; }
@@ -1613,6 +1668,8 @@ __global__ void __launch_bounds__(kSaciaScoreThreads) sacia_score_batch_kernel(S
   float4* ghi = glo + n_groups;
   float* terms = reinterpret_cast<float*>(ghi + n_groups);
   unsigned short* seed = reinterpret_cast<unsigned short*>(terms + a.ns);
+  const int ns = a.src_counts ? a.src_counts[f] : a.ns;
+  const float4* src_scan = a.src_scan + (a.src_stride ? (size_t)f * a.ns : 0);
   __shared__ Mat4 T;
   __shared__ float wpart[2][kSaciaScoreThreads / 32];
   __shared__ float s_best[2];
@@ -1651,15 +1708,15 @@ __global__ void __launch_bounds__(kSaciaScoreThreads) sacia_score_batch_kernel(S
     float run = 0.0f;
     bool stop = false;
     int chunk = 0;
-    const float shrink = 1.0f - 4.0f * (float)(a.ns + 32) * 5.97e-8f;   // twice the bound 2 n 2^-24 on the gap between two summation orders
-    for (int base = 0; base < a.ns; base += kSaciaScoreThreads, ++chunk) {
+    const float shrink = 1.0f - 4.0f * (float)(ns + 32) * 5.97e-8f;   // twice the bound 2 n 2^-24 on the gap between two summation orders
+    for (int base = 0; base < ns; base += kSaciaScoreThreads, ++chunk) {
       const int i = base + tid;
       float term = 0.0f;
       float x = 0.0f, y = 0.0f, z = 0.0f;
       bool search = false;
       int orig = 0;
-      if (i < a.ns) {
-        const float4 p = __ldg(a.src_scan + i);
+      if (i < ns) {
+        const float4 p = __ldg(src_scan + i);
         orig = __float_as_int(p.w);
         xform_point(M, p.x, p.y, p.z, x, y, z);
         term = 1.0f;
@@ -1706,7 +1763,7 @@ __global__ void __launch_bounds__(kSaciaScoreThreads) sacia_score_batch_kernel(S
         }
       }
       if (search && best <= a.threshold) term = best / a.threshold;
-      if (i < a.ns) terms[orig] = term;
+      if (i < ns) terms[orig] = term;
       float part = term;
 #pragma unroll
       for (int o = 16; o > 0; o >>= 1) part += __shfl_xor_sync(full, part, o);
@@ -1722,7 +1779,7 @@ __global__ void __launch_bounds__(kSaciaScoreThreads) sacia_score_batch_kernel(S
       float error = INFINITY;
       if (!stop) {
         error = 0.0f;
-        for (int j = 0; j < a.ns; ++j) error += terms[j];
+        for (int j = 0; j < ns; ++j) error += terms[j];
         atomicMin(frame_best, __float_as_uint(error));   // errors are >= 0: the bit pattern orders like the value
       }
       a.errors[(size_t)f * a.H + h] = error;
@@ -1799,7 +1856,7 @@ int transform_device(ope_ctx* ctx, const ope_cloud* in, const Mat4& T, ope_cloud
 
 int umeyama_device(ope_ctx* ctx, const float4* src, const float4* tgt, const int* d_isrc, const int* d_itgt, size_t n,
                    float T[16]) {
-  const int nb = (int)std::min<size_t>(std::max<size_t>(1, (n + kRedThreads - 1) / kRedThreads), (size_t)ctx->sm_count * 4);
+  const int nb = umeyama_blocks(ctx, n);
   Scratch<double> partials(ctx);
   Scratch<float> out(ctx);
   OPE_TRY(partials.alloc((size_t)nb * kMomentAcc));
@@ -1812,6 +1869,21 @@ int umeyama_device(ope_ctx* ctx, const float4* src, const float4* tgt, const int
   OPE_TRY(read_back(ctx, out.p, 16 * sizeof(float), &h));
   std::memcpy(T, h, 16 * sizeof(float));
   return OPE_OK;
+}
+
+int umeyama_blocks(ope_ctx* ctx, size_t n) {
+  return (int)std::min<size_t>(std::max<size_t>(1, (n + kRedThreads - 1) / kRedThreads), (size_t)ctx->sm_count * 4);
+}
+int track_commit_device(ope_ctx* ctx, const TrackCommit* d_commits, const TrackCommit* h_commits, int n, float* d_rigid) {
+  if (n <= 0) return OPE_OK;
+  int max_nb = 1;
+  for (int i = 0; i < n; ++i) max_nb = std::max(max_nb, h_commits[i].nb);
+  Scratch<double> partials(ctx);
+  OPE_TRY(partials.alloc((size_t)n * max_nb * kMomentAcc));
+  track_commit_kernel<<<dim3(max_nb, n), kRedThreads, 0, ctx->stream>>>(d_commits, partials.p);
+  OPE_TRY(check_launch(ctx, "track_commit_kernel"));
+  track_umeyama_final_kernel<<<n, 32 * kMomentAcc, 0, ctx->stream>>>(d_commits, partials.p, max_nb, d_rigid);
+  return check_launch(ctx, "track_umeyama_final_kernel");
 }
 
 int fitness_device(ope_ctx* ctx, const ope_cloud* src, const ope_cloud* tgt, const Mat4& T, double max_range, double* out) {
@@ -2525,7 +2597,7 @@ int sacia_batch_device(ope_ctx* ctx, const SaciaBatch& a_in, int frames, int max
   if (frames <= 0 || a.H <= 0) return OPE_OK;
   if (a.nr_samples < 1 || a.nr_samples > kSaciaMaxSamples || a.k_corr < 1 || a.k_corr > 16) return fail(ctx, OPE_ERR_INVALID, "bad SAC-IA parameters");
   if (a.h_begin < 0 || a.h_end > a.H || a.h_begin > a.h_end) return fail(ctx, OPE_ERR_INVALID, "bad SAC-IA hypothesis range");
-  if (grid && frames != 1) return fail(ctx, OPE_ERR_INVALID, "the grid SAC-IA scorer takes one frame");
+  if (grid && (frames != 1 || a.src_counts)) return fail(ctx, OPE_ERR_INVALID, "the grid SAC-IA scorer takes one frame");
   if (!grid && max_nt > kSaciaSmemMaxTargets) return fail(ctx, OPE_ERR_CAPACITY, "batched SAC-IA: target larger than the shared-memory path");
   { const char* e = std::getenv("OPE_SACIA_EARLY_EXIT"); if (e && std::atoi(e) == 0) a.early_exit = 0; }
   const int nh = a.h_end - a.h_begin;
@@ -2547,9 +2619,10 @@ int sacia_batch_device(ope_ctx* ctx, const SaciaBatch& a_in, int frames, int max
     OPE_TRY(check_launch(ctx, "sacia_kernel"));
   } else if (nh > 0) {
     OPE_TRY(seed_tab.alloc((size_t)frames * kSeedCells)); OPE_TRY(seed_geo.alloc((size_t)frames)); OPE_TRY(best_bits.alloc((size_t)frames));
-    OPE_TRY(src_scan.alloc((size_t)a.ns));
+    const int sources = a.src_stride ? frames : 1;
+    OPE_TRY(src_scan.alloc((size_t)sources * a.ns));
     a.seed_tab = seed_tab.p; a.seed_geo = seed_geo.p; a.best_bits = best_bits.p; a.src_scan = src_scan.p;
-    sacia_source_order_kernel<<<1, kSaciaThreads, 0, ctx->stream>>>(a.src, a.ns, src_scan.p);
+    sacia_source_order_kernel<<<sources, kSaciaThreads, 0, ctx->stream>>>(a, a.ns, src_scan.p);
     OPE_TRY(check_launch(ctx, "sacia_source_order_kernel"));
     const size_t nt8 = ((size_t)max_nt + 7) & ~(size_t)7, bytes = sacia_score_bytes(max_nt, a.ns);
     // every block of a frame stages its target and finds the same box; a few frames split the cells over more blocks

@@ -29,7 +29,7 @@ EXPORTS = [
     "ope_normals_knn", "ope_fpfh", "ope_feature_knn",
     "ope_umeyama", "ope_point_to_plane", "ope_fitness", "ope_correspondences", "ope_icp_align", "ope_icp_align_fixed", "ope_sacia_align", "ope_sacia_align_sharded",
     "ope_comm_unique_id", "ope_comm_nccl_version", "ope_comm_create", "ope_comm_destroy", "ope_comm_rank", "ope_comm_world", "ope_sacia_draw",
-    "ope_pose_tracker_create", "ope_pose_tracker_destroy", "ope_pose_estimate_final", "ope_pose_estimate_final_device", "ope_pose_batch",
+    "ope_pose_tracker_create", "ope_pose_tracker_destroy", "ope_pose_estimate_final", "ope_pose_estimate_final_device", "ope_pose_batch", "ope_pose_tracker_step_batch",
     "ope_pose_stage_ms", "ope_pose_batch_stage_ms", "ope_icp_params_default", "ope_sacia_params_default", "ope_pose_params_default",
     "ope_scene_params_default", "ope_scene_batch_create", "ope_scene_batch_frame", "ope_scene_batch_destroy", "ope_scene_pose_batch",
 ]
@@ -437,6 +437,26 @@ class Context:
                                   C.c_size_t(n), tb, int(workers), res, status)
         st = np.array(list(status)[:n], np.int32)
         self._chk(rc)
+        return [res[i] for i in range(n)], st
+
+    def pose_track_batch(self, trackers, sources, targets, tables=None):
+        """Advance each PoseTracker by one frame (ope_pose_tracker_step_batch): trackers[i] with its device Cloud sources[i]
+        (its handle is replaced in place, as estimate_final_device does) against targets[i] (host array or Cloud). Returns
+        (list of PoseResult, status array); a tracker that failed has its code in status, a failure of the call itself raises."""
+        n = len(trackers)
+        assert len(sources) == n and len(targets) == n
+        arr, keep = self._frame_inputs(targets)
+        th = (C.c_void_p * max(n, 1))(*[t.h for t in trackers])
+        sh = (C.c_void_p * max(n, 1))(*[s.h for s in sources])
+        res = (T.PoseResult * max(n, 1))()
+        status = (C.c_int32 * max(n, 1))()
+        tb = None if tables is None else (T.RngTable * n)(*tables)
+        rc = lib().ope_pose_tracker_step_batch(self.h, th, sh, arr, C.c_size_t(n), tb, res, status)
+        for i, s in enumerate(sources):
+            s.h = C.c_void_p(sh[i])
+        st = np.array(list(status)[:n], np.int32)
+        if rc != 0 and not (st == rc).any():
+            self._chk(rc)
         return [res[i] for i in range(n)], st
 
     # ---- registration ----

@@ -201,6 +201,19 @@ def make_frame(model, frame, outlier_frac=0.0, hand=False, z_range=(0.6, 1.6)):
     return cluster_from_scene(cloud, mask), cloud, pose
 
 
+def make_sequence(model, seq, n_frames, max_deg=10.0, max_t=0.02):
+    """A tracking sequence: per frame (cluster points, organised cloud, pose), the pose random at frame 0 and then composed with
+    small_pose steps."""
+    rng = rng_for(seq, stream=5)
+    pose = random_pose(rng)
+    out = []
+    for _ in range(n_frames):
+        cloud, mask = render_scene(model, pose, rng)
+        out.append((cluster_from_scene(cloud, mask), cloud, pose))
+        pose = small_pose(rng, max_deg, max_t) @ pose
+    return out
+
+
 def icp_pair(n=50000, seed=0, model=None, max_deg=10.0, max_t=0.02, sigma=0.001, outlier_frac=0.10):
     """C2: target = n model-surface points, source = an independent n-sample under a small perturbation,
     sigma = 1 mm noise, 10 % of the source replaced by outliers in the (inflated) bounding box."""
