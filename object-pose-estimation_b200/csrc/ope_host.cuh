@@ -195,6 +195,16 @@ inline int check_launch(ope_ctx* ctx, const char* what) {
   return OPE_OK;
 }
 
+// copy n elements from device to a host vector and wait
+template <typename T>
+int download(ope_ctx* ctx, const T* d, size_t n, std::vector<T>& h) {
+  h.resize(n);
+  if (n == 0) return OPE_OK;
+  OPE_CUDA_TRY(ctx, cudaMemcpyAsync(h.data(), d, n * sizeof(T), cudaMemcpyDeviceToHost, ctx->stream));
+  OPE_CUDA_TRY(ctx, stream_sync(ctx));
+  return OPE_OK;
+}
+
 // copy `bytes` from device to the pinned staging buffer and wait; returns the host pointer
 inline int read_back(ope_ctx* ctx, const void* dsrc, size_t bytes, void** host) {
   if (bytes > ctx->pinned_bytes) return fail(ctx, OPE_ERR_INVALID, "read_back larger than staging buffer");
@@ -357,22 +367,30 @@ struct BSampleArgs {
   int* out_counts[2];               // leaf l: counts[f]
   int* flags;                       // per frame: |= 1 when a sample overflowed its capacity / the voxel frame is too large
 };
-// UniformSampling of every frame's cloud at each leaf, one block per (frame, leaf): grid (frames, leaves)
-int bsample_batch(ope_ctx* ctx, const BSampleArgs& a, int frames, int leaves);
-// a chunk's sampled clouds: [0] 1 cm target, [1] 8 mm target, [2] source, each frames x kBCap points (and their normals, their
-// NaN-normal compactions); counts / ccounts: 3 x frames; flags, active: per frame
-struct BatchClouds { float4 *sampled, *normals, *compacted, *cnormals; int *counts, *ccounts, *flags, *active; };
-struct ChunkTimer;
-int fine_stage(ope_ctx* ctx, const ope_pose_params& P, int B, const BatchClouds& c, BSampleArgs sa, std::vector<int>& h_active,
-               std::vector<ope_reg_result>& by_frame, std::vector<double>& h_fit, std::vector<int>& h_cc, ChunkTimer* tm);
-// ---- batch.cu: stages a chunk's targets in one device array (see there) ----
-int stage_frames(ope_ctx* ctx, const ope_frame_input* frames, int B, std::vector<int>& h_active, std::vector<int>& h_off,
-                 std::vector<int>& h_cnt, Scratch<float4>& clusters, Scratch<const float4*>& d_src, size_t* total_out);
-
-// ---- batch.cu: one chunk of frames of ope_pose_batch through the frame-spanning launches; done[i] = 1 where frame i was finished ----
-int pose_batch_chunk(ope_ctx* ctx, const ope_pose_params& P, const ope_cloud* d_model, const ope_cloud* sp, const float* d_fs, const Mat4& rigid,
-                     const ope_frame_input* frames, size_t n_frames, const ope_rng_table* tables, ope_pose_result* results, char* done,
-                     const std::atomic<size_t>* tables_ready, size_t tables_needed);
+// ---- batch.cu: one chunk of frames through the frame-spanning stages (ope_pose_batch, ope_pose_tracker_step_batch) ----
+// Per frame i < B: what the caller fills in, what the table hook sees and sets, and what the chunk leaves for the active frames.
+struct PoseChunk {
+  const ope_frame_input* targets = nullptr;
+  size_t first = 0;                          // the chunk's first frame in the call (messages)
+  std::vector<int> active;                   // in: frames that try the fast path; out: frames finished here
+  std::vector<int> coarse;                   // frames that run SAC-IA (empty: every frame)
+  // SAC-IA's source: one cloud with its FPFH for every frame (src_pts, src_fpfh, src_n), or per frame a cloud (src_clouds,
+  // src_cloud_n) that the chunk samples at the coarse leaf and describes itself
+  const float4* src_pts = nullptr; const float* src_fpfh = nullptr; int src_n = 0;
+  std::vector<const float4*> src_clouds; std::vector<int> src_cloud_n;
+  std::vector<const float4*> fine_src; std::vector<int> fine_n;   // the fine stage's source (moved by the coarse pose after SAC-IA)
+  // the table hook runs once per chunk, before SAC-IA: `active` and `n_src_coarse` are final (it may clear `active` to finish
+  // nothing), a per-frame source sample is at src_samples + i * kBCap (device); it points tables[i] at each SAC-IA frame's table
+  const float4* src_samples = nullptr;
+  std::vector<const ope_rng_table*> tables;
+  std::vector<ope_reg_result> coarse_res, fine;
+  std::vector<double> fitness;
+  std::vector<int> n_src_coarse, n_tgt_coarse, n_src_fine, n_tgt_fine;
+  bool ran_coarse(int i) const { return coarse.empty() || coarse[(size_t)i]; }
+};
+int pose_chunk(ope_ctx* ctx, const ope_pose_params& P, int B, PoseChunk& c, const std::function<int(PoseChunk&)>& tables_hook);
+// estimateFinalPose's result for finished frame i: finalPose = rigid * (coarse * fine)
+ope_pose_result chunk_pose_result(const PoseChunk& c, int i, const Mat4& rigid);
 
 // ---- pipeline.cu: the lanes of the frame-spanning batches (see there) ----
 int run_chunks_on_lanes(ope_ctx* ctx, size_t n, const std::atomic<int>* stop,

@@ -527,10 +527,21 @@ int ope_pose_batch(ope_ctx* ctx, const ope_pose_params* prm, const float* model_
   std::vector<char> done(n_frames, 0);
   {
     const char* mode = std::getenv("OPE_BATCH_MODE");   // "workers": the per-frame path only (one stream per worker thread)
-    if (!(mode && std::strcmp(mode, "workers") == 0)) {
-      const int lrc = run_chunks_on_lanes(ctx, n_frames, &draw_rc, [&](ope_ctx* c, size_t f0, size_t nf, size_t) {
-        return pose_batch_chunk(c, P, model.c, sp.c, fs.p, rigid, frames + f0, nf, tables + f0, results + f0, done.data() + f0, &tables_ready,
-                                f0 + nf);
+    if (!(mode && std::strcmp(mode, "workers") == 0) && icp_small_batch_applicable(P.icp, 1, 1) && P.icp.n_rejectors >= 0) {
+      const int lrc = run_chunks_on_lanes(ctx, n_frames, &draw_rc, [&](ope_ctx* c, size_t f0, size_t nf, size_t) -> int {
+        PoseChunk ch;   // every frame's SAC-IA source is the model's cached 1 cm sample, its fine source the model under the coarse pose
+        ch.targets = frames + f0; ch.first = f0; ch.active.assign(nf, 1);
+        ch.src_pts = sp.c->pts; ch.src_fpfh = fs.p; ch.src_n = (int)sp.c->n;
+        ch.fine_src.assign(nf, model.c->pts); ch.fine_n.assign(nf, (int)model.c->n);
+        OPE_TRY(pose_chunk(c, P, (int)nf, ch, [&](PoseChunk& k) -> int {
+          // the tables of this chunk may still be on their way (drawn by the helper thread while the device worked)
+          while (tables_ready.load(std::memory_order_acquire) < f0 + nf) sched_yield();
+          for (size_t i = 0; i < nf; ++i) k.tables[i] = tables + f0 + i;
+          return OPE_OK;
+        }));
+        for (size_t i = 0; i < nf; ++i)
+          if (ch.active[i]) { results[f0 + i] = chunk_pose_result(ch, (int)i, rigid); done[f0 + i] = 1; }
+        return OPE_OK;
       });
       if (lrc != OPE_OK) {
         if (draw_rc.load() != OPE_OK) tables_ready.store(n_frames);
