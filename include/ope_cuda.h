@@ -150,12 +150,14 @@ int ope_radius_cloud(ope_ctx* ctx, const ope_cloud* tgt, const ope_cloud* qry, f
 
 /* ---- down-sampling ------------------------------------------------------------------------------------ */
 /* pcl::UniformSampling::setRadiusSearch(leaf) + compute(indices) (D&L/src/poseestimator.cpp:141-144; SURVEY A.1).
- * out_idx must hold ope_cloud_size entries; ascending voxel-key order. */
+ * out_idx must hold ope_cloud_size entries; ascending voxel-key order. OPE_ERR_GRID_TOO_LARGE when the voxel frame has more than
+ * INT_MAX voxels (PCL's int voxel index would overflow); larger frames below that are processed in windows of voxels. */
 int ope_uniform_sample(ope_ctx* ctx, const ope_cloud* cloud, float leaf, int32_t* out_idx, size_t* out_n);
 /* the same, result kept on the device as a new cloud (fused copyPointCloud) */
 int ope_uniform_sample_cloud(ope_ctx* ctx, const ope_cloud* cloud, float leaf, ope_cloud** out);
 /* pcl::VoxelGrid::setLeafSize + filter (D&L/src/processingpcd.cpp:45-59; SURVEY A.2). rgb: packed float per
- * point or NULL. out_xyz holds 3*n floats, out_rgb n floats (or NULL). */
+ * point or NULL. out_xyz holds 3*n floats, out_rgb n floats (or NULL). OPE_ERR_GRID_TOO_LARGE where PCL refuses ("Leaf size is
+ * too small for the input dataset": more than INT_MAX voxels by its own count). */
 int ope_voxel_grid(ope_ctx* ctx, const ope_cloud* cloud, const float* rgb, float lx, float ly, float lz,
                    float* out_xyz, float* out_rgb, size_t* out_n);
 

@@ -13,7 +13,9 @@
 namespace ope {
 
 static constexpr int kThreads = 256;
-static constexpr int64_t kMaxVoxelCells = (int64_t)1 << 28;
+// Dense voxel tables (UniformSampling, VoxelGrid) cover a frame in windows of at most this many consecutive voxel indices, so
+// their memory does not grow with the frame (2 GB of 64-bit keys for UniformSampling at most).
+static constexpr int64_t kVoxelWindowCells = (int64_t)1 << 28;
 
 // ============================================================================================ kernels ==
 __device__ __forceinline__ int bin_coord(float v, float o, float inv, int min_b) {
@@ -204,20 +206,26 @@ __global__ void scan_add_kernel(int* __restrict__ data, size_t n, const int* __r
 }
 
 // ---- cell build ----
-__global__ void cell_count_kernel(const float4* __restrict__ pts, int n, Binning bin, int* __restrict__ counts1) {
+// The cell build covers the cells [c0, c0 + nwin) (a window of a voxel table, see kVoxelWindowCells; all cells of a search grid):
+// points of other cells are skipped, counts1 / B / cell_start are indexed by cell - c0.
+__global__ void cell_count_kernel(const float4* __restrict__ pts, int n, Binning bin, int64_t c0, int64_t nwin,
+                                  int* __restrict__ counts1) {
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
     float4 p = __ldg(pts + i);
     if (!finite3(p.x, p.y, p.z)) continue;
-    atomicAdd(counts1 + bin_cell(bin, p.x, p.y, p.z), 1);
+    const int64_t c = bin_cell(bin, p.x, p.y, p.z) - c0;
+    if ((uint64_t)c < (uint64_t)nwin) atomicAdd(counts1 + c, 1);
   }
 }
 // B = cell_start base (see build_cells): after this kernel B[1+c] has advanced to the end of cell c.
-__global__ void cell_scatter_kernel(const float4* __restrict__ pts, int n, Binning bin, int* __restrict__ B,
+__global__ void cell_scatter_kernel(const float4* __restrict__ pts, int n, Binning bin, int64_t c0, int64_t nwin, int* __restrict__ B,
                                     float4* __restrict__ sorted) {
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
     float4 p = __ldg(pts + i);
     if (!finite3(p.x, p.y, p.z)) continue;
-    int pos = atomicAdd(B + 1 + bin_cell(bin, p.x, p.y, p.z), 1);
+    const int64_t c = bin_cell(bin, p.x, p.y, p.z) - c0;
+    if ((uint64_t)c >= (uint64_t)nwin) continue;
+    int pos = atomicAdd(B + 1 + c, 1);
     sorted[pos] = make_float4(p.x, p.y, p.z, __int_as_float(i));
   }
 }
@@ -226,11 +234,11 @@ __global__ void cell_scatter_kernel(const float4* __restrict__ pts, int n, Binni
 // thousand points (a 5 cm clustering grid over a full-resolution frame) costs its points a thousand cached loads each instead of
 // one thread a million moves.
 __global__ void cell_rank_kernel(const float4* __restrict__ scattered, const int* __restrict__ cell_start, int64_t ncells, Binning bin,
-                                 float4* __restrict__ sorted) {
+                                 int64_t c0, float4* __restrict__ sorted) {
   const int total = cell_start[ncells];
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
     const float4 v = scattered[i];
-    const int c = bin_cell(bin, v.x, v.y, v.z);
+    const int c = (int)(bin_cell(bin, v.x, v.y, v.z) - c0);
     const int b = cell_start[c], e = cell_start[c + 1];
     const int key = __float_as_int(v.w);
     int rank = 0;
@@ -306,13 +314,16 @@ __global__ void gather_kernel(const float4* __restrict__ pts, const float4* __re
   if (nrm && out_nrm) out_nrm[i] = __ldg(nrm + j);
 }
 
-// UniformSampling first pass (SURVEY A.1): per voxel keep argmin over (||p4 - ijk4||^2, index).
-__global__ void uniform_key_kernel(const float4* __restrict__ pts, int n, Binning bin, unsigned long long* __restrict__ keys) {
+// UniformSampling first pass (SURVEY A.1): per voxel of the window [c0, c0 + nwin) keep argmin over (||p4 - ijk4||^2, index);
+// keys is indexed by voxel - c0.
+__global__ void uniform_key_kernel(const float4* __restrict__ pts, int n, Binning bin, int64_t c0, int64_t nwin,
+                                   unsigned long long* __restrict__ keys) {
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
     float4 p = __ldg(pts + i);
     if (!finite3(p.x, p.y, p.z)) continue;
     int ix = (int)floorf(p.x * bin.inv[0]), iy = (int)floorf(p.y * bin.inv[1]), iz = (int)floorf(p.z * bin.inv[2]);
-    int64_t cell = ((int64_t)(iz - bin.min_b[2]) * bin.dim[1] + (iy - bin.min_b[1])) * bin.dim[0] + (ix - bin.min_b[0]);
+    int64_t cell = ((int64_t)(iz - bin.min_b[2]) * bin.dim[1] + (iy - bin.min_b[1])) * bin.dim[0] + (ix - bin.min_b[0]) - c0;
+    if ((uint64_t)cell >= (uint64_t)nwin) continue;
     float a = p.x - (float)ix, b = p.y - (float)iy, c = p.z - (float)iz;
     float d = a * a;
     d = d + b * b;
@@ -499,8 +510,9 @@ int exclusive_scan_i32(ope_ctx* ctx, int* data, size_t n) {
   return check_launch(ctx, "scan_add_kernel");
 }
 
-int build_cells(ope_ctx* ctx, const float4* pts, size_t n, const Binning& bin, int** cell_start, float4** sorted) {
-  const int64_t ncells = (int64_t)bin.dim[0] * bin.dim[1] * bin.dim[2];
+int build_cells(ope_ctx* ctx, const float4* pts, size_t n, const Binning& bin, int** cell_start, float4** sorted, int64_t c0,
+                int64_t nwin) {
+  const int64_t ncells = nwin >= 0 ? nwin : (int64_t)bin.dim[0] * bin.dim[1] * bin.dim[2] - c0;
   int* B = nullptr;
   float4* S = nullptr;
   OPE_TRY(dalloc(ctx, &B, (size_t)ncells + 2));
@@ -510,18 +522,18 @@ int build_cells(ope_ctx* ctx, const float4* pts, size_t n, const Binning& bin, i
   cudaError_t e = cudaMemsetAsync(B, 0, ((size_t)ncells + 2) * sizeof(int), ctx->stream);
   if (e != cudaSuccess) return bail(fail(ctx, OPE_ERR_CUDA, "memset failed: %s", cudaGetErrorString(e)));
   if (n > 0) {
-    cell_count_kernel<<<grid_blocks(ctx, n), kThreads, 0, ctx->stream>>>(pts, (int)n, bin, B + 1);
+    cell_count_kernel<<<grid_blocks(ctx, n), kThreads, 0, ctx->stream>>>(pts, (int)n, bin, c0, ncells, B + 1);
     if ((rc = check_launch(ctx, "cell_count_kernel")) != OPE_OK) return bail(rc);
   }
   // exclusive scan over B[1 .. ncells+1]: B[1+c] = start of cell c, B[1+ncells] = total
   if ((rc = exclusive_scan_i32(ctx, B + 1, (size_t)ncells + 1)) != OPE_OK) return bail(rc);
   if (n > 0) {
-    cell_scatter_kernel<<<grid_blocks(ctx, n), kThreads, 0, ctx->stream>>>(pts, (int)n, bin, B, S);
+    cell_scatter_kernel<<<grid_blocks(ctx, n), kThreads, 0, ctx->stream>>>(pts, (int)n, bin, c0, ncells, B, S);
     if ((rc = check_launch(ctx, "cell_scatter_kernel")) != OPE_OK) return bail(rc);
     // now B[c] = start of cell c for c in [0, ncells], B[0] = 0
     float4* R = nullptr;
     if ((rc = dalloc(ctx, &R, n)) != OPE_OK) return bail(rc);
-    cell_rank_kernel<<<grid_blocks(ctx, n), kThreads, 0, ctx->stream>>>(S, B, ncells, bin, R);
+    cell_rank_kernel<<<grid_blocks(ctx, n), kThreads, 0, ctx->stream>>>(S, B, ncells, bin, c0, R);
     rc = check_launch(ctx, "cell_rank_kernel");
     dfree(ctx, S);   // stream-ordered: released after the kernel
     S = R;
@@ -614,9 +626,6 @@ static int pcl_voxel_frame(ope_ctx* ctx, ope_cloud* c, const float leaf[3], Binn
   }
   bin->morton_bits = 0;
   *ncells = (int64_t)bin->dim[0] * bin->dim[1] * bin->dim[2];
-  if ((double)bin->dim[0] * bin->dim[1] * bin->dim[2] > (double)kMaxVoxelCells)
-    return fail(ctx, OPE_ERR_GRID_TOO_LARGE, "leaf size too small for the input: %lld voxels (cap %lld)",
-                (long long)*ncells, (long long)kMaxVoxelCells);
   return OPE_OK;
 }
 
@@ -627,39 +636,56 @@ int uniform_sample_device(ope_ctx* ctx, ope_cloud* cloud, float leaf, int** d_id
   Binning bin; int64_t ncells;
   float l3[3] = {leaf, leaf, leaf};
   OPE_TRY(pcl_voxel_frame(ctx, cloud, l3, &bin, &ncells));
+  // PCL's UniformSampling numbers the voxels with an int: beyond INT_MAX voxels its result is undefined
+  if (ncells > 0x7fffffffll)
+    return fail(ctx, OPE_ERR_GRID_TOO_LARGE, "leaf size too small for the input: %lld voxels overflow the int voxel index",
+                (long long)ncells);
+  // the frame in windows of consecutive voxel indices, each selected in ascending voxel order: the windows concatenate in
+  // ascending voxel order too. A table of at most 2^16 voxels is one window, selected in one launch.
+  const int64_t win = std::min(ncells, kVoxelWindowCells);
+  const bool single = ncells <= (1 << 16) && !std::getenv("OPE_UNIFORM_MULTI_PASS");
   Scratch<unsigned long long> keys(ctx);
   Scratch<int> flags(ctx);
-  OPE_TRY(keys.alloc((size_t)ncells));
-  OPE_CUDA_TRY(ctx, cudaMemsetAsync(keys.p, 0xff, (size_t)ncells * 8, ctx->stream));
-  uniform_key_kernel<<<grid_blocks(ctx, cloud->n), kThreads, 0, ctx->stream>>>(cloud->pts, (int)cloud->n, bin, keys.p);
-  OPE_TRY(check_launch(ctx, "uniform_key_kernel"));
-  if (ncells <= (1 << 16) && !std::getenv("OPE_UNIFORM_MULTI_PASS")) {
-    // small table: one launch selects; the index buffer is sized for the worst case (every cell / every point occupied)
-    const size_t cap = std::min<size_t>((size_t)ncells, cloud->n);
-    int* idx = nullptr;
-    OPE_TRY(dalloc(ctx, &idx, cap + 1));
-    uniform_select_single_kernel<<<1, kScan1Threads, 0, ctx->stream>>>(keys.p, (int)ncells, idx, idx + cap);
-    int rc = check_launch(ctx, "uniform_select_single_kernel");
-    void* h = nullptr;
-    if (rc == OPE_OK) rc = read_back(ctx, idx + cap, sizeof(int), &h);
-    if (rc != OPE_OK) { dfree(ctx, idx); return rc; }
-    *d_idx = idx; *out_n = (size_t) * (const int*)h;
-    return OPE_OK;
-  }
-  OPE_TRY(flags.alloc((size_t)ncells + 1));
-  OPE_CUDA_TRY(ctx, cudaMemsetAsync(flags.p + ncells, 0, sizeof(int), ctx->stream));
-  occupied_flag_u64_kernel<<<grid_blocks(ctx, (size_t)ncells), kThreads, 0, ctx->stream>>>(keys.p, ncells, flags.p);
-  OPE_TRY(check_launch(ctx, "occupied_flag_u64_kernel"));
-  OPE_TRY(exclusive_scan_i32(ctx, flags.p, (size_t)ncells + 1));
-  void* h;
-  OPE_TRY(read_back(ctx, flags.p + ncells, sizeof(int), &h));
-  const int m = *(const int*)h;
+  OPE_TRY(keys.alloc((size_t)win));
+  if (!single) OPE_TRY(flags.alloc((size_t)win + 1));
+  // the index buffer is sized for the worst case (every cell / every point occupied), plus the count of the one-launch select
+  const size_t cap = std::min<size_t>((size_t)ncells, cloud->n);
   int* idx = nullptr;
-  OPE_TRY(dalloc(ctx, &idx, (size_t)m));
-  uniform_compact_kernel<<<grid_blocks(ctx, (size_t)ncells), kThreads, 0, ctx->stream>>>(keys.p, ncells, flags.p, idx);
-  int rc = check_launch(ctx, "uniform_compact_kernel");
-  if (rc != OPE_OK) { dfree(ctx, idx); return rc; }
-  *d_idx = idx; *out_n = (size_t)m;
+  OPE_TRY(dalloc(ctx, &idx, cap + 1));
+  auto bail = [&](int rc) { dfree(ctx, idx); return rc; };
+  size_t m = 0;
+  for (int64_t c0 = 0; c0 < ncells; c0 += win) {
+    const int64_t nw = std::min(win, ncells - c0);
+    cudaError_t e = cudaMemsetAsync(keys.p, 0xff, (size_t)nw * 8, ctx->stream);
+    if (e != cudaSuccess) return bail(fail(ctx, OPE_ERR_CUDA, "memset failed: %s", cudaGetErrorString(e)));
+    uniform_key_kernel<<<grid_blocks(ctx, cloud->n), kThreads, 0, ctx->stream>>>(cloud->pts, (int)cloud->n, bin, c0, nw, keys.p);
+    int rc = check_launch(ctx, "uniform_key_kernel");
+    void* h = nullptr;
+    if (single) {
+      if (rc == OPE_OK) {
+        uniform_select_single_kernel<<<1, kScan1Threads, 0, ctx->stream>>>(keys.p, (int)nw, idx, idx + cap);
+        rc = check_launch(ctx, "uniform_select_single_kernel");
+      }
+      if (rc == OPE_OK) rc = read_back(ctx, idx + cap, sizeof(int), &h);
+      if (rc != OPE_OK) return bail(rc);
+      m = (size_t) * (const int*)h;
+      continue;
+    }
+    if (rc == OPE_OK && cudaMemsetAsync(flags.p + nw, 0, sizeof(int), ctx->stream) != cudaSuccess)
+      rc = fail(ctx, OPE_ERR_CUDA, "memset failed");
+    if (rc == OPE_OK) {
+      occupied_flag_u64_kernel<<<grid_blocks(ctx, (size_t)nw), kThreads, 0, ctx->stream>>>(keys.p, nw, flags.p);
+      rc = check_launch(ctx, "occupied_flag_u64_kernel");
+    }
+    if (rc == OPE_OK) rc = exclusive_scan_i32(ctx, flags.p, (size_t)nw + 1);
+    if (rc == OPE_OK) rc = read_back(ctx, flags.p + nw, sizeof(int), &h);
+    if (rc != OPE_OK) return bail(rc);
+    const int mw = *(const int*)h;
+    uniform_compact_kernel<<<grid_blocks(ctx, (size_t)nw), kThreads, 0, ctx->stream>>>(keys.p, nw, flags.p, idx + m);
+    if ((rc = check_launch(ctx, "uniform_compact_kernel")) != OPE_OK) return bail(rc);
+    m += (size_t)mw;
+  }
+  *d_idx = idx; *out_n = m;
   return OPE_OK;
 }
 
@@ -1046,37 +1072,45 @@ int ope_voxel_grid(ope_ctx* ctx, const ope_cloud* cloud_c, const float* rgb, flo
   }
   Binning bin; int64_t ncells;
   OPE_TRY(pcl_voxel_frame(ctx, cloud, leaf, &bin, &ncells));
-  int* cell_start = nullptr; float4* sorted = nullptr;
-  OPE_TRY(build_cells(ctx, cloud->pts, cloud->n, bin, &cell_start, &sorted));
+  // the frame in windows of consecutive voxel indices (see uniform_sample_device): centroids in ascending voxel order
+  const int64_t win = std::min(ncells, kVoxelWindowCells);
+  const size_t cap = std::min<size_t>((size_t)ncells, cloud->n);
   Scratch<int> flags(ctx);
   Scratch<float> drgb(ctx), oxyz(ctx), orgb(ctx);
-  int rc = flags.alloc((size_t)ncells + 1);
-  auto done = [&](int code) { dfree(ctx, cell_start); dfree(ctx, sorted); return code; };
-  if (rc != OPE_OK) return done(rc);
+  OPE_TRY(flags.alloc((size_t)win + 1));
+  OPE_TRY(oxyz.alloc(cap * 3));
+  OPE_TRY(orgb.alloc(cap));
   if (rgb) {
-    if ((rc = drgb.alloc(cloud->n)) != OPE_OK) return done(rc);
+    OPE_TRY(drgb.alloc(cloud->n));
     if (cudaMemcpyAsync(drgb.p, rgb, cloud->n * sizeof(float), cudaMemcpyHostToDevice, ctx->stream) != cudaSuccess)
-      return done(fail(ctx, OPE_ERR_CUDA, "rgb upload failed"));
+      return fail(ctx, OPE_ERR_CUDA, "rgb upload failed");
   }
-  cudaMemsetAsync(flags.p + ncells, 0, sizeof(int), ctx->stream);
-  occupied_flag_cells_kernel<<<grid_blocks(ctx, (size_t)ncells), kThreads, 0, ctx->stream>>>(cell_start, ncells, flags.p);
-  if ((rc = check_launch(ctx, "occupied_flag_cells_kernel")) != OPE_OK) return done(rc);
-  if ((rc = exclusive_scan_i32(ctx, flags.p, (size_t)ncells + 1)) != OPE_OK) return done(rc);
-  void* h;
-  if ((rc = read_back(ctx, flags.p + ncells, sizeof(int), &h)) != OPE_OK) return done(rc);
-  const int m = *(const int*)h;
-  if ((rc = oxyz.alloc((size_t)m * 3)) != OPE_OK) return done(rc);
-  if ((rc = orgb.alloc((size_t)m)) != OPE_OK) return done(rc);
-  voxel_centroid_kernel<<<grid_blocks(ctx, (size_t)ncells), kThreads, 0, ctx->stream>>>(
-      cell_start, ncells, sorted, rgb ? drgb.p : nullptr, flags.p, oxyz.p, orgb.p);
-  if ((rc = check_launch(ctx, "voxel_centroid_kernel")) != OPE_OK) return done(rc);
-  cudaError_t e = cudaMemcpyAsync(out_xyz, oxyz.p, (size_t)m * 3 * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream);
+  size_t m = 0;
+  for (int64_t c0 = 0; c0 < ncells; c0 += win) {
+    const int64_t nw = std::min(win, ncells - c0);
+    int* cell_start = nullptr; float4* sorted = nullptr;
+    OPE_TRY(build_cells(ctx, cloud->pts, cloud->n, bin, &cell_start, &sorted, c0, nw));
+    auto done = [&](int code) { dfree(ctx, cell_start); dfree(ctx, sorted); return code; };
+    cudaMemsetAsync(flags.p + nw, 0, sizeof(int), ctx->stream);
+    occupied_flag_cells_kernel<<<grid_blocks(ctx, (size_t)nw), kThreads, 0, ctx->stream>>>(cell_start, nw, flags.p);
+    int rc = check_launch(ctx, "occupied_flag_cells_kernel");
+    if (rc == OPE_OK) rc = exclusive_scan_i32(ctx, flags.p, (size_t)nw + 1);
+    void* h = nullptr;
+    if (rc == OPE_OK) rc = read_back(ctx, flags.p + nw, sizeof(int), &h);
+    if (rc != OPE_OK) return done(rc);
+    const int mw = *(const int*)h;
+    voxel_centroid_kernel<<<grid_blocks(ctx, (size_t)nw), kThreads, 0, ctx->stream>>>(
+        cell_start, nw, sorted, rgb ? drgb.p : nullptr, flags.p, oxyz.p + 3 * m, orgb.p + m);
+    if ((rc = done(check_launch(ctx, "voxel_centroid_kernel"))) != OPE_OK) return rc;
+    m += (size_t)mw;
+  }
+  cudaError_t e = cudaMemcpyAsync(out_xyz, oxyz.p, m * 3 * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream);
   if (e == cudaSuccess && rgb && out_rgb)
-    e = cudaMemcpyAsync(out_rgb, orgb.p, (size_t)m * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream);
+    e = cudaMemcpyAsync(out_rgb, orgb.p, m * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream);
   if (e == cudaSuccess) e = ope::stream_sync(ctx);
-  if (e != cudaSuccess) return done(fail(ctx, OPE_ERR_CUDA, "voxel grid download failed: %s", cudaGetErrorString(e)));
-  *out_n = (size_t)m;
-  return done(OPE_OK);
+  if (e != cudaSuccess) return fail(ctx, OPE_ERR_CUDA, "voxel grid download failed: %s", cudaGetErrorString(e));
+  *out_n = m;
+  return OPE_OK;
 }
 
 }  // extern "C"

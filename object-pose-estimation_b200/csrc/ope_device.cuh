@@ -412,6 +412,9 @@ OPE_HD void umeyama_small(const float* s, const float* d, int n, Mat4& out) {
 // ---- pcl::computePairFeatures + the FPFH binning, SURVEY A.5 --------------------------------------------
 // Returns the three bin indices (each in [0, 11)). Degenerate pairs are binned with f1 = f2 = f3 = 0 because
 // FPFHEstimation's wrapper ignores the free function's return value.
+// Eigen's 4-component dot of PCL's Vector4f map with w = 0, summed as (x + y) + (z + 0): the "+ 0" turns a -0 into +0, and the
+// sign of a zero decides atan2(+-0, x) = +-pi (the first or the last f1 bin) and atan2(0, +-0)
+OPE_HD float dot3w0(const float a[3], const float b[3]) { return (a[0] * b[0] + a[1] * b[1]) + (a[2] * b[2] + 0.0f); }
 OPE_HD void pair_feature_bins(float p1x, float p1y, float p1z, const float n1[3], float p2x, float p2y, float p2z,
                               const float n2[3], int& h1, int& h2, int& h3) {
   float dp[3] = {p2x - p1x, p2y - p1y, p2z - p1z};
@@ -419,8 +422,8 @@ OPE_HD void pair_feature_bins(float p1x, float p1y, float p1z, const float n1[3]
   float f4 = sqrtf(dp[0] * dp[0] + dp[1] * dp[1] + dp[2] * dp[2]);
   if (f4 != 0.0f) {
     float a[3] = {n1[0], n1[1], n1[2]}, b[3] = {n2[0], n2[1], n2[2]};
-    float angle1 = (a[0] * dp[0] + a[1] * dp[1] + a[2] * dp[2]) / f4;
-    float angle2 = (b[0] * dp[0] + b[1] * dp[1] + b[2] * dp[2]) / f4;
+    float angle1 = dot3w0(a, dp) / f4;
+    float angle2 = dot3w0(b, dp) / f4;
     if (acos_f(fabsf(angle1)) > acos_f(fabsf(angle2))) {
       for (int k = 0; k < 3; ++k) { float t = a[k]; a[k] = b[k]; b[k] = t; dp[k] *= -1; }
       f3 = -angle2;
@@ -436,8 +439,8 @@ OPE_HD void pair_feature_bins(float p1x, float p1y, float p1z, const float n1[3]
       v[0] /= v_norm; v[1] /= v_norm; v[2] /= v_norm;
       float w[3];
       cross3(a, v, w);
-      f2 = v[0] * b[0] + v[1] * b[1] + v[2] * b[2];
-      f1 = atan2_f(w[0] * b[0] + w[1] * b[1] + w[2] * b[2], a[0] * b[0] + a[1] * b[1] + a[2] * b[2]);
+      f2 = dot3w0(v, b);
+      f1 = atan2_f(dot3w0(w, b), dot3w0(a, b));
     }
   }
   const float d_pi = 1.0f / (2.0f * (float)3.14159265358979323846);

@@ -268,8 +268,10 @@ int cloud_any_grid(ope_ctx* ctx, const ope_cloud* c, GridView* out);
 // suggested cell edge for k-NN queries against this cloud (surface-density heuristic)
 float knn_cell_size(const ope_cloud* c, int k);
 int exclusive_scan_i32(ope_ctx* ctx, int* data, size_t n);
-// build cell_start (ncells+1) and the cell-sorted, index-ordered point array for an arbitrary binning
-int build_cells(ope_ctx* ctx, const float4* pts, size_t n, const Binning& bin, int** cell_start, float4** sorted);
+// build cell_start (ncells+1) and the cell-sorted, index-ordered point array for an arbitrary binning, over its cells
+// [c0, c0 + nwin) (nwin < 0: to the last cell; cell_start is indexed by cell - c0); points of other cells are left out
+int build_cells(ope_ctx* ctx, const float4* pts, size_t n, const Binning& bin, int** cell_start, float4** sorted, int64_t c0 = 0,
+                int64_t nwin = -1);
 // device-side versions used by the pipeline
 int uniform_sample_device(ope_ctx* ctx, ope_cloud* cloud, float leaf, int** d_idx, size_t* out_n);
 int gather_cloud(ope_ctx* ctx, const ope_cloud* cloud, const int* d_idx, size_t n, ope_cloud** out);
