@@ -701,8 +701,9 @@ const char* ope_version(void) { return "ope_cuda 0.1 sm_100a"; }
 int ope_ctx_create(int device, void* stream, ope_ctx** out) {
   if (!out) return OPE_ERR_INVALID;
   *out = nullptr;
-  // ope_pose_batch runs up to 64 streams; the default of 8 hardware work queues would serialise them pairwise. Only effective
-  // when this is the process's first CUDA call; a host that initialises CUDA earlier sets the variable itself (INTEGRATION.md).
+  // the frame-spanning batches run up to 8 lanes, each on its own stream, next to the caller's streams; the default of 8 hardware
+  // work queues would make them share queues. Only effective when this is the process's first CUDA call; a host that
+  // initialises CUDA earlier sets the variable itself (INTEGRATION.md).
   setenv("CUDA_DEVICE_MAX_CONNECTIONS", "32", 0);
   int count = 0;
   if (cudaGetDeviceCount(&count) != cudaSuccess || count <= 0 || device < 0 || device >= count) {

@@ -46,8 +46,8 @@ struct ope_ctx {
   int device = 0;
   cudaStream_t stream = nullptr;
   bool owns_stream = false;
-  cudaMemPool_t pool = nullptr;   // this context's own stream-ordered pool: allocations of concurrent contexts (ope_pose_batch
-                                  // workers) never wait on each other's frees
+  cudaMemPool_t pool = nullptr;   // this context's own stream-ordered pool: allocations of concurrent contexts (the lanes of
+                                  // the frame-spanning batches) never wait on each other's frees
   int sm_count = 148;
   int64_t launches = 0;
   std::string error;
@@ -57,13 +57,14 @@ struct ope_ctx {
   size_t stage_bytes = 0;
   cudaEvent_t kev[3][2] = {{nullptr, nullptr}, {nullptr, nullptr}, {nullptr, nullptr}};  // [which][begin/end] around the dominant kernels
   bool kev_valid[3] = {false, false, false};
-  std::vector<ope_ctx*> workers;  // ope_pose_batch: per-thread contexts (own stream, pool, staging), kept warm between calls
+  std::vector<ope_ctx*> workers;  // run_chunks_on_lanes: the helper lanes' contexts (own stream, pool, staging), kept warm between calls
   cudaEvent_t sync_event = nullptr;  // set: waits sleep on this cudaEventBlockingSync event instead of spinning in cudaStreamSynchronize
-                                     // (ope_pose_batch workers beyond the host's core count)
+                                     // (lanes beyond the host's core count)
   unsigned* ticket = nullptr;        // device counter, zero between kernels (see bbox_partial_kernel)
   bool sync_yield = false;           // with sync_event: poll it and sched_yield() between polls instead of sleeping
+  // both set only by pose_one_frame (pipeline.cu) for the duration of one ope_pose_batch frame outside the frame-spanning launches
   bool icp_prefer_small = false;  // small clouds: prefer the thread-per-query ICP kernel (least device time per alignment)
-  int icp_max_blocks = 0;      // > 0: cap of the cooperative icp_kernel grid (batch workers share the SMs between frames)
+  int icp_max_blocks = 0;      // > 0: cap of the cooperative icp_kernel grid (the frame shares the SMs with the other lanes)
   int64_t feature_knn_gemm_queries = 0;  // queries answered through the tcgen05 distance GEMM ...
   int64_t feature_knn_fallbacks = 0;     // ... of which the exact kernel had to re-answer (candidate set not provably complete)
   bool batch_timing = false;             // ope_pose_batch: per-stage CUDA-event laps of the frame-spanning launches
@@ -396,7 +397,7 @@ ope_pose_result chunk_pose_result(const PoseChunk& c, int i, const Mat4& rigid);
 
 // ---- pipeline.cu: the lanes of the frame-spanning batches (see there) ----
 int run_chunks_on_lanes(ope_ctx* ctx, size_t n, const std::atomic<int>* stop,
-                        const std::function<int(ope_ctx*, size_t, size_t, size_t)>& run_chunk);
+                        const std::function<int(ope_ctx*, size_t, size_t, size_t)>& run_chunk, size_t chunk_items = 0);
 
 // ---- p2plane.cu: TransformationEstimationPointToPlaneLLS / ...PointToPlane (Levenberg-Marquardt) ----
 int point_to_plane_device(ope_ctx* ctx, const float4* src, const float4* tgt, const float4* tgt_n, const int* d_is, const int* d_it,

@@ -277,10 +277,11 @@ int ope_pose_estimate_final_device(ope_pose_tracker* t, ope_cloud** source, cons
 
 namespace ope {
 // Runs run_chunk(lane context, first item, items, chunk index) over items [0, n) in chunks on a few lanes at once (OPE_BATCH_LANES,
-// OPE_BATCH_CHUNK override the defaults below). Chunks are handed out in index order. A lane stops at the first failing chunk or
-// when *stop is set; the return value is the first failure's code (its message in ctx->error). Every worker stream is idle on return.
+// OPE_BATCH_CHUNK override the defaults below; chunk_items > 0 fixes the chunk size). Chunks are handed out in index order. A
+// lane stops at the first failing chunk or when *stop is set; the return value is the first failure's code (its message in
+// ctx->error). Every worker stream is idle on return.
 int run_chunks_on_lanes(ope_ctx* ctx, size_t n, const std::atomic<int>* stop,
-                        const std::function<int(ope_ctx*, size_t, size_t, size_t)>& run_chunk) {
+                        const std::function<int(ope_ctx*, size_t, size_t, size_t)>& run_chunk, size_t chunk_items) {
   // Chunks of frames run through the frame-spanning launches on a few LANES at once: lane 0 is this thread on this context,
   // the others are helper threads on worker contexts (own stream, own scratch pool). A lane's host work between its stages
   // (staging the clusters, copying decision tables, reading counts back) then overlaps the other lanes' kernels instead of
@@ -301,8 +302,8 @@ int run_chunks_on_lanes(ope_ctx* ctx, size_t n, const std::atomic<int>* stop,
   }
   int lanes = std::max(1, std::min(le ? std::atoi(le) : std::max(2, cores - 1), 8));
   if (ctx->batch_timing) lanes = 1;   // per-stage device times are only meaningful when the stages do not share the device
-  size_t chunk = (size_t)std::max(1, ce ? std::atoi(ce) : 296);
-  if (!ce) {
+  size_t chunk = chunk_items ? chunk_items : (size_t)std::max(1, ce ? std::atoi(ce) : 296);
+  if (!ce && !chunk_items) {
     if (lanes > 1) {
       // measured (tools/bench_batch_lanes.py): many small chunks in flight beat few large ones — ~32 frames per chunk, every
       // lane the same number of chunks
@@ -383,61 +384,47 @@ extern "C" {
 // ---- batched first-frame localisation (C5) ----------------------------------------------------------------------------------
 namespace {
 
-struct BatchShared {
-  const ope_pose_params* prm;
-  const ope_cloud* model;        // full-resolution model (read-only, device)
-  const ope_cloud* sp;           // its coarse sample with normals (read-only)
-  const float* fs;               // FPFH of sp (read-only, device)
-  const ope_frame_input* frames;
-  size_t n_frames;
-  const ope_rng_table* tables;
-  ope_pose_result* results;
-  int32_t* status;
-  std::atomic<size_t> next{0};
-  int device = 0;
-  int icp_blocks = 0;
-};
-
-void batch_worker(BatchShared* S, ope_ctx* ctx, int* first_error, std::string* first_message) {
-  int rc = OPE_OK;
-  cudaSetDevice(S->device);
-  ctx->icp_max_blocks = S->icp_blocks;
-  ctx->icp_prefer_small = true;
-  for (;;) {
-    const size_t f = S->next.fetch_add(1);
-    if (f >= S->n_frames) break;
-    const ope_frame_input& in = S->frames[f];
-    ope_pose_tracker* t = nullptr;
-    rc = ope_pose_tracker_create(ctx, S->prm, &t);
-    ope_cloud* src = nullptr;
-    ope_cloud* tgt_owned = nullptr;
-    const ope_cloud* tgt = nullptr;
-    if (rc == OPE_OK) {
-      t->timing = false;
-      t->cache_sp = S->sp; t->cache_fs = S->fs; t->cache_model_n = S->model->n;
-      rc = clone_cloud(ctx, S->model, &src);
-    }
-    if (rc == OPE_OK) {
-      if (in.points) {
-        if (in.n > 0) rc = ope_cloud_upload(ctx, in.points, in.n, in.stride, in.offset, nullptr, 0, 0, &tgt_owned);
-        tgt = tgt_owned;
-      } else if (in.cloud && ((const ope_cloud*)in.cloud)->n > 0) {
-        // a private copy: the stages cache the bounding box and search grids IN the cloud they work on, and two frames may
-        // name the same caller-owned cloud (or the caller may use it from its own context meanwhile)
-        ope_cloud view = *(const ope_cloud*)in.cloud;
-        view.normals = nullptr; view.grids.clear(); view.bbox_valid = false;
-        rc = clone_cloud(ctx, &view, &tgt_owned);
-        tgt = tgt_owned;
-      }
-    }
-    if (rc == OPE_OK) rc = ope_pose_estimate_final_device(t, &src, tgt, S->tables ? &S->tables[f] : nullptr, &S->results[f]);
-    if (rc != OPE_OK && *first_error == OPE_OK) { *first_error = rc; *first_message = ctx->error; }
-    if (S->status) S->status[f] = rc;
-    if (src) ope_cloud_free(ctx, src);
-    if (tgt_owned) ope_cloud_free(ctx, tgt_owned);
-    if (t) ope_pose_tracker_destroy(t);
+// A frame outside the frame-spanning launches' envelope, on context c: what a fresh PoseEstimator returns for it, with the
+// model side (model, its 1 cm sample sp with normals, the FPFH fs of sp) borrowed from the batch.
+int pose_one_frame(ope_ctx* c, const ope_pose_params& P, const ope_cloud* model, const ope_cloud* sp, const float* fs,
+                   const ope_frame_input& in, const ope_rng_table* table, ope_pose_result* res) {
+  // The frame's ICP runs next to the other lanes' chunks: the thread-per-query kernel where it applies (least device time per
+  // alignment), and the cooperative icp_kernel's grid capped so that its blocks leave room for them. The cap is a constant:
+  // the block count orders the kernel's sums, so a frame's result must not depend on the lanes. c may be the caller's context.
+  struct IcpSettings {
+    ope_ctx* c; bool prefer_small; int max_blocks;
+    ~IcpSettings() { c->icp_prefer_small = prefer_small; c->icp_max_blocks = max_blocks; }
+  } restore{c, c->icp_prefer_small, c->icp_max_blocks};
+  c->icp_prefer_small = true;
+  c->icp_max_blocks = std::max(8, c->sm_count / 8);
+  ope_pose_tracker* t = nullptr;
+  int rc = ope_pose_tracker_create(c, &P, &t);
+  ope_cloud* src = nullptr;
+  ope_cloud* tgt_owned = nullptr;
+  const ope_cloud* tgt = nullptr;
+  if (rc == OPE_OK) {
+    t->timing = false;
+    t->cache_sp = sp; t->cache_fs = fs; t->cache_model_n = model->n;
+    rc = clone_cloud(c, model, &src);
   }
-  ope_ctx_synchronize(ctx);
+  if (rc == OPE_OK) {
+    if (in.points) {
+      if (in.n > 0) rc = ope_cloud_upload(c, in.points, in.n, in.stride, in.offset, nullptr, 0, 0, &tgt_owned);
+      tgt = tgt_owned;
+    } else if (in.cloud && ((const ope_cloud*)in.cloud)->n > 0) {
+      // a private copy: the stages cache the bounding box and search grids IN the cloud they work on, and two frames may
+      // name the same caller-owned cloud (or the caller may use it from its own context meanwhile)
+      ope_cloud view = *(const ope_cloud*)in.cloud;
+      view.normals = nullptr; view.grids.clear(); view.bbox_valid = false;
+      rc = clone_cloud(c, &view, &tgt_owned);
+      tgt = tgt_owned;
+    }
+  }
+  if (rc == OPE_OK) rc = ope_pose_estimate_final_device(t, &src, tgt, table, res);
+  if (src) ope_cloud_free(c, src);
+  if (tgt_owned) ope_cloud_free(c, tgt_owned);
+  if (t) ope_pose_tracker_destroy(t);
+  return rc;
 }
 
 }  // namespace
@@ -449,7 +436,6 @@ int ope_pose_batch(ope_ctx* ctx, const ope_pose_params* prm, const float* model_
   if (n_frames == 0) return OPE_OK;
   ope_pose_params P;
   if (prm) P = *prm; else ope_pose_params_default(&P);
-  workers = std::max(1, std::min<int>(workers > 0 ? workers : 8, (int)std::min<size_t>(n_frames, 64)));
   // ---- the frame-invariant model side, once (SURVEY 8f-3) — and kept across calls while the caller's model does not change ----
   struct Borrowed { ope_cloud* c = nullptr; } model, sp;
   struct BorrowedF { float* p = nullptr; } fs;
@@ -523,92 +509,58 @@ int ope_pose_batch(ope_ctx* ctx, const ope_pose_params* prm, const float* model_
     try { drawer = std::thread(draw_all); } catch (...) { draw_all(); }   // no thread available: draw here, as before
     tables = drawn.data();
   }
-  // ---- frame-spanning launches (batch.cu): one launch per stage for a whole chunk of frames ----
-  std::vector<char> done(n_frames, 0);
-  {
-    const char* mode = std::getenv("OPE_BATCH_MODE");   // "workers": the per-frame path only (one stream per worker thread)
-    if (!(mode && std::strcmp(mode, "workers") == 0) && icp_small_batch_applicable(P.icp, 1, 1) && P.icp.n_rejectors >= 0) {
-      const int lrc = run_chunks_on_lanes(ctx, n_frames, &draw_rc, [&](ope_ctx* c, size_t f0, size_t nf, size_t) -> int {
-        PoseChunk ch;   // every frame's SAC-IA source is the model's cached 1 cm sample, its fine source the model under the coarse pose
-        ch.targets = frames + f0; ch.first = f0; ch.active.assign(nf, 1);
-        ch.src_pts = sp.c->pts; ch.src_fpfh = fs.p; ch.src_n = (int)sp.c->n;
-        ch.fine_src.assign(nf, model.c->pts); ch.fine_n.assign(nf, (int)model.c->n);
-        OPE_TRY(pose_chunk(c, P, (int)nf, ch, [&](PoseChunk& k) -> int {
-          // the tables of this chunk may still be on their way (drawn by the helper thread while the device worked)
-          while (tables_ready.load(std::memory_order_acquire) < f0 + nf) sched_yield();
-          for (size_t i = 0; i < nf; ++i) k.tables[i] = tables + f0 + i;
-          return OPE_OK;
-        }));
-        for (size_t i = 0; i < nf; ++i)
-          if (ch.active[i]) { results[f0 + i] = chunk_pose_result(ch, (int)i, rigid); done[f0 + i] = 1; }
-        return OPE_OK;
-      });
-      if (lrc != OPE_OK) {
-        if (draw_rc.load() != OPE_OK) tables_ready.store(n_frames);
-        return lrc;
+  // ---- frame-spanning launches (batch.cu): one launch per stage for a whole chunk of frames; the frames outside their envelope
+  // (tiny / empty / oversized clusters, or every frame when the ICP parameters are outside it) are collected for a second pass ----
+  const bool fast = icp_small_batch_applicable(P.icp, 1, 1) && P.icp.n_rejectors >= 0;
+  std::mutex frame_mu;
+  std::vector<size_t> rest;
+  int lrc = run_chunks_on_lanes(ctx, n_frames, &draw_rc, [&](ope_ctx* c, size_t f0, size_t nf, size_t) -> int {
+    PoseChunk ch;   // every frame's SAC-IA source is the model's cached 1 cm sample, its fine source the model under the coarse pose
+    ch.targets = frames + f0; ch.first = f0; ch.active.assign(nf, fast ? 1 : 0);
+    ch.src_pts = sp.c->pts; ch.src_fpfh = fs.p; ch.src_n = (int)sp.c->n;
+    ch.fine_src.assign(nf, model.c->pts); ch.fine_n.assign(nf, (int)model.c->n);
+    OPE_TRY(pose_chunk(c, P, (int)nf, ch, [&](PoseChunk& k) -> int {
+      // the tables of this chunk may still be on their way (drawn by the helper thread while the device worked)
+      while (tables_ready.load(std::memory_order_acquire) < f0 + nf) sched_yield();
+      for (size_t i = 0; i < nf; ++i) k.tables[i] = tables + f0 + i;
+      return OPE_OK;
+    }));
+    for (size_t i = 0; i < nf; ++i) {
+      const size_t f = f0 + i;
+      if (ch.active[i]) {
+        results[f] = chunk_pose_result(ch, (int)i, rigid);
+        if (status) status[f] = OPE_OK;
+        continue;
       }
-      if (draw_rc.load() != OPE_OK) return fail(ctx, draw_rc.load(), "selectSamples failed");
-      if (status) for (size_t f = 0; f < n_frames; ++f) if (done[f]) status[f] = OPE_OK;
+      std::lock_guard<std::mutex> lock(frame_mu);
+      rest.push_back(f);
     }
+    return OPE_OK;
+  });
+  if (lrc != OPE_OK) {
+    if (draw_rc.load() != OPE_OK) tables_ready.store(n_frames);
+    return lrc;
   }
   if (drawer.joinable()) drawer.join();
   if (draw_rc.load() != OPE_OK) return fail(ctx, draw_rc.load(), "selectSamples failed");
-  // ---- whatever the fast path did not take (tiny / empty / oversized clusters): the per-frame path, worker threads ----
-  std::vector<ope_frame_input> rest_frames;
-  std::vector<ope_rng_table> rest_tables;
-  std::vector<size_t> rest_of;
-  for (size_t f = 0; f < n_frames; ++f)
-    if (!done[f]) { rest_frames.push_back(frames[f]); rest_tables.push_back(tables[f]); rest_of.push_back(f); }
-  if (rest_frames.empty()) return OPE_OK;
-  std::vector<ope_pose_result> rest_results(rest_frames.size());
-  std::vector<int32_t> rest_status(rest_frames.size(), OPE_OK);
-  struct Scatter {   // copies the sub-batch's results back on every exit path
-    std::vector<ope_pose_result>& r; std::vector<int32_t>& st; std::vector<size_t>& of; ope_pose_result* results; int32_t* status;
-    ~Scatter() { for (size_t i = 0; i < of.size(); ++i) { results[of[i]] = r[i]; if (status) status[of[i]] = st[i]; } }
-  } scatter{rest_results, rest_status, rest_of, results, status};
-  workers = std::max(1, std::min<int>(workers, (int)rest_frames.size()));
-  OPE_TRY(ope_ctx_synchronize(ctx));   // the workers read the model side from their own streams
-  BatchShared S;
-  S.prm = &P; S.model = model.c; S.sp = sp.c; S.fs = fs.p; S.frames = rest_frames.data(); S.n_frames = rest_frames.size(); S.tables = rest_tables.data();
-  S.results = rest_results.data(); S.status = rest_status.data(); S.device = ctx->device;
-  {
-    // the fused ICP loop is a cooperative launch: its blocks must all be co-resident, so concurrent frames only overlap if
-    // each takes a share of the SMs
-    const char* e = std::getenv("OPE_BATCH_ICP_BLOCKS");
-    S.icp_blocks = e ? std::atoi(e) : std::max(8, ctx->sm_count / std::min(workers, 8));
-  }
-  std::vector<int> errs(workers, OPE_OK);
-  std::vector<std::string> msgs(workers);
-  while ((int)ctx->workers.size() < workers) {
-    ope_ctx* w = nullptr;
-    const int rc = ope_ctx_create(ctx->device, nullptr, &w);
-    if (rc != OPE_OK) return fail(ctx, rc, "worker context creation failed");
-    ctx->workers.push_back(w);
-  }
-  {
-    // more workers than host cores: their waits must sleep, not spin (OPE_BATCH_BLOCKING_SYNC=0/1 overrides)
-    const char* e = std::getenv("OPE_BATCH_BLOCKING_SYNC");
-    const int mode = e ? std::atoi(e) : (workers > (int)std::thread::hardware_concurrency() ? 2 : 0);   // 0 spin, 1 sleep, 2 poll + yield
-    const bool blocking = mode != 0;
-    for (int w = 0; w < workers; ++w) {
-      ope_ctx* c = ctx->workers[w];
-      c->sync_yield = mode == 2;
-      if (blocking && !c->sync_event) { if (cudaEventCreateWithFlags(&c->sync_event, cudaEventBlockingSync | cudaEventDisableTiming) != cudaSuccess) c->sync_event = nullptr; }
-      if (!blocking && c->sync_event) { cudaEventDestroy(c->sync_event); c->sync_event = nullptr; }
+  // ---- the collected frames through the per-frame path, one frame per chunk on the same lanes ----
+  std::sort(rest.begin(), rest.end());
+  size_t failed_frame = n_frames;   // the lowest frame that failed on the per-frame path, its code and message
+  int failed_rc = OPE_OK;
+  std::string failed_msg;
+  lrc = run_chunks_on_lanes(ctx, rest.size(), nullptr, [&](ope_ctx* c, size_t i0, size_t, size_t) -> int {
+    const size_t f = rest[i0];
+    // a frame's failure is its own: the other frames of the batch go on
+    const int rc = pose_one_frame(c, P, model.c, sp.c, fs.p, frames[f], tables + f, &results[f]);
+    if (status) status[f] = rc;
+    if (rc != OPE_OK) {
+      std::lock_guard<std::mutex> lock(frame_mu);
+      if (f < failed_frame) { failed_frame = f; failed_rc = rc; failed_msg = c->error; }
     }
-  }
-  std::vector<std::thread> pool;
-  int started = 1;
-  try {   // nothing may throw across the C ABI: if the host cannot start more threads, the ones that exist do all the work
-    for (int w = 1; w < workers; ++w) { pool.emplace_back(batch_worker, &S, ctx->workers[w], &errs[w], &msgs[w]); ++started; }
-  } catch (...) {
-  }
-  (void)started;
-  batch_worker(&S, ctx->workers[0], &errs[0], &msgs[0]);
-  for (auto& th : pool) th.join();
-  cudaSetDevice(ctx->device);
-  for (int w = 0; w < workers; ++w)
-    if (errs[w] != OPE_OK) return fail(ctx, errs[w], "batch worker %d: %s", w, msgs[w].c_str());
+    return OPE_OK;
+  }, 1);
+  if (lrc != OPE_OK) return lrc;
+  if (failed_rc != OPE_OK) return fail(ctx, failed_rc, "frame %zu: %s", failed_frame, failed_msg.c_str());
   return OPE_OK;
 }
 

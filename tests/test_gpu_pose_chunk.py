@@ -57,7 +57,7 @@ def test_pose_batch_equals_the_first_tracker_step(ctx, synth, cuda_lib, model, f
     assert all(r.ran_coarse == 1 for r in got)
     for f in range(len(frames) - 1):   # the fast path: the same chunk, bit for bit
         assert bytes(got[f]) == bytes(ref[f]), f
-    # the frame outside the envelope: ope_pose_batch's workers and the tracker step's serial loop run different ICP kernels
+    # the frame outside the envelope: ope_pose_batch's per-frame path and the tracker step's serial loop run different ICP kernels
     g, r = got[-1], ref[-1]
     assert g.n_tgt_coarse > 2048 and g.n_tgt_fine > 0
     for name in ("final_pose", "coarse_pose", "fine_pose", "rigid_model_pose"):

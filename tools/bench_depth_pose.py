@@ -12,7 +12,8 @@ Frames are 640x480 uint16 depth images of synth.make_frame scenes (depth = rint(
   * the same frames through the single-frame calls (ope_depth_to_cloud -> ope_pass_through -> ope_segment_objects_on_plane);
   * end to end from host uint16 (614 KB H2D per frame) through ope_scene_pose_batch on cluster 0, frames/s;
   * per full-frame launch (torch.profiler, a run of its own): algorithmic bytes over kernel time, share of 7.7 TB/s;
-  * the sizes of the clusters handed on; parity with the single-frame path on every frame and with the oracle on a sample.
+  * the sizes of the clusters handed on (and how many exceed the pose batch's 1 cm capacity); parity with the single-frame path
+    on every frame and with the oracle on a sample.
 """
 import argparse
 import json
@@ -100,7 +101,9 @@ def main():
         wall = time.perf_counter() - h0
         sizes0 = np.array([r.n_tgt_coarse for r in res])
         out["end_to_end"][str(n)] = {"ms": e0.elapsed_time(e1), "frames_per_sec": 1e3 * n / e0.elapsed_time(e1), "host_wall_s": wall,
-                                     "scene_ms": e0.elapsed_time(e_mid), "pose_ms": e_mid.elapsed_time(e1), "status_ok": int((st == 0).sum())}
+                                     "scene_ms": e0.elapsed_time(e_mid), "pose_ms": e_mid.elapsed_time(e1), "status_ok": int((st == 0).sum()),
+                                     # frames beyond the frame-spanning launches' 1 cm capacity: they take the per-frame path
+                                     "frames_over_2048_at_1cm": int((sizes0 > 2048).sum())}
         if n == sizes[-1]:
             cl = np.array([sb.info[f].n_clusters for f in range(n)])
             c0 = np.array([(sb.frame(f)[1] == 0).sum() if cl[f] > 0 else 0 for f in range(a.unique)])

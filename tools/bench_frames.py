@@ -9,7 +9,7 @@ the per-rank device times are max-reduced and the frame counts summed only to pr
 Scenes are generated once (64 distinct frames, cycled) outside the timed region; every frame starts a fresh tracker, so
 SAC-IA runs on every frame (the expensive first-frame path of the reference)."""
 import os
-os.environ.setdefault("CUDA_DEVICE_MAX_CONNECTIONS", "32")   # ope_pose_batch: one hardware queue per worker stream (before CUDA starts)
+os.environ.setdefault("CUDA_DEVICE_MAX_CONNECTIONS", "32")   # ope_pose_batch: one hardware queue per lane stream (before CUDA starts)
 import json, os, sys, time
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -57,15 +57,10 @@ def main():
                 src.free()
             tr.close()
 
-    # one spinning host thread per worker stream: do not oversubscribe the host cores when several ranks share a box
-    local_world = int(os.environ.get("LOCAL_WORLD_SIZE", world))
-    cores_per_rank = max(1, (os.cpu_count() or 16) // max(local_world, 1))
     workers = int(sys.argv[sys.argv.index("--workers") + 1]) if "--workers" in sys.argv else 16
-    if workers > cores_per_rank:
-        os.environ.setdefault("OPE_BATCH_BLOCKING_SYNC", "2")   # more worker threads than cores for this rank: poll + yield, do not spin
 
     def run_batch(host):
-        # ope_pose_batch: worker threads with their own streams, model side cached (SURVEY 8f-3); the decision tables are drawn
+        # ope_pose_batch: lanes with their own streams, model side cached (SURVEY 8f-3); the decision tables are drawn
         # from libc rand() in frame order inside the call
         libc.srand(1)
         inputs = [frames[f % distinct] if host else targets[f % distinct] for f in mine]
@@ -100,7 +95,7 @@ def main():
         print(json.dumps({"metric": "frames_per_sec_fpfh_sacia_icp_640x480", "n_gpus": world, "frames": n, "scaling": "strong",
                           "value": out["frames_per_s"], "e2e": out["e2e_frames_per_s"], "unit": "frames/s",
                           "config": {"workload": "C5: %d independent frames, full first-frame path, frame f -> rank f mod N" % n,
-                                     "mode": "serial trackers" if "--serial" in sys.argv else "ope_pose_batch, %d workers per GPU" % workers,
+                                     "mode": "serial trackers" if "--serial" in sys.argv else "ope_pose_batch, one call per GPU",
                                      "host_cores": os.cpu_count()}}))
     ctx.close()
     if dist is not None:

@@ -91,14 +91,14 @@ def main():
         ro, to = synth.pose_error(o_fine.reshape(4, 4).T @ o_coarse.reshape(4, 4).T, pose)
         rec_g += rg < np.deg2rad(5) and tg < 0.01
         rec_o += ro < np.deg2rad(5) and to < 0.01
-    # the same frames through ope_pose_batch (16 worker streams, model side cached, thread-per-query ICP kernel): every frame
+    # the same frames through ope_pose_batch (chunk lanes, model side cached, thread-per-query ICP kernel): every frame
     # replays the decision table a fresh PoseEstimator draws after srand(1)
     import orc_py
     orc_py.srand(1)
     sp = model[orc_py.uniform_sample(model, 0.01)]
     table = cuda_lib.rng_table(*orc_py.sacia_draw(sp, 400, 5, 5, 0.01))
     clusters = [synth.make_frame(model, 1000 + f)[0] for f, *_ in cpu]
-    ctx.pose_batch(model, clusters[:32], tables=[table] * min(32, n), workers=16)   # warm the workers
+    ctx.pose_batch(model, clusters[:32], tables=[table] * min(32, n), workers=16)   # warm the lanes
     t1 = time.perf_counter()
     bres, bstatus = ctx.pose_batch(model, clusters, tables=[table] * n, workers=16)
     batch_s = time.perf_counter() - t1
