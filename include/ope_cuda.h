@@ -138,6 +138,45 @@ void ope_scene_batch_destroy(ope_scene_batch* s);
 int ope_scene_pose_batch(const ope_scene_batch* s, const ope_pose_params* prm, const float* model_xyz, size_t n_model,
                          const int32_t* cluster, const ope_rng_table* tables, int workers, ope_pose_result* results, int32_t* status);
 
+/* pcl::compute3DCentroid of a device cloud (include/ope_pcl/filters.h): serial float sums over the finite points in index order,
+ * then each divided by (float) n; c = 0 when no point is finite. n_used (may be NULL): the number of finite points. */
+int ope_cloud_centroid(ope_ctx* ctx, const ope_cloud* cloud, float c[3], int32_t* n_used);
+/* the same for the clusters of frame f in rank order: xyz gets n_clusters x 3 floats (the whole cropped cloud, one centroid, when
+ * n_clusters == -1; none when the frame's scene status is an error); *n_out: the number of centroids written. */
+int ope_scene_batch_centroids(const ope_scene_batch* s, size_t frame, float* xyz, int32_t* n_out);
+void ope_track_params_default(ope_track_params* p);
+/* The node's cluster choice and the tracker step in one call (D&L/src/rosinterface.cpp:243-327, SURVEY 3.1 and A.0): camera i
+ * is frame i of s (n == the number of frames) with trackers[i] and its device source *sources[i]. The call equals this serial
+ * loop of public calls bit for bit, libc rand() consumption included:
+ *   - branch: a frame whose scene status is an error -> NO_SCENE (tracker and source untouched, the frame's code in status[i]);
+ *     a tracker that never completed a step (firstTimePose == 0) -> acquisition; any other -> tracking.
+ *   - tracking: m = ope_cloud_centroid(*sources[i]) (the model as last placed in the scene), c_k = the centroid of cluster k
+ *     (ope_scene_batch_centroids); the chosen cluster is the FIRST in rank order with sqrtf((dx*dx + dy*dy) + dz*dz) < gate
+ *     (float, no FMA). The tracker steps on it as ope_pose_tracker_step_batch steps it -> TRACKED. No cluster inside the gate
+ *     (n_clusters == 0 included): with reacquire the camera goes to acquisition (REACQUIRED on success), else LOST (tracker and
+ *     source untouched). The reference keeps "the cluster whose centroid is less than 5 cm from the model's"; first-in-rank rather
+ *     than nearest is this library's reading of that sentence (the reference file is not in this tree).
+ *   - acquisition: try r (r = 0, 1, ... < n_clusters, at most max_tries; one try on the whole cloud when n_clusters == -1) is a
+ *     fresh tracker with trackers[i]'s parameters on a device copy of the pristine model (trackers[i]'s cloudModel if it has one,
+ *     else *sources[i]) against cluster r, as ope_scene_pose_batch cuts it. The first try with fitness < accept_fitness ||
+ *     align_strength > accept_strength is committed: trackers[i] is then what a freshly created tracker is after
+ *     ope_pose_estimate_final_device(copy of the model, that cluster), and *sources[i] is replaced by that call's source.
+ *     No accepted try -> NOT_FOUND: tracker and source untouched, results[i] = the last try's (zero without a try).
+ *   - order (the rand() stream): rounds r = 0, 1, ...; round 0 holds every tracking camera's step and every acquiring camera's
+ *     rank-0 try (a reacquiring camera enters at round 0, after its failed gate), round r >= 1 the rank-r tries of the cameras
+ *     still searching; in a round the cameras go in index order, and the round is ONE ope_pose_tracker_step_batch call (tables
+ *     drawn from libc rand()).
+ * results / choice / status: n entries each; status[i] is the code of the step whose result is results[i] (OPE_OK for a
+ * camera that made no step, a failed try counts as not accepted). Returns OPE_OK or the first failing camera's code.
+ * Argument checks are those of ope_pose_tracker_step_batch (distinct trackers and sources, all on s's context) and n; a violation
+ * returns OPE_ERR_INVALID before anything changes. tp == NULL: ope_track_params_default. */
+int ope_scene_track_step(const ope_scene_batch* s, const ope_track_params* tp, ope_pose_tracker* const* trackers, ope_cloud** sources,
+                         size_t n, ope_pose_result* results, ope_track_choice* choice, int32_t* status);
+/* host wall time (ms) of the phases of the context's last ope_scene_track_step: out[0] centroids + gate (one launch, one
+ * read-back), out[1] commit of the accepted tries, out[2 + r] round r (cut + tracker step). *n_out: 2 + rounds; at most cap
+ * entries are written. */
+int ope_scene_track_phase_ms(const ope_ctx* ctx, double* out, int cap, int32_t* n_out);
+
 /* ---- spatial search: replaces pcl::search::KdTree / KdTreeFLANN (SURVEY A.3) -------------------------- */
 /* nearestKSearch for nq host queries; out_idx/out_d2 are nq*k, padded with -1 / +inf. k <= 32. */
 int ope_knn(ope_ctx* ctx, const ope_cloud* tgt, const void* qry, size_t nq, size_t stride, size_t offset, int k,

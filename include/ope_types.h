@@ -199,6 +199,32 @@ typedef struct ope_scene_frame {
   int32_t reserved;
 } ope_scene_frame;
 
+/* ope_scene_track_step: the cluster choice of the reference's online loop (D&L/src/rosinterface.cpp:243-327, SURVEY 3.1 and A.0);
+ * ope_track_params_default gives the values below. */
+typedef struct ope_track_params {
+  double accept_fitness;    /* 1e-4: a pose is accepted iff fitness < accept_fitness || align_strength > accept_strength */
+  double accept_strength;   /* 0.4 */
+  float gate;               /* 0.05 m: centroid distance that keeps a tracked object on a cluster */
+  int32_t max_tries;        /* acquisition tries per call; 0 = every cluster */
+  int32_t reacquire;        /* 1: a tracker with no cluster inside the gate searches again in the same call */
+} ope_track_params;
+
+/* what one camera of ope_scene_track_step did */
+enum {
+  OPE_TRACK_TRACKED = 0,    /* stepped on the first cluster inside the gate */
+  OPE_TRACK_ACQUIRED,       /* a fresh search accepted a cluster */
+  OPE_TRACK_REACQUIRED,     /* lost by the gate, then a search in the same call accepted a cluster */
+  OPE_TRACK_NOT_FOUND,      /* a search accepted no cluster */
+  OPE_TRACK_LOST,           /* no cluster inside the gate and no search (reacquire = 0) */
+  OPE_TRACK_NO_SCENE        /* the frame's scene status is an error */
+};
+typedef struct ope_track_choice {
+  int32_t mode;             /* OPE_TRACK_* */
+  int32_t cluster;          /* the rank stepped on (0 for a whole-cloud frame), -1 if none */
+  int32_t tries;            /* acquisition tries made in this call */
+  float gate_distance;      /* tracking: the distance of the chosen cluster (or of the nearest one when lost); NaN otherwise */
+} ope_track_choice;
+
 /* One frame of a batch (ope_pose_batch): the segmented scene cluster either as host points (stride/offset in BYTES as in
  * ope_cloud_upload) or, when points == NULL, as a device-resident cloud that no other call touches during the batch. */
 typedef struct ope_frame_input {

@@ -133,6 +133,19 @@ class SceneFrame(C.Structure):
                 ("iterations", C.c_int32 * 2), ("n_clusters", C.c_int32), ("reserved", C.c_int32)]
 
 
+class TrackParams(C.Structure):
+    _fields_ = [("accept_fitness", C.c_double), ("accept_strength", C.c_double), ("gate", C.c_float), ("max_tries", C.c_int32),
+                ("reacquire", C.c_int32)]
+
+
+TRACK_TRACKED, TRACK_ACQUIRED, TRACK_REACQUIRED, TRACK_NOT_FOUND, TRACK_LOST, TRACK_NO_SCENE = range(6)
+TRACK_MODES = ("tracked", "acquired", "reacquired", "not_found", "lost", "no_scene")
+
+
+class TrackChoice(C.Structure):
+    _fields_ = [("mode", C.c_int32), ("cluster", C.c_int32), ("tries", C.c_int32), ("gate_distance", C.c_float)]
+
+
 class FrameInput(C.Structure):
     _fields_ = [("points", C.c_void_p), ("n", C.c_size_t), ("stride", C.c_size_t), ("offset", C.c_size_t), ("cloud", C.c_void_p)]
 

@@ -73,6 +73,7 @@ struct ope_ctx {
   std::vector<ModelCacheEntry> model_cache;   // at most 4 entries, least recently used replaced (pipeline.cu)
   unsigned long long model_cache_clock = 0;
   int64_t model_cache_hits = 0, model_cache_misses = 0;
+  std::vector<double> track_phase_ms;   // ope_scene_track_step's last call: gate, commit, round 0, 1, ... (host wall ms)
 };
 
 // PoseEstimator (D&L/include/poseestimator.h): the state one tracker carries from frame to frame
@@ -122,6 +123,20 @@ struct ope_cloud {
   float bbox[6];               // min xyz, max xyz over finite points
   int n_finite = 0;
   std::vector<GridEntry> grids;
+};
+
+// ope_scene_batch_create's result: the cropped clouds and labels of every frame, resident on the device (segment.cu)
+struct ope_scene_batch {
+  ope_ctx* ctx = nullptr;
+  struct Frame {
+    const float4* pts = nullptr;   // n_cropped points (device, inside one of `blocks`)
+    const int* labels = nullptr;   // n_cropped labels (device)
+    ope_scene_frame info{};
+    int status = OPE_OK;
+    std::vector<int> sizes;        // point count of cluster 0, 1, ...
+  };
+  std::vector<Frame> frames;
+  std::vector<void*> blocks;       // device allocations, one pair per chunk
 };
 
 namespace ope {
@@ -398,6 +413,16 @@ ope_pose_result chunk_pose_result(const PoseChunk& c, int i, const Mat4& rigid);
 // ---- pipeline.cu: the lanes of the frame-spanning batches (see there) ----
 int run_chunks_on_lanes(ope_ctx* ctx, size_t n, const std::atomic<int>* stop,
                         const std::function<int(ope_ctx*, size_t, size_t, size_t)>& run_chunk, size_t chunk_items = 0);
+
+// ---- track.cu: ope_pose_tracker_step_batch's argument checks (targets may be null: not checked) and its body ----
+int step_batch_check(ope_ctx* ctx, ope_pose_tracker* const* trackers, ope_cloud* const* sources, const ope_frame_input* targets, size_t n);
+int tracker_step_batch(ope_ctx* ctx, ope_pose_tracker* const* trackers, ope_cloud** sources, const ope_frame_input* targets, size_t n,
+                       const ope_rng_table* tables, ope_pose_result* results, int32_t* status);
+
+// ---- segment.cu: one block per cut copies the points of pts[0 .. n) whose label is `want` (INT_MIN: every point; labels may then
+// be null) in index order to out + out_off ----
+struct SceneCut { const float4* pts; const int* labels; int n; int want; long long out_off; };
+int scene_cut_device(ope_ctx* ctx, const SceneCut* d_cuts, int n_cuts, float4* out);
 
 // ---- p2plane.cu: TransformationEstimationPointToPlaneLLS / ...PointToPlane (Levenberg-Marquardt) ----
 int point_to_plane_device(ope_ctx* ctx, const float4* src, const float4* tgt, const float4* tgt_n, const int* d_is, const int* d_it,

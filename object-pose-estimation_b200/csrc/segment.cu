@@ -540,8 +540,8 @@ __global__ void label_rest_kernel(const int* __restrict__ off, const int* __rest
   }
 }
 
-// ope_scene_pose_batch: block b copies the points of cut b whose label is `want` (INT_MIN: every point) in index order to out + out_off
-struct SceneCut { const float4* pts; const int* labels; int n; int want; long long out_off; };
+// ope_scene_pose_batch, ope_scene_track_step: block b copies the points of cut b whose label is `want` (INT_MIN: every point) in
+// index order to out + out_off
 __global__ void __launch_bounds__(1024) scene_cut_kernel(const SceneCut* __restrict__ cuts, float4* __restrict__ out) {
   __shared__ int warp_count[32];
   const SceneCut c = cuts[blockIdx.x];
@@ -561,20 +561,13 @@ __global__ void __launch_bounds__(1024) scene_cut_kernel(const SceneCut* __restr
   }
 }
 
-}  // namespace ope
+int scene_cut_device(ope_ctx* ctx, const SceneCut* d_cuts, int n_cuts, float4* out) {
+  if (n_cuts == 0) return OPE_OK;
+  scene_cut_kernel<<<(unsigned)n_cuts, 1024, 0, ctx->stream>>>(d_cuts, out);
+  return check_launch(ctx, "scene_cut_kernel");
+}
 
-struct ope_scene_batch {
-  ope_ctx* ctx = nullptr;
-  struct Frame {
-    const float4* pts = nullptr;   // n_cropped points (device, inside one of `blocks`)
-    const int* labels = nullptr;   // n_cropped labels (device)
-    ope_scene_frame info{};
-    int status = OPE_OK;
-    std::vector<int> sizes;        // point count of cluster 0, 1, ...
-  };
-  std::vector<Frame> frames;
-  std::vector<void*> blocks;       // device allocations, one pair per chunk
-};
+}  // namespace ope
 
 namespace {
 
@@ -1191,8 +1184,7 @@ int ope_scene_pose_batch(const ope_scene_batch* s, const ope_pose_params* prm, c
   OPE_TRY(buf.alloc(total)); OPE_TRY(d_cuts.alloc(cuts.size()));
   if (!cuts.empty()) {
     OPE_TRY(upload(ctx, d_cuts.p, cuts));
-    scene_cut_kernel<<<(unsigned)cuts.size(), 1024, 0, ctx->stream>>>(d_cuts.p, buf.p);
-    OPE_TRY(check_launch(ctx, "scene_cut_kernel"));
+    OPE_TRY(scene_cut_device(ctx, d_cuts.p, (int)cuts.size(), buf.p));
   }
   OPE_CUDA_TRY(ctx, stream_sync(ctx));   // the pose batch reads the clusters from other streams
   std::vector<ope_cloud> views(B);

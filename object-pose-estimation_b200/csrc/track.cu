@@ -188,23 +188,25 @@ int track_chunk(ope_ctx* ctx, Call& call, size_t f0, int B, size_t k) {
 
 using namespace ope;
 
-extern "C" int ope_pose_tracker_step_batch(ope_ctx* ctx, ope_pose_tracker* const* trackers, ope_cloud** sources, const ope_frame_input* targets,
-                                           size_t n, const ope_rng_table* tables, ope_pose_result* results, int32_t* status) {
-  OPE_ENTER(ctx);
-  if (!ctx || (n && (!trackers || !sources || !targets || !results))) return OPE_ERR_INVALID;
-  if (n == 0) return OPE_OK;
-  {
-    std::set<const void*> seen_t, seen_s;
-    for (size_t i = 0; i < n; ++i) {
-      if (!trackers[i] || trackers[i]->ctx != ctx) return fail(ctx, OPE_ERR_INVALID, "tracker %zu is missing or belongs to another context", i);
-      if (!sources[i] || sources[i]->ctx != ctx) return fail(ctx, OPE_ERR_INVALID, "source %zu is missing or belongs to another context", i);
-      if (!seen_t.insert(trackers[i]).second) return fail(ctx, OPE_ERR_INVALID, "tracker %zu is listed twice", i);
-      if (!seen_s.insert(sources[i]).second) return fail(ctx, OPE_ERR_INVALID, "source %zu is listed twice", i);
-      const ope_frame_input& in = targets[i];
-      if (!in.points && in.cloud && ((const ope_cloud*)in.cloud)->ctx != ctx)
-        return fail(ctx, OPE_ERR_INVALID, "target %zu belongs to another context", i);
-    }
+namespace ope {
+
+int step_batch_check(ope_ctx* ctx, ope_pose_tracker* const* trackers, ope_cloud* const* sources, const ope_frame_input* targets, size_t n) {
+  std::set<const void*> seen_t, seen_s;
+  for (size_t i = 0; i < n; ++i) {
+    if (!trackers[i] || trackers[i]->ctx != ctx) return fail(ctx, OPE_ERR_INVALID, "tracker %zu is missing or belongs to another context", i);
+    if (!sources[i] || sources[i]->ctx != ctx) return fail(ctx, OPE_ERR_INVALID, "source %zu is missing or belongs to another context", i);
+    if (!seen_t.insert(trackers[i]).second) return fail(ctx, OPE_ERR_INVALID, "tracker %zu is listed twice", i);
+    if (!seen_s.insert(sources[i]).second) return fail(ctx, OPE_ERR_INVALID, "source %zu is listed twice", i);
+    if (!targets) continue;
+    const ope_frame_input& in = targets[i];
+    if (!in.points && in.cloud && ((const ope_cloud*)in.cloud)->ctx != ctx)
+      return fail(ctx, OPE_ERR_INVALID, "target %zu belongs to another context", i);
   }
+  return OPE_OK;
+}
+
+int tracker_step_batch(ope_ctx* ctx, ope_pose_tracker* const* trackers, ope_cloud** sources, const ope_frame_input* targets, size_t n,
+                       const ope_rng_table* tables, ope_pose_result* results, int32_t* status) {
   const ope_pose_params P = trackers[0]->prm;
   std::vector<Step> steps(n);
   struct Release {   // clouds allocated for trackers that did not finish on the fast path
@@ -286,4 +288,15 @@ extern "C" int ope_pose_tracker_step_batch(ope_ctx* ctx, ope_pose_tracker* const
   }
   OPE_CUDA_TRY(ctx, stream_sync(ctx));
   return first == OPE_OK ? OPE_OK : fail(ctx, first, "tracker step: %s", msg.c_str());
+}
+
+}  // namespace ope
+
+extern "C" int ope_pose_tracker_step_batch(ope_ctx* ctx, ope_pose_tracker* const* trackers, ope_cloud** sources, const ope_frame_input* targets,
+                                           size_t n, const ope_rng_table* tables, ope_pose_result* results, int32_t* status) {
+  OPE_ENTER(ctx);
+  if (!ctx || (n && (!trackers || !sources || !targets || !results))) return OPE_ERR_INVALID;
+  if (n == 0) return OPE_OK;
+  OPE_TRY(step_batch_check(ctx, trackers, sources, targets, n));
+  return tracker_step_batch(ctx, trackers, sources, targets, n, tables, results, status);
 }

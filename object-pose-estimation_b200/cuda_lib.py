@@ -32,6 +32,7 @@ EXPORTS = [
     "ope_pose_tracker_create", "ope_pose_tracker_destroy", "ope_pose_estimate_final", "ope_pose_estimate_final_device", "ope_pose_batch", "ope_pose_tracker_step_batch",
     "ope_pose_stage_ms", "ope_pose_batch_stage_ms", "ope_icp_params_default", "ope_sacia_params_default", "ope_pose_params_default",
     "ope_scene_params_default", "ope_scene_batch_create", "ope_scene_batch_frame", "ope_scene_batch_destroy", "ope_scene_pose_batch",
+    "ope_cloud_centroid", "ope_scene_batch_centroids", "ope_track_params_default", "ope_scene_track_step", "ope_scene_track_phase_ms",
 ]
 
 
@@ -88,6 +89,13 @@ def sacia_params(**kw):
 def pose_params(**kw):
     p = T.PoseParams()
     lib().ope_pose_params_default(C.byref(p))
+    _set(p, kw)
+    return p
+
+
+def track_params(**kw):
+    p = T.TrackParams()
+    lib().ope_track_params_default(C.byref(p))
     _set(p, kw)
     return p
 
@@ -201,6 +209,22 @@ class Context:
         out = (C.c_double * 12)()
         self._chk(lib().ope_pose_batch_stage_ms(self.h, int(enable), out))
         return dict(zip(self.BATCH_STAGES, list(out)[:11]))
+
+    def track_phase_ms(self):
+        """host ms of the phases of the last SceneBatch.track: {"gate", "commit", "rounds": [round 0, 1, ...]}"""
+        k = C.c_int32(0)
+        self._chk(lib().ope_scene_track_phase_ms(self.h, None, 0, C.byref(k)))
+        out = (C.c_double * max(k.value, 1))()
+        self._chk(lib().ope_scene_track_phase_ms(self.h, out, k.value, C.byref(k)))
+        v = list(out)[:k.value]
+        return {"gate": v[0], "commit": v[1], "rounds": v[2:]} if v else {"gate": 0.0, "commit": 0.0, "rounds": []}
+
+    def centroid(self, cloud):
+        """pcl::compute3DCentroid of a device cloud: (xyz (3,) float32, number of finite points)"""
+        c = (C.c_float * 3)()
+        k = C.c_int32(0)
+        self._chk(lib().ope_cloud_centroid(self.h, cloud.h, c, C.byref(k)))
+        return np.array(list(c), np.float32), k.value
 
     def invalidate(self, cloud):
         self._chk(lib().ope_cloud_invalidate(self.h, cloud.h))
@@ -564,6 +588,35 @@ class SceneBatch:
         st = np.array(list(status)[:n], np.int32)
         self.ctx._chk(rc)
         return [res[i] for i in range(n)], st
+
+    def centroids(self, f):
+        """compute3DCentroid of frame f's clusters in rank order: (k, 3) float32 (one row, the whole cloud, when n_clusters == -1)"""
+        k = max(self.info[f].n_clusters, 1)
+        xyz = np.empty((k, 3), np.float32)
+        m = C.c_int32(0)
+        self.ctx._chk(lib().ope_scene_batch_centroids(self.h, C.c_size_t(f), xyz.ctypes.data_as(f32p), C.byref(m)))
+        return xyz[:m.value].copy()
+
+    def track(self, trackers, sources, **track_params):
+        """ope_scene_track_step: camera i = frame i with PoseTracker trackers[i] and its device Cloud sources[i] (the handle is
+        replaced in place when the tracker steps or acquires). track_params: any ope_track_params field. Returns (list of
+        PoseResult, list of TrackChoice, status array); a failing camera has its code in status, a failure of the call itself
+        raises."""
+        n = len(self.info)
+        assert len(trackers) == n and len(sources) == n
+        tp = globals()["track_params"](**track_params)
+        th = (C.c_void_p * max(n, 1))(*[t.h for t in trackers])
+        sh = (C.c_void_p * max(n, 1))(*[s.h for s in sources])
+        res = (T.PoseResult * max(n, 1))()
+        ch = (T.TrackChoice * max(n, 1))()
+        status = (C.c_int32 * max(n, 1))()
+        rc = lib().ope_scene_track_step(self.h, C.byref(tp), th, sh, C.c_size_t(n), res, ch, status)
+        for i, s in enumerate(sources):
+            s.h = C.c_void_p(sh[i])
+        st = np.array(list(status)[:n], np.int32)
+        if rc != 0 and not (st == rc).any():
+            self.ctx._chk(rc)
+        return [res[i] for i in range(n)], [ch[i] for i in range(n)], st
 
     def close(self):
         # the handle holds device memory of its context: destroyed before the context is

@@ -214,6 +214,45 @@ def make_sequence(model, seq, n_frames, max_deg=10.0, max_t=0.02):
     return out
 
 
+TABLE_UP = np.array([0.0, -np.cos(np.deg2rad(30.0)), -np.sin(np.deg2rad(30.0))])   # render_scene's table normal
+TABLE_AWAY = np.array([0.0, -np.sin(np.deg2rad(30.0)), np.cos(np.deg2rad(30.0))])  # in the table plane, away from the camera
+
+
+def make_scene_sequence(model, seq, n_frames, distractors=2, jump_at=None, max_deg=5.0, max_t=0.01):
+    """A multi-object tracking sequence in depth images: the object on the table in front of the camera, turned and moved by a
+    small_pose step (about its own centre) per frame, next to `distractors` (0, 1 or 2) static objects on the same table at least
+    10 cm away from it: a cylinder larger than the object (its cluster is the largest, rank 0) and a small box. At frame jump_at
+    the object moves 12 cm further along the table. Returns (depth (n_frames, 480, 640) uint16 millimetres, object poses)."""
+    rng = rng_for(seq, stream=6)
+    R = random_rotation(rng)
+    # x = -0.12 at z = 1: the middle of the crop, whose x is the image column measured from cy (depth_to_cloud's row/column quirk)
+    t = np.array([rng.uniform(-0.16, -0.08), 0.0, rng.uniform(0.95, 1.05)])
+    # the object's centre sits half its extent above the table; distractors stand on the same level, to its left and right
+    base = t - TABLE_UP * 0.05
+    still = []
+    if distractors >= 1:
+        cyl = _sample_cylinder(rng, 60000, 0.07, 0.22, 0.0)                # axis along the table normal, foot on the table
+        frame = np.stack([np.array([1.0, 0.0, 0.0]), TABLE_AWAY, TABLE_UP], 1)
+        still.append(cyl @ frame.T + base + np.array([0.30, 0.0, 0.0]) - TABLE_UP * 0.01)
+    if distractors >= 2:
+        box = _sample_box(rng, 20000, (-0.03, -0.03, 0.0), (0.03, 0.03, 0.06))
+        frame = np.stack([np.array([1.0, 0.0, 0.0]), TABLE_AWAY, TABLE_UP], 1)
+        still.append(box @ frame.T + base + np.array([-0.27, 0.0, 0.0]) - TABLE_UP * 0.01)
+    depth, poses = [], []
+    for k in range(n_frames):
+        if k == jump_at:
+            t = t + 0.12 * TABLE_AWAY
+        pose = np.eye(4)
+        pose[:3, :3], pose[:3, 3] = R, t
+        pts = np.concatenate([apply(pose, model)] + [p.astype(np.float32) for p in still], 0)
+        cloud, _ = render_scene(pts, np.eye(4), rng)
+        depth.append(np.rint(np.nan_to_num(cloud[..., 2], nan=0.0).astype(np.float64) * 1000.0).astype(np.uint16))
+        poses.append(pose)
+        step = small_pose(rng, max_deg, max_t)
+        R, t = step[:3, :3] @ R, t + step[:3, 3]
+    return np.stack(depth), poses
+
+
 def icp_pair(n=50000, seed=0, model=None, max_deg=10.0, max_t=0.02, sigma=0.001, outlier_frac=0.10):
     """C2: target = n model-surface points, source = an independent n-sample under a small perturbation,
     sigma = 1 mm noise, 10 % of the source replaced by outliers in the (inflated) bounding box."""
