@@ -178,7 +178,8 @@ int ope_scene_track_step(const ope_scene_batch* s, const ope_track_params* tp, o
 int ope_scene_track_phase_ms(const ope_ctx* ctx, double* out, int cap, int32_t* n_out);
 
 /* ---- spatial search: replaces pcl::search::KdTree / KdTreeFLANN (SURVEY A.3) -------------------------- */
-/* nearestKSearch for nq host queries; out_idx/out_d2 are nq*k, padded with -1 / +inf. k <= 32. */
+/* nearestKSearch for nq host queries; out_idx/out_d2 are nq*k, ascending (d2, index), padded with -1 / +inf. 1 <= k <=
+ * OPE_KNN_MAX_K (256), OPE_ERR_INVALID otherwise. */
 int ope_knn(ope_ctx* ctx, const ope_cloud* tgt, const void* qry, size_t nq, size_t stride, size_t offset, int k,
             int32_t* out_idx, float* out_d2);
 /* same with the queries already on the device */
@@ -203,8 +204,15 @@ int ope_voxel_grid(ope_ctx* ctx, const ope_cloud* cloud, const float* rgb, float
 
 /* ---- features ------------------------------------------------------------------------------------------- */
 /* pcl::NormalEstimation::setKSearch(k) + compute (D&L/src/poseestimator.cpp:151-156, BM/src/regmeshpcd.cpp:74-90;
- * SURVEY A.4). Writes the normals into the cloud (device) and, if out4 != NULL, to the host (n*4). */
+ * SURVEY A.4). Writes the normals into the cloud (device) and, if out4 != NULL, to the host (n*4). 1 <= k <= OPE_KNN_MAX_K,
+ * OPE_ERR_INVALID otherwise. The covariance is summed over the k nearest in ascending (d2, index) order. */
 int ope_normals_knn(ope_ctx* ctx, ope_cloud* cloud, int k, const float viewpoint[3], float* out4);
+/* pcl::NormalEstimation::setRadiusSearch(radius) + compute. Neighbours: the finite points with d2 < radius^2 (strict; the query
+ * itself included), summed in ascending (d2, index) order. A non-finite point, or one with fewer than 3 neighbours, gets NaN normal
+ * and curvature. The normal is flipped toward the viewpoint (NULL: the origin). Writes the normals into the cloud (device) and, if
+ * out4 != NULL, to the host (n*4). Any neighbour count runs; lists longer than the shared-memory capacity take device scratch in
+ * tiles bounded by OPE_RADIUS_NORMALS_SCRATCH_BYTES (INTEGRATION.md section 5). radius <= 0 or not finite: OPE_ERR_INVALID. */
+int ope_normals_radius(ope_ctx* ctx, ope_cloud* cloud, float radius, const float viewpoint[3], float* out4);
 /* pcl::FPFHEstimation::setRadiusSearch + compute (D&L/src/poseestimator.cpp:121-125; SURVEY A.5). The cloud must
  * carry normals. out: n*33 floats (host). out_spfh (n*33) may be NULL. */
 int ope_fpfh(ope_ctx* ctx, const ope_cloud* cloud, float radius, float* out, float* out_spfh);

@@ -72,6 +72,8 @@ enum {
 };
 
 #define OPE_MAX_REJECTORS 4
+/* largest k of ope_knn, ope_knn_cloud and ope_normals_knn (and of ope_pose_params.normal_k); k above it is OPE_ERR_INVALID */
+#define OPE_KNN_MAX_K 256
 
 /* IterativeClosestPoint[WithNormals] configuration. Defaults: VP/registration_mod.h:102-130,
  * VP/default_convergence_criteria_mod.h:94-110, VP/icp_mod.h:136-152. */

@@ -5,7 +5,9 @@
 // 132 FPFH write) plus an m-neighbour gather of 32 B (SPFH pass) / 136 B (FPFH pass) per neighbour from L2.
 #include <algorithm>
 
+#include <climits>
 #include <cstdlib>
+#include <vector>
 #include <mutex>
 
 #include "ope_host.cuh"
@@ -120,6 +122,150 @@ __global__ void __launch_bounds__(kNormThreads) normals_smem_batch_kernel(const 
   const int n = counts[blockIdx.y];
   if (n <= 0 || (int)blockIdx.x * (kNormThreads / 32) >= n) return;   // more blocks than this cloud has points: nothing to do
   normals_smem_body(pts + (size_t)blockIdx.y * stride, n, k, vpx, vpy, vpz, out + (size_t)blockIdx.y * stride);
+}
+
+// k > 32 (warp_knn_list): the warp's list in shared memory, then lane 0 sums the covariance over it in list order — the same
+// serial float chain as the kernels above, so pointNormal of the oracle is the reference for both. SMEM: the whole cloud in
+// shared memory and the brute-force scan (clouds of up to kNormSmemMax points), otherwise the grid.
+template <bool SMEM>
+__global__ void __launch_bounds__(kNormThreads) normals_list_kernel(GridView g, const float4* __restrict__ pts, int n, int k, float vpx,
+                                                                    float vpy, float vpz, float4* __restrict__ out) {
+  extern __shared__ __align__(16) float4 tg_list[];
+  __shared__ OctStack stacks[SMEM ? 1 : kNormThreads / 32];
+  __shared__ KnnList lists[kNormThreads / 32];
+  __shared__ int s_fin;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  KnnList* L = &lists[warp];
+  int n_finite = 0;
+  if (SMEM) {
+    int fin = 0;
+    for (int j = threadIdx.x; j < n; j += kNormThreads) {
+      const float4 t = __ldg(pts + j);
+      tg_list[j] = t;
+      fin += finite3(t.x, t.y, t.z) ? 1 : 0;
+    }
+    if (threadIdx.x == 0) s_fin = 0;
+    __syncthreads();
+    for (int o = 16; o > 0; o >>= 1) fin += __shfl_xor_sync(0xffffffffu, fin, o);
+    if (lane == 0) atomicAdd(&s_fin, fin);
+    __syncthreads();
+    n_finite = s_fin;
+  }
+  const int wid = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, n_warps = (gridDim.x * blockDim.x) >> 5;
+  const float nan = __int_as_float(0x7fc00000);
+  for (int i = wid; i < n; i += n_warps) {
+    const float4 q = SMEM ? tg_list[i] : __ldg(pts + i);
+    const bool ok = finite3(q.x, q.y, q.z);
+    const int cnt = SMEM ? warp_knn_list_smem(tg_list, n, n_finite, L, ok, q.x, q.y, q.z, k)
+                         : warp_knn_list(g, &stacks[SMEM ? 0 : warp], L, ok, q.x, q.y, q.z, k);
+    if (lane == 0) {
+      float r[4] = {nan, nan, nan, nan};
+      if (ok && cnt >= 3) {
+        CovAccum acc;
+        acc.reset();
+        for (int j = 0; j < cnt; ++j) {
+          const int t = __float_as_int(L->e[j].y);
+          const float4 p = SMEM ? tg_list[t] : __ldg(pts + t);
+          acc.add(p.x, p.y, p.z);
+        }
+        normal_from_accum(acc, cnt, q.x, q.y, q.z, vpx, vpy, vpz, r);
+      }
+      out[i] = make_float4(r[0], r[1], r[2], r[3]);
+    }
+    __syncwarp();
+  }
+}
+
+// ----------------------------------------------------------------------------------------- radius normals ----
+// NormalEstimation::setRadiusSearch(r): the neighbours are the finite points with d2 < r2 (the query included), summed in
+// ascending (d2, index) order. Neighbourhoods run from none to ~10^4 points, so:
+//   count pass   one warp per query counts its neighbours (lanes stride over the grid's leaf ranges);
+//   main pass    one block per query gathers its neighbours as 64-bit keys (d2 bits << 32 | index: d2 >= 0, so the key order is
+//                the (d2, index) order) in any order, sorts them with a block-wide bitonic network, and thread 0 sums the
+//                covariance over the sorted keys. A list of up to kRadSmemKeys keys lives in shared memory; a longer one in its
+//                slice of a global scratch buffer, which the host fills by query tiles sized to a byte budget.
+static constexpr int kRadThreads = 256;
+static constexpr int kRadSmemKeys = 8192;   // 64 KB of shared memory per block
+__global__ void radius_count_warp_kernel(GridView g, const float4* __restrict__ pts, int n, float r2, int* __restrict__ counts) {
+  const int lane = threadIdx.x & 31;
+  const int wid = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, n_warps = (gridDim.x * blockDim.x) >> 5;
+  for (int i = wid; i < n; i += n_warps) {
+    const float4 q = __ldg(pts + i);
+    int cnt = 0;
+    if (finite3(q.x, q.y, q.z))
+      grid_radius_ranges(g, q.x, q.y, q.z, r2, 64, [&](int b, int e) {
+        for (int j = b + lane; j < e; j += 32) {
+          const float4 p = __ldg(g.pts + j);
+          cnt += dist2(q.x, q.y, q.z, p.x, p.y, p.z) < r2 ? 1 : 0;
+        }
+      });
+    for (int o = 16; o > 0; o >>= 1) cnt += __shfl_xor_sync(0xffffffffu, cnt, o);
+    if (lane == 0) counts[i] = cnt;
+  }
+}
+
+// Ascending sort of a[0, n) by the block: the bitonic network in its all-ascending form (each merge starts by comparing mirrored
+// elements), so every comparator (i, j) has i < j and the positions >= n act as +inf that never move: no padding is stored.
+__device__ __forceinline__ void block_bitonic_sort(unsigned long long* a, int n) {
+  int N = 1;
+  while (N < n) N <<= 1;
+  for (int k = 2; k <= N; k <<= 1) {
+    for (int s = k >> 1; s > 0; s >>= 1) {
+      for (int t = threadIdx.x; t < N / 2; t += blockDim.x) {
+        const int i = (t / s) * 2 * s + (t % s);
+        const int j = (s == k >> 1) ? (i ^ (k - 1)) : i + s;
+        if (j < n) {
+          const unsigned long long x = a[i], y = a[j];
+          if (y < x) { a[i] = y; a[j] = x; }
+        }
+      }
+      __syncthreads();
+    }
+  }
+}
+
+// queries [q0, q1): counts from the count pass; a query with more than kRadSmemKeys neighbours keeps its keys at
+// scratch + (big_off[i] - big_off[q0])
+__global__ void __launch_bounds__(kRadThreads) normals_radius_kernel(GridView g, const float4* __restrict__ pts, int q0, int q1, float r2,
+                                                                     const int* __restrict__ counts, const long long* __restrict__ big_off,
+                                                                     unsigned long long* __restrict__ scratch, float vpx, float vpy,
+                                                                     float vpz, float4* __restrict__ out) {
+  extern __shared__ __align__(16) unsigned long long keys_smem[];
+  __shared__ int s_fill;
+  const float nan = __int_as_float(0x7fc00000);
+  for (int i = q0 + blockIdx.x; i < q1; i += gridDim.x) {
+    const int cnt = counts[i];
+    const float4 q = __ldg(pts + i);
+    if (cnt < 3) {   // also every non-finite query (count 0)
+      if (threadIdx.x == 0) out[i] = make_float4(nan, nan, nan, nan);
+      continue;
+    }
+    unsigned long long* keys = cnt <= kRadSmemKeys ? keys_smem : scratch + (big_off[i] - big_off[q0]);
+    if (threadIdx.x == 0) s_fill = 0;
+    __syncthreads();
+    grid_radius_ranges(g, q.x, q.y, q.z, r2, 64, [&](int b, int e) {
+      for (int j = b + (int)threadIdx.x; j < e; j += kRadThreads) {
+        const float4 p = __ldg(g.pts + j);
+        const float d2 = dist2(q.x, q.y, q.z, p.x, p.y, p.z);
+        if (d2 < r2)
+          keys[atomicAdd(&s_fill, 1)] = ((unsigned long long)__float_as_uint(d2) << 32) | (unsigned)__float_as_int(p.w);
+      }
+    });
+    __syncthreads();
+    block_bitonic_sort(keys, cnt);
+    if (threadIdx.x == 0) {
+      CovAccum acc;
+      acc.reset();
+      for (int j = 0; j < cnt; ++j) {
+        const float4 p = __ldg(pts + (unsigned)keys[j]);
+        acc.add(p.x, p.y, p.z);
+      }
+      float r[4];
+      normal_from_accum(acc, cnt, q.x, q.y, q.z, vpx, vpy, vpz, r);
+      out[i] = make_float4(r[0], r[1], r[2], r[3]);
+    }
+    __syncthreads();   // the keys are reused by the block's next query
+  }
 }
 
 // ------------------------------------------------------------------------------------------- SPFH ------
@@ -398,9 +544,26 @@ __global__ void compact_cloud_kernel(const float4* __restrict__ pts, const float
 
 // ================================================================================================ host ==
 int normals_device(ope_ctx* ctx, ope_cloud* cloud, int k, const float vp[3]) {
-  if (k < 1 || k > 32) return fail(ctx, OPE_ERR_INVALID, "normal estimation k must be in [1, 32]");
+  static_assert(kKnnListMax == OPE_KNN_MAX_K, "the shared-memory list holds OPE_KNN_MAX_K entries");
+  if (k < 1 || k > OPE_KNN_MAX_K) return fail(ctx, OPE_ERR_INVALID, "normal estimation k must be in [1, %d]", OPE_KNN_MAX_K);
   if (!cloud->normals) OPE_TRY(dalloc(ctx, &cloud->normals, cloud->n));
   if (cloud->n == 0) return OPE_OK;
+  if (k > 32) {
+    GridView g;
+    std::memset(&g, 0, sizeof(g));
+    if (cloud->n <= (size_t)kNormSmemMax && !std::getenv("OPE_NORMALS_FORCE_GRID")) {
+      OPE_TRY(dyn_smem(ctx, (const void*)normals_list_kernel<true>, kNormSmemMax * sizeof(float4)));
+      const unsigned blocks = (unsigned)std::min<size_t>(div_up(cloud->n * 32, kNormThreads), (size_t)ctx->sm_count * 2);
+      normals_list_kernel<true><<<blocks, kNormThreads, cloud->n * sizeof(float4), ctx->stream>>>(g, cloud->pts, (int)cloud->n, k, vp[0],
+                                                                                                   vp[1], vp[2], cloud->normals);
+      return check_launch(ctx, "normals_list_kernel<smem>");
+    }
+    OPE_TRY(cloud_bbox(ctx, cloud));
+    OPE_TRY(cloud_grid(ctx, cloud, knn_cell_size(cloud, k), &g));
+    normals_list_kernel<false><<<(unsigned)std::min<size_t>(div_up(cloud->n * 32, kNormThreads), (size_t)ctx->sm_count * 8), kNormThreads, 0,
+                                 ctx->stream>>>(g, cloud->pts, (int)cloud->n, k, vp[0], vp[1], vp[2], cloud->normals);
+    return check_launch(ctx, "normals_list_kernel");
+  }
   if (cloud->n <= (size_t)kNormSmemMax && !std::getenv("OPE_NORMALS_FORCE_GRID")) {
     const size_t bytes = cloud->n * sizeof(float4);
     OPE_TRY(dyn_smem(ctx, (const void*)normals_smem_kernel, kNormSmemMax * sizeof(float4)));
@@ -414,6 +577,62 @@ int normals_device(ope_ctx* ctx, ope_cloud* cloud, int k, const float vp[3]) {
   normals_kernel<<<(unsigned)std::min<size_t>(div_up(cloud->n * 32, kNormThreads), (size_t)ctx->sm_count * 8), kNormThreads, 0, ctx->stream>>>(g, cloud->pts, (int)cloud->n, k, vp[0], vp[1], vp[2],
                                                                  cloud->normals);
   return check_launch(ctx, "normals_kernel");
+}
+
+// Scratch budget of the lists longer than kRadSmemKeys: OPE_RADIUS_NORMALS_SCRATCH_BYTES (default 256 MiB). A query whose own list
+// exceeds it still runs, alone in its tile.
+static size_t radius_scratch_budget() {
+  const char* e = std::getenv("OPE_RADIUS_NORMALS_SCRATCH_BYTES");
+  const long long v = e ? std::atoll(e) : 0;
+  return v > 0 ? (size_t)v : ((size_t)256 << 20);
+}
+
+int normals_radius_device(ope_ctx* ctx, ope_cloud* cloud, float radius, const float vp[3]) {
+  if (!(radius > 0) || !std::isfinite(radius)) return fail(ctx, OPE_ERR_INVALID, "normal estimation radius must be positive and finite");
+  if (!cloud->normals) OPE_TRY(dalloc(ctx, &cloud->normals, cloud->n));
+  const size_t n = cloud->n;
+  if (n == 0) return OPE_OK;
+  if (n > (size_t)INT_MAX) return fail(ctx, OPE_ERR_INVALID, "radius normals: cloud larger than INT_MAX points");
+  GridView g;
+  OPE_TRY(cloud_grid(ctx, cloud, radius * 0.5f, &g));
+  const float r2 = radius * radius;
+  Scratch<int> cnt(ctx);
+  OPE_TRY(cnt.alloc(n));
+  radius_count_warp_kernel<<<(unsigned)std::min<size_t>(div_up(n * 32, kNormThreads), (size_t)ctx->sm_count * 8), kNormThreads, 0,
+                             ctx->stream>>>(g, cloud->pts, (int)n, r2, cnt.p);
+  OPE_TRY(check_launch(ctx, "radius_count_warp_kernel"));
+  std::vector<int> h_cnt;
+  OPE_TRY(download(ctx, cnt.p, n, h_cnt));
+  // global slices of the long lists, then tiles of consecutive queries whose long lists fit the budget together
+  std::vector<long long> off(n + 1, 0);
+  for (size_t i = 0; i < n; ++i) off[i + 1] = off[i] + (h_cnt[i] > kRadSmemKeys ? h_cnt[i] : 0);
+  const long long budget = (long long)(radius_scratch_budget() / sizeof(unsigned long long));
+  std::vector<std::pair<int, int>> tiles;
+  long long scratch_keys = 0;
+  for (size_t q0 = 0; q0 < n;) {
+    size_t q1 = q0 + 1;
+    while (q1 < n && off[q1 + 1] - off[q0] <= budget) ++q1;
+    tiles.emplace_back((int)q0, (int)q1);
+    scratch_keys = std::max(scratch_keys, off[q1] - off[q0]);
+    q0 = q1;
+  }
+  Scratch<long long> d_off(ctx);
+  Scratch<unsigned long long> keys(ctx);
+  if (off[n] > 0) {
+    OPE_TRY(d_off.alloc(n + 1));
+    OPE_TRY(keys.alloc((size_t)scratch_keys));
+    OPE_CUDA_TRY(ctx, cudaMemcpyAsync(d_off.p, off.data(), (n + 1) * sizeof(long long), cudaMemcpyHostToDevice, ctx->stream));
+  }
+  int max_smem = 0;
+  for (size_t i = 0; i < n; ++i) if (h_cnt[i] <= kRadSmemKeys) max_smem = std::max(max_smem, h_cnt[i]);
+  OPE_TRY(dyn_smem(ctx, (const void*)normals_radius_kernel, kRadSmemKeys * sizeof(unsigned long long)));
+  for (const auto& t : tiles) {
+    const unsigned blocks = (unsigned)std::min<size_t>((size_t)(t.second - t.first), (size_t)ctx->sm_count * 4);
+    normals_radius_kernel<<<blocks, kRadThreads, (size_t)max_smem * sizeof(unsigned long long), ctx->stream>>>(
+        g, cloud->pts, t.first, t.second, r2, cnt.p, d_off.p, keys.p, vp[0], vp[1], vp[2], cloud->normals);
+    OPE_TRY(check_launch(ctx, "normals_radius_kernel"));   // the next tile reuses the scratch after this one, in stream order
+  }
+  return OPE_OK;
 }
 
 int fpfh_device(ope_ctx* ctx, const ope_cloud* cloud, float radius, float** d_fpfh, float** d_spfh_out) {
@@ -584,6 +803,17 @@ int ope_normals_knn(ope_ctx* ctx, ope_cloud* cloud, int k, const float viewpoint
   if (!ctx || !cloud) return OPE_ERR_INVALID;
   const float zero[3] = {0, 0, 0};
   OPE_TRY(normals_device(ctx, cloud, k, viewpoint ? viewpoint : zero));
+  if (out4 && cloud->n)
+    OPE_CUDA_TRY(ctx, cudaMemcpyAsync(out4, cloud->normals, cloud->n * sizeof(float4), cudaMemcpyDeviceToHost, ctx->stream));
+  OPE_CUDA_TRY(ctx, ope::stream_sync(ctx));
+  return OPE_OK;
+}
+
+int ope_normals_radius(ope_ctx* ctx, ope_cloud* cloud, float radius, const float viewpoint[3], float* out4) {
+  OPE_ENTER(ctx);
+  if (!ctx || !cloud) return OPE_ERR_INVALID;
+  const float zero[3] = {0, 0, 0};
+  OPE_TRY(normals_radius_device(ctx, cloud, radius, viewpoint ? viewpoint : zero));
   if (out4 && cloud->n)
     OPE_CUDA_TRY(ctx, cudaMemcpyAsync(out4, cloud->normals, cloud->n * sizeof(float4), cudaMemcpyDeviceToHost, ctx->stream));
   OPE_CUDA_TRY(ctx, ope::stream_sync(ctx));

@@ -285,6 +285,26 @@ __global__ void __launch_bounds__(kKnnThreads) knn_kernel(GridView g, const floa
     __syncwarp();
   }
 }
+// k > 32: the list in shared memory (warp_knn_list), written out with -1 / +inf padding past the count
+__global__ void __launch_bounds__(kKnnThreads) knn_list_kernel(GridView g, const float4* __restrict__ qry, int nq, int k,
+                                                               int* __restrict__ out_idx, float* __restrict__ out_d2) {
+  __shared__ OctStack stacks[kKnnThreads / 32];
+  __shared__ KnnList lists[kKnnThreads / 32];
+  OctStack* st = &stacks[threadIdx.x >> 5];
+  KnnList* L = &lists[threadIdx.x >> 5];
+  const int lane = threadIdx.x & 31;
+  const int wid = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, n_warps = (gridDim.x * blockDim.x) >> 5;
+  for (int i = wid; i < nq; i += n_warps) {
+    const float4 q = __ldg(qry + i);
+    const int cnt = warp_knn_list(g, st, L, finite3(q.x, q.y, q.z), q.x, q.y, q.z, k);
+    for (int j = lane; j < k; j += 32) {
+      const float2 v = j < cnt ? L->e[j] : make_float2(INFINITY, __int_as_float(-1));
+      out_idx[(size_t)i * k + j] = __float_as_int(v.y);
+      if (out_d2) out_d2[(size_t)i * k + j] = v.x;
+    }
+    __syncwarp();
+  }
+}
 __global__ void radius_count_kernel(GridView g, const float4* __restrict__ qry, int nq, float r2, int* __restrict__ counts) {
   int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= nq) return;
@@ -940,7 +960,8 @@ int ope_cloud_set_normals(ope_ctx* ctx, ope_cloud* c, const float* normals4) {
 }
 
 static int knn_impl(ope_ctx* ctx, const ope_cloud* tgt, const float4* d_qry, size_t nq, int k, int32_t* out_idx, float* out_d2) {
-  if (k < 1 || k > 32) return fail(ctx, OPE_ERR_INVALID, "k must be in [1, 32]");
+  static_assert(kKnnListMax == OPE_KNN_MAX_K, "the shared-memory list holds OPE_KNN_MAX_K entries");
+  if (k < 1 || k > OPE_KNN_MAX_K) return fail(ctx, OPE_ERR_INVALID, "k must be in [1, %d]", OPE_KNN_MAX_K);
   if (nq == 0) return OPE_OK;
   OPE_TRY(cloud_bbox(ctx, const_cast<ope_cloud*>(tgt)));
   GridView g;
@@ -954,6 +975,10 @@ static int knn_impl(ope_ctx* ctx, const ope_cloud* tgt, const float4* d_qry, siz
     nn1_kernel<<<(unsigned)std::min<size_t>(div_up(nq, kKnnThreads), (size_t)ctx->sm_count * 4), kKnnThreads,
                  sizeof(Nn1Smem<kKnnThreads>), ctx->stream>>>(g, d_qry, (int)nq, di.p, dd.p);
     OPE_TRY(check_launch(ctx, "nn1_kernel"));
+  } else if (k > 32) {
+    knn_list_kernel<<<(unsigned)std::min<size_t>(div_up(nq * 32, kKnnThreads), (size_t)ctx->sm_count * 8), kKnnThreads, 0,
+                      ctx->stream>>>(g, d_qry, (int)nq, k, di.p, dd.p);
+    OPE_TRY(check_launch(ctx, "knn_list_kernel"));
   } else {
     knn_kernel<<<(unsigned)std::min<size_t>(div_up(nq * 32, kKnnThreads), (size_t)ctx->sm_count * 8), kKnnThreads, 0,
                  ctx->stream>>>(g, d_qry, (int)nq, k, di.p, dd.p);

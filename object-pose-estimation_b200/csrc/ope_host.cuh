@@ -296,6 +296,8 @@ int cloud_content_hash(ope_ctx* ctx, const ope_cloud* cloud, unsigned long long*
 
 // ---- features.cu ----
 int normals_device(ope_ctx* ctx, ope_cloud* cloud, int k, const float vp[3]);
+// NormalEstimation with setRadiusSearch(radius): neighbours d2 < radius^2, summed in (d2, index) order (features.cu)
+int normals_radius_device(ope_ctx* ctx, ope_cloud* cloud, float radius, const float vp[3]);
 int fpfh_device(ope_ctx* ctx, const ope_cloud* cloud, float radius, float** d_fpfh, float** d_spfh_or_null);
 int feature_knn_device(ope_ctx* ctx, const float* d_ftgt, size_t nt, const float* d_fqry, size_t nq, int dim, int k,
                        int* d_idx, float* d_d2);

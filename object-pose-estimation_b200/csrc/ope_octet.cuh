@@ -587,4 +587,134 @@ __device__ __forceinline__ int warp_knn_smem_bounded(const float4* tg, int nt, i
   return k;
 }
 
+// ---- k nearest for 32 < k <= kKnnListMax: the sorted list in SHARED memory ---------------------------------------------
+// One query per warp, as warp_knn, but the list no longer fits one entry per lane: it lives in the warp's KnnList, 8 B per entry
+// (d2, index bits), ascending (d2, index). Candidates come 32 at a time (one per lane); the ones that beat the k-th entry are
+// merged in one step: each ranks itself within the batch (shuffles) and within the list (binary search), each list entry counts
+// the batch entries below it (binary search in the sorted batch), and every entry is written to its merged position. (d2, index)
+// pairs are distinct, so the positions are a permutation and the list equals the one inserting the candidates one by one builds.
+static constexpr int kKnnListMax = 256;   // OPE_KNN_MAX_K
+struct KnnList {
+  float2 e[kKnnListMax];   // the list
+  float2 b[32];            // the sorted batch being merged
+};
+
+// Merge this lane's candidate (when `cand`) into L (cnt entries, at most k kept). All 32 lanes call; returns the new count.
+__device__ __forceinline__ int knn_list_merge(KnnList* L, int cnt, int k, bool cand, float d2, int idx) {
+  const unsigned full = 0xffffffffu;
+  const int lane = threadIdx.x & 31;
+  const unsigned cm = __ballot_sync(full, cand);
+  if (cm == 0u) return cnt;
+  const int nc = __popc(cm);
+  int rb = 0;   // rank within the batch
+#pragma unroll
+  for (int o = 0; o < 32; ++o) {
+    const float od = __shfl_sync(full, d2, o);
+    const int oi = __shfl_sync(full, idx, o);
+    rb += (((cm >> o) & 1u) && nb_less(od, oi, d2, idx)) ? 1 : 0;
+  }
+  int rl = 0;   // rank within the list
+  if (cand) {
+    int hi = cnt;
+    while (rl < hi) {
+      const int m = (rl + hi) >> 1;
+      const float2 v = L->e[m];
+      if (nb_less(v.x, __float_as_int(v.y), d2, idx)) rl = m + 1; else hi = m;
+    }
+    L->b[rb] = make_float2(d2, __int_as_float(idx));
+  }
+  __syncwarp();
+  float2 keep[kKnnListMax / 32];
+  int pos[kKnnListMax / 32];
+#pragma unroll
+  for (int t = 0; t < kKnnListMax / 32; ++t) {
+    const int j = lane + 32 * t;
+    pos[t] = k;   // not kept
+    if (j < cnt) {
+      keep[t] = L->e[j];
+      const int vi = __float_as_int(keep[t].y);
+      int lo = 0, hi = nc;
+      while (lo < hi) {
+        const int m = (lo + hi) >> 1;
+        const float2 c = L->b[m];
+        if (nb_less(c.x, __float_as_int(c.y), keep[t].x, vi)) lo = m + 1; else hi = m;
+      }
+      pos[t] = j + lo;
+    }
+  }
+  __syncwarp();
+#pragma unroll
+  for (int t = 0; t < kKnnListMax / 32; ++t)
+    if (pos[t] < k) L->e[pos[t]] = keep[t];
+  if (cand && rb + rl < k) L->e[rb + rl] = make_float2(d2, __int_as_float(idx));
+  __syncwarp();
+  return min(cnt + nc, k);
+}
+
+// Exact k nearest (32 < k <= kKnnListMax) of the warp's query on the grid: warp_knn's traversal (nearest node first, nodes
+// pruned by the current k-th distance), warp_knn's candidate rule, the list in L. Returns the count (min(k, g.n)); the
+// entries L->e[0 .. count) are valid after the call.
+__device__ __forceinline__ int warp_knn_list(const GridView& g, OctStack* st, KnnList* L, bool active, float qx, float qy, float qz, int k) {
+  const Coop<32> o;
+  const float ux = (qx - g.ox) * g.inv_h, uy = (qy - g.oy) * g.inv_h, uz = (qz - g.oz) * g.inv_h;
+  if (k > g.n) k = g.n;
+  int cnt = 0;
+  if (!(active && g.n > 0 && k > 0)) return 0;
+  float kth_d = FLT_MAX;
+  int kth_i = 0x7fffffff;
+  int sp = coop_push_ball(g, st, o, true, ux, uy, uz, FLT_MAX);
+  while (sp > 0) {
+    --sp;
+    const OctEntry en = st->s[sp];
+    __syncwarp();
+    float bound = (cnt == k) ? kth_d : FLT_MAX;
+    const bool live = en.d2 <= bound;
+    const int level = (int)(en.node >> 27);
+    const bool leaf = level == 0 || en.e - en.b <= kWarpLeaf;
+    if (live && leaf) {
+      for (int base = en.b; base < en.e; base += 32) {
+        const int i = base + (int)o.sub;
+        float d2 = FLT_MAX;
+        int idx = 0x7fffffff;
+        if (i < en.e) {
+          const float4 p = __ldg(g.pts + i);
+          d2 = dist2(qx, qy, qz, p.x, p.y, p.z);
+          idx = __float_as_int(p.w);
+        }
+        const bool cand = idx != 0x7fffffff && d2 <= FLT_MAX && (cnt < k || nb_less(d2, idx, kth_d, kth_i));
+        cnt = knn_list_merge(L, cnt, k, cand, d2, idx);
+        if (cnt == k) { const float2 v = L->e[k - 1]; kth_d = v.x; kth_i = __float_as_int(v.y); }
+      }
+      bound = (cnt == k) ? kth_d : FLT_MAX;
+    }
+    sp += coop_expand(g, st, o, sp, live && !leaf, en.node, en.e, ux, uy, uz, bound);
+  }
+  return cnt;
+}
+
+// The same list among nt target points held in SHARED memory in their original order (warp_knn_smem's scan, n_finite = number
+// of finite targets, k clamped to it): the same entries as warp_knn_list.
+__device__ __forceinline__ int warp_knn_list_smem(const float4* tg, int nt, int n_finite, KnnList* L, bool active, float qx, float qy,
+                                                  float qz, int k) {
+  const int lane = threadIdx.x & 31;
+  if (k > n_finite) k = n_finite;
+  int cnt = 0;
+  if (!(active && k > 0)) return 0;
+  float kth_d = FLT_MAX;
+  int kth_i = 0x7fffffff;
+  for (int base = 0; base < nt; base += 32) {
+    const int j = base + lane;
+    float d2 = FLT_MAX;
+    int idx = 0x7fffffff;
+    if (j < nt) {
+      const float4 t = tg[j];
+      if (finite3(t.x, t.y, t.z)) { d2 = dist2(qx, qy, qz, t.x, t.y, t.z); idx = j; }
+    }
+    const bool cand = idx != 0x7fffffff && d2 <= FLT_MAX && (cnt < k || nb_less(d2, idx, kth_d, kth_i));
+    cnt = knn_list_merge(L, cnt, k, cand, d2, idx);
+    if (cnt == k) { const float2 v = L->e[k - 1]; kth_d = v.x; kth_i = __float_as_int(v.y); }
+  }
+  return cnt;
+}
+
 }  // namespace ope

@@ -511,7 +511,8 @@ int ope_pose_batch(ope_ctx* ctx, const ope_pose_params* prm, const float* model_
   }
   // ---- frame-spanning launches (batch.cu): one launch per stage for a whole chunk of frames; the frames outside their envelope
   // (tiny / empty / oversized clusters, or every frame when the ICP parameters are outside it) are collected for a second pass ----
-  const bool fast = icp_small_batch_applicable(P.icp, 1, 1) && P.icp.n_rejectors >= 0;
+  // normal_k above 32 is outside the frame-spanning normal kernel: every frame then runs on the per-frame path
+  const bool fast = icp_small_batch_applicable(P.icp, 1, 1) && P.icp.n_rejectors >= 0 && P.normal_k <= 32;
   std::mutex frame_mu;
   std::vector<size_t> rest;
   int lrc = run_chunks_on_lanes(ctx, n_frames, &draw_rc, [&](ope_ctx* c, size_t f0, size_t nf, size_t) -> int {

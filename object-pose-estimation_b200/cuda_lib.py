@@ -26,7 +26,7 @@ EXPORTS = [
     "ope_cloud_select", "ope_cloud_transform", "ope_cloud_set_normals", "ope_cloud_append", "ope_register_point_clouds",
     "ope_pass_through", "ope_euclidean_clusters", "ope_plane_ransac", "ope_segment_objects_on_plane", "ope_segment_params_default", "ope_knn", "ope_knn_cloud", "ope_radius_cloud", "ope_depth_to_cloud", "ope_depth_to_cloud_batch",
     "ope_uniform_sample", "ope_uniform_sample_cloud", "ope_voxel_grid",
-    "ope_normals_knn", "ope_fpfh", "ope_feature_knn",
+    "ope_normals_knn", "ope_normals_radius", "ope_fpfh", "ope_feature_knn",
     "ope_umeyama", "ope_point_to_plane", "ope_fitness", "ope_correspondences", "ope_icp_align", "ope_icp_align_fixed", "ope_sacia_align", "ope_sacia_align_sharded",
     "ope_comm_unique_id", "ope_comm_nccl_version", "ope_comm_create", "ope_comm_destroy", "ope_comm_rank", "ope_comm_world", "ope_sacia_draw",
     "ope_pose_tracker_create", "ope_pose_tracker_destroy", "ope_pose_estimate_final", "ope_pose_estimate_final_device", "ope_pose_batch", "ope_pose_tracker_step_batch",
@@ -372,7 +372,7 @@ class Context:
 
     # ---- search ----
     def knn(self, tgt, qry, k):
-        """tgt: Cloud; qry: Cloud or (N,>=3) array."""
+        """tgt: Cloud; qry: Cloud or (N,>=3) array; 1 <= k <= 256 (OPE_KNN_MAX_K)."""
         nq = len(qry)
         idx = np.empty((nq, k), np.int32)
         d2 = np.empty((nq, k), np.float32)
@@ -436,6 +436,13 @@ class Context:
         out = np.empty((len(cloud), 4), np.float32)
         v = (C.c_float * 3)(*vp)
         self._chk(lib().ope_normals_knn(self.h, cloud.h, k, v, out.ctypes.data_as(f32p)))
+        return out
+
+    def normals_radius(self, cloud, r, vp=(0, 0, 0)):
+        """NormalEstimation with setRadiusSearch(r): (n, 4) nx, ny, nz, curvature; also written into the cloud."""
+        out = np.empty((len(cloud), 4), np.float32)
+        v = (C.c_float * 3)(*vp)
+        self._chk(lib().ope_normals_radius(self.h, cloud.h, C.c_float(r), v, out.ctypes.data_as(f32p)))
         return out
 
     def fpfh(self, cloud, r, want_spfh=False):
