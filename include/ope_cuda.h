@@ -230,7 +230,12 @@ int ope_umeyama(ope_ctx* ctx, const ope_cloud* src, const ope_cloud* tgt, const 
 /* TransformationEstimationPointToPlaneLLS (kind = OPE_TE_POINT_TO_PLANE_LLS; the default of IterativeClosestPointWithNormals,
  * VP/icp_mod.h:352-357) and TransformationEstimationPointToPlane (kind = OPE_TE_POINT_TO_PLANE: Levenberg-Marquardt over the
  * 6-parameter rigid warp, what BuildModel sets, BM/src/regmeshpcd.cpp:162,193) ::estimateRigidTransformation [UPSTREAM].
- * tgt must carry normals. lm_info: 3 ints (Eigen LM status, function evaluations, iterations) or NULL. */
+ * tgt must carry normals. lm_info: 3 ints (Eigen LM status, function evaluations, iterations) or NULL.
+ * LM with fewer than 6 pairs returns the identity and lm_info (0, 0, 0): PCL refuses fewer than 4, and Eigen's minimizeInit
+ * refuses m < n (ImproperInputParameters) before any evaluation, which leaves x = 0.
+ * Deliberate deviation (LLS): PCL 1.7.2 solves x = ATA.inverse() * ATb, which is not finite when A^T A is exactly singular (all
+ * pairs on one plane, two planes or a cylinder when the sums are exact); an ICP loop would carry that NaN transform into every
+ * later iteration. Here the elimination stops at an exactly zero pivot and the result is the identity. */
 int ope_point_to_plane(ope_ctx* ctx, const ope_cloud* src, const ope_cloud* tgt, const int32_t* isrc, const int32_t* itgt, size_t n,
                        int kind, float T[16], int32_t* lm_info);
 

@@ -104,6 +104,22 @@ OPE_HD void xform_point(const Mat4& T, float x, float y, float z, float& ox, flo
   oy = T(1, 0) * x + T(1, 1) * y + T(1, 2) * z + T(1, 3);
   oz = T(2, 0) * x + T(2, 1) * y + T(2, 2) * z + T(2, 3);
 }
+// (warp(s) - t) . n as PCL's point-to-plane LM functor evaluates it: Vector4f with w = 0, Eigen's packet reduction with SSE3+
+// horizontal adds, (p0 + p1) + (p2 + p3) — the one Eigen model of the whole path (DESIGN.md section 2)
+OPE_HD float plane_residual(const Mat4& W, const float4 s, const float4 t, const float4 n) {
+  float wx, wy, wz;
+  xform_point(W, s.x, s.y, s.z, wx, wy, wz);
+  const float p0 = (wx - t.x) * n.x, p1 = (wy - t.y) * n.y, p2 = (wz - t.z) * n.z;
+  return (p0 + p1) + (p2 + 0.0f);
+}
+// one row of TransformationEstimationPointToPlaneLLS's A x = b: (s x n, n) and n . t - n . s, float products widened
+OPE_HD void plane_lls_row(const float4 s, const float4 t, const float4 n, double v[6], double& d) {
+  v[0] = (double)(n.z * s.y - n.y * s.z);
+  v[1] = (double)(n.x * s.z - n.z * s.x);
+  v[2] = (double)(n.y * s.x - n.x * s.y);
+  v[3] = (double)n.x; v[4] = (double)n.y; v[5] = (double)n.z;
+  d = (double)(n.x * t.x + n.y * t.y + n.z * t.z - n.x * s.x - n.y * s.y - n.z * s.z);
+}
 OPE_HD void xform_normal(const Mat4& T, float x, float y, float z, float& ox, float& oy, float& oz) {
   ox = T(0, 0) * x + T(0, 1) * y + T(0, 2) * z;
   oy = T(1, 0) * x + T(1, 1) * y + T(1, 2) * z;

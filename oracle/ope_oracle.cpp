@@ -372,7 +372,8 @@ void warpRigid6D(const float x[6], Mat4& M) {
 // TransformationEstimationPointToPlane [UPSTREAM transformation_estimation_point_to_plane.h + transformation_estimation_lm.hpp],
 // the estimator BuildModel plugs into IterativeClosestPointWithNormals (BM/src/regmeshpcd.cpp:162,193):
 // residual_i = (warp(src_i) - tgt_i) . n_tgt_i, minimised over the 6 warp parameters by Eigen's Levenberg-Marquardt with a
-// forward-difference Jacobian, starting from x = 0. Fewer than 4 pairs: PCL_ERROR and the identity.
+// forward-difference Jacobian, starting from x = 0. Fewer than 4 pairs: PCL_ERROR and the identity; 4 or 5: lmMinimize refuses
+// m < n (ImproperInputParameters) and x stays 0, the identity too.
 orc::LmRoute g_lm_route = orc::LM_ROUTE_NORMAL_EQ;   // orc_lm_set_route(): the Householder route is a cross-check
 
 void pointToPlaneLM(const CloudView& src, const CloudView& tgt, const std::vector<ope_correspondence>& corr, float T[16],

@@ -11,7 +11,11 @@
 //   LM_ROUTE_HOUSEHOLDER  factors the full m x n Jacobian by Householder reflections, as Eigen's ColPivHouseholderQR does;
 //   LM_ROUTE_NORMAL_EQ    (default, the canonical one) accumulates J^T J and J^T f in double — sums that do not depend on
 //                         the order of the rows to 1e-16 — and takes R as the pivoted Cholesky factor, Q^T f = R^-T P^T J^T f.
-// They agree to ~1e-10 relative (cond(J)^2 * eps); tests/test_oracle.py checks that. The canonical route is the second one
+// Where every direction of the 6 parameters is well observed they take the same steps to the same pose (within 1e-6 rad /
+// 1e-7 m; tests/test_oracle.py and tests/test_gpu_transform_estimation.py::test_lm_routes_envelope check that). Where a
+// direction is unobservable (pairs on one plane: rotation about its normal) or nearly so (a sphere 30 m from the origin:
+// rotation about its centre; the normal equations square cond(J)), the routes may take different steps and stop at
+// different points along that direction with the same residual norm. The canonical route is the second one
 // because an ICP loop around LM amplifies last-bit differences of one solve (the forward-difference Jacobian of float
 // residuals is noisy and LM stops at sqrt(eps_float) tolerances), so the oracle and anything compared with it must agree on
 // the sums to rounding, which only order-independent accumulation gives.

@@ -1,6 +1,7 @@
 // tests/hostemu/hostemu.cpp — TEST INFRASTRUCTURE. Compiles the product's OPE_HD device functions
 // (csrc/ope_device.cuh, csrc/ope_grid.cuh) with the HOST compiler so their per-query logic (ring search
-// termination, tie order, eigen33, pair features, SVD) can be checked against the oracle without a GPU.
+// termination, tie order, eigen33, pair features, SVD) can be checked against the oracle without a GPU, and
+// the host half of the point-to-plane estimators (csrc/ope_p2plane.h) against a serial accumulator.
 // The grid is built serially here with the same binning formula as csrc/grid.cu. Never shipped, never loaded
 // by the product.
 #include <algorithm>
@@ -12,6 +13,7 @@ using std::isfinite;
 static long g_counts[4] = {0, 0, 0, 0};
 #define OPE_COUNT(what) (g_counts[what]++)
 #include "../../object-pose-estimation_b200/csrc/ope_grid.cuh"
+#include "../../object-pose-estimation_b200/csrc/ope_p2plane.h"
 
 using namespace ope;
 
@@ -51,6 +53,43 @@ void build(const float* xyz, int n, float h_wanted, HostGrid& g) {
     g.sorted[cur[grid_cell_code(g.v, p[0], p[1], p[2])]++] = make_float4(p[0], p[1], p[2], i2f(i));
   }
   g.v.start = g.cell_start.data(); g.v.pts = g.sorted.data();
+}
+
+// the sums p2plane.cu's kernels reduce, taken pair after pair: what the device returns whenever the double sums are exact
+struct SerialP2p {
+  std::vector<float4> s, t, nr;
+  double out[28];
+  int jacobian(const Mat4 W[7], const float h[6], const double** r) {
+    for (double& v : out) v = 0.0;
+    for (size_t i = 0; i < s.size(); ++i) {
+      const float f = plane_residual(W[0], s[i], t[i], nr[i]);
+      double J[6];
+      for (int j = 0; j < 6; ++j) J[j] = (double)((plane_residual(W[1 + j], s[i], t[i], nr[i]) - f) / h[j]);
+      int e = 0;
+      for (int a = 0; a < 6; ++a)
+        for (int b = a; b < 6; ++b) out[e++] += J[a] * J[b];
+      for (int a = 0; a < 6; ++a) out[21 + a] += J[a] * (double)f;
+      out[27] += (double)f * (double)f;
+    }
+    *r = out;
+    return 0;
+  }
+  int residual(const Mat4& W, const double** r) {
+    out[0] = 0.0;
+    for (size_t i = 0; i < s.size(); ++i) { const float f = plane_residual(W, s[i], t[i], nr[i]); out[0] += (double)f * (double)f; }
+    *r = out;
+    return 0;
+  }
+};
+
+SerialP2p p2p_pairs(const float* s, const float* t, const float* n, int m) {
+  SerialP2p a;
+  for (int i = 0; i < m; ++i) {
+    a.s.push_back(make_float4(s[3 * i], s[3 * i + 1], s[3 * i + 2], 1.0f));
+    a.t.push_back(make_float4(t[3 * i], t[3 * i + 1], t[3 * i + 2], 1.0f));
+    a.nr.push_back(make_float4(n[3 * i], n[3 * i + 1], n[3 * i + 2], 0.0f));
+  }
+  return a;
 }
 }  // namespace
 
@@ -140,6 +179,40 @@ void emu_umeyama_moments(const float* s, const float* d, int n, float* T16) {
     for (int c = 0; c < 3; ++c) for (int r = 0; r < 3; ++r) acc[7 + c * 3 + r] += (double)d[3 * i + r] * (double)s[3 * i + c];
   }
   Mat4 M; umeyama_from_moments(acc, M); std::memcpy(T16, M.m, 64);
+}
+
+
+// TransformationEstimationPointToPlane (LM) over the pairs (s[i], t[i], n[i]), xyz rows: p2plane.cu's host driver.
+// info: (status, nfev, iterations); trace: (smallest Jacobian rank, smallest qrsolv nsing) the driver met.
+int emu_p2p_lm(const float* s, const float* t, const float* n, int m, float* T16, int32_t* info, int32_t* trace) {
+  SerialP2p acc = p2p_pairs(s, t, n, m);
+  p2p::LmTrace tr;
+  Mat4 T;
+  const int rc = p2p::lm_estimate(acc, m, &T, info, &tr);
+  std::memcpy(T16, T.m, 64);
+  trace[0] = tr.min_rank; trace[1] = tr.min_nsing;
+  return rc;
+}
+
+// TransformationEstimationPointToPlaneLLS: the device kernel's rows (non-finite ones skipped) + p2plane.cu's host solve.
+// Returns whether the 6x6 system had no exactly zero pivot.
+int emu_p2p_lls(const float* s, const float* t, const float* n, int m, float* T16) {
+  SerialP2p a = p2p_pairs(s, t, n, m);
+  double r[27];
+  for (double& v : r) v = 0.0;
+  for (int i = 0; i < m; ++i) {
+    if (!finite3(a.s[i].x, a.s[i].y, a.s[i].z) || !finite3(a.t[i].x, a.t[i].y, a.t[i].z) || !finite3(a.nr[i].x, a.nr[i].y, a.nr[i].z)) continue;
+    double v[6], d;
+    plane_lls_row(a.s[i], a.t[i], a.nr[i], v, d);
+    int e = 0;
+    for (int p = 0; p < 6; ++p)
+      for (int q = p; q < 6; ++q) r[e++] += v[p] * v[q];
+    for (int p = 0; p < 6; ++p) r[21 + p] += v[p] * d;
+  }
+  bool solved;
+  const Mat4 T = p2p::lls_transform(r, &solved);
+  std::memcpy(T16, T.m, 64);
+  return solved ? 1 : 0;
 }
 
 }  // extern "C"
