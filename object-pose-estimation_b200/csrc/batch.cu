@@ -408,7 +408,7 @@ static int fine_stage(ope_ctx* ctx, const ope_pose_params& P, int B, const Batch
   for (int i = 0; i < B; ++i) {
     if (!h_active[(size_t)i]) continue;
     const int nt = h_cc[(size_t)i], nsrc = h_cc[(size_t)B + i];
-    if (nt < P.min_target_points || !icp_small_batch_applicable(P.icp, (size_t)nsrc, (size_t)nt)) { h_active[(size_t)i] = 0; continue; }
+    if (nt < P.min_target_points || !icp_small_applicable(P.icp, (size_t)nsrc, (size_t)nt)) { h_active[(size_t)i] = 0; continue; }
     IcpBatchFrame fr;
     fr.tgt_pts = fine_pts + slab + (size_t)i * kBCap; fr.tgt_nrm = fine_nrm + slab + (size_t)i * kBCap; fr.n_tgt = nt;
     fr.src_pts = fine_pts + 2 * slab + (size_t)i * kBCap; fr.src_nrm = fine_nrm + 2 * slab + (size_t)i * kBCap; fr.n_src = nsrc;

@@ -354,7 +354,7 @@ int feature_knn_batch(ope_ctx* ctx, const float* ftgt, const int* d_counts, int 
 int sacia_batch_device(ope_ctx* ctx, const SaciaBatch& a, int frames, int max_nt, const GridView* grid, ope_reg_result* d_results);
 int fitness_batch_device(ope_ctx* ctx, const float4* tgt, const int* tgt_counts, const float4* src, const int* src_counts, int stride, int frames,
                          int max_nt, const ope_reg_result* d_icp, const int* d_active, double* d_out);
-bool icp_small_batch_applicable(const ope_icp_params& prm, size_t n_src, size_t n_tgt);
+bool icp_small_applicable(const ope_icp_params& prm, size_t n_src, size_t n_tgt);
 int icp_small_batch_device(ope_ctx* ctx, const ope_icp_params& prm, const IcpBatchFrame* frames, int n_frames, ope_reg_result* d_results);
 
 // one tracker's state commit (track_commit_kernel): the new alignedSource and the copy that replaces the source, and the dense
@@ -413,6 +413,8 @@ int pose_chunk(ope_ctx* ctx, const ope_pose_params& P, int B, PoseChunk& c, cons
 ope_pose_result chunk_pose_result(const PoseChunk& c, int i, const Mat4& rigid);
 
 // ---- pipeline.cu: the lanes of the frame-spanning batches (see there) ----
+// at most this many lanes run at once: the thread-per-query ICP launch checks that the device holds their blocks (registration.cu)
+static constexpr int kMaxLanes = 8;
 int run_chunks_on_lanes(ope_ctx* ctx, size_t n, const std::atomic<int>* stop,
                         const std::function<int(ope_ctx*, size_t, size_t, size_t)>& run_chunk, size_t chunk_items = 0);
 

@@ -291,7 +291,7 @@ int run_chunks_on_lanes(ope_ctx* ctx, size_t n, const std::atomic<int>* stop,
   const char* ce = std::getenv("OPE_BATCH_CHUNK");
   const char* le = std::getenv("OPE_BATCH_LANES");
   // lanes: one host thread each, plus the thread that draws the tables — as many as this process has cores for (its affinity
-  // mask, shared with the other ranks of a torchrun-style launch on the same node), at most 8
+  // mask, shared with the other ranks of a torchrun-style launch on the same node), at most kMaxLanes
   int cores = (int)std::thread::hardware_concurrency();
   {
     cpu_set_t set;
@@ -300,7 +300,7 @@ int run_chunks_on_lanes(ope_ctx* ctx, size_t n, const std::atomic<int>* stop,
     const char* lw = std::getenv("LOCAL_WORLD_SIZE");
     if (lw && std::atoi(lw) > 1) cores = std::max(1, cores / std::atoi(lw));
   }
-  int lanes = std::max(1, std::min(le ? std::atoi(le) : std::max(2, cores - 1), 8));
+  int lanes = std::max(1, std::min(le ? std::atoi(le) : std::max(2, cores - 1), kMaxLanes));
   if (ctx->batch_timing) lanes = 1;   // per-stage device times are only meaningful when the stages do not share the device
   size_t chunk = chunk_items ? chunk_items : (size_t)std::max(1, ce ? std::atoi(ce) : 296);
   if (!ce && !chunk_items) {
@@ -512,7 +512,7 @@ int ope_pose_batch(ope_ctx* ctx, const ope_pose_params* prm, const float* model_
   // ---- frame-spanning launches (batch.cu): one launch per stage for a whole chunk of frames; the frames outside their envelope
   // (tiny / empty / oversized clusters, or every frame when the ICP parameters are outside it) are collected for a second pass ----
   // normal_k above 32 is outside the frame-spanning normal kernel: every frame then runs on the per-frame path
-  const bool fast = icp_small_batch_applicable(P.icp, 1, 1) && P.icp.n_rejectors >= 0 && P.normal_k <= 32;
+  const bool fast = icp_small_applicable(P.icp, 1, 1) && P.icp.n_rejectors >= 0 && P.normal_k <= 32;
   std::mutex frame_mu;
   std::vector<size_t> rest;
   int lrc = run_chunks_on_lanes(ctx, n_frames, &draw_rc, [&](ope_ctx* c, size_t f0, size_t nf, size_t) -> int {

@@ -272,8 +272,6 @@ struct IcpDev {
   int tgt_in_smem;            // normal shooting against a small target: the target lives in shared memory (warp_knn_smem)
   int n_tgt;                  // points in the target cloud
   int split_min;              // far queries with more candidate points than this are split by start node
-  int small_max;              // unused (an octet queue for small far queries was measured on C2 and lost: the octets of one warp
-                              // diverge — every query has its own control flow — and serialise; every far query gets a warp)
   float4* def_q;              // far-query queue: x, y, z, seed d2          (block b's segment starts at its slice)
   int4* def_m;                //                  sorted position, seed index, original index, start node (-1: all)
   float4* def_res;            // result of a queue entry: d1, i1 (bits), s2, r2
@@ -901,7 +899,7 @@ __global__ void __launch_bounds__(kIcpThreads, 1) icp_kernel(IcpDev a) {
 // ================================================================ ICP, small clouds: one source point per THREAD ====
 // The DetectAndLocalize fine stage (normal shooting, k = 20) works on ~2 k source points against a ~1.5 k point cluster. The
 // kernel above gives every such query a whole warp and the whole GPU to one alignment; this one keeps the target in shared
-// memory and gives every query ONE thread, so an alignment needs ceil(n / 512) blocks (4 SMs instead of 118) and a batch of
+// memory and gives every query ONE thread, so an alignment needs ceil(n / 256) blocks (8 SMs instead of 118) and a batch of
 // independent frames (ope_pose_batch) fills the device with concurrent alignments.
 //   per iteration and thread: bound = largest distance to the previous iteration's k neighbours (tight: they are still the k
 //   nearest for almost every point) -> one pass over the target in shared memory (broadcast reads) collecting the points within
@@ -911,10 +909,11 @@ __global__ void __launch_bounds__(kIcpThreads, 1) icp_kernel(IcpDev a) {
 //   The rare query whose bound admits more than kSlabSlots points, and the first (unseeded) iteration, use the cooperative
 //   warp_knn_smem for that query. Same results as icp_kernel (parity tests run both).
 static constexpr int kSlabSlots = 32;
-static constexpr int kIcpSmallMaxBlocks = 32;
-
-static constexpr int kIcpSmallThreads = 128;   // 4 warps: the per-target scan is a latency chain, so a block gains little from more
-                                               // warps; small blocks let the blocks of SEVERAL alignments share an SM
+// A block keeps its alignment's target (points + group boxes) in shared memory next to 256 bytes of candidate slots per thread,
+// so wider blocks share one target copy among more warps: 2 x 256 threads fit an SM where 3 x 128 do (16 resident warps instead
+// of 12 of this latency-bound kernel). Up to 16 blocks: 4 096 source points.
+static constexpr int kIcpSmallThreads = 256;
+static constexpr int kIcpSmallMaxBlocks = 16;
 // A thread's column of the candidate slab (entries THREADS apart) as a binary max-heap in (d2, index) order: v sinks from node i
 // of a heap of n entries.
 template <int THREADS>
@@ -1315,10 +1314,6 @@ __device__ __forceinline__ void icp_small_body(const IcpDev& a, const int bid, c
   }
 }
 
-template <int THREADS>
-__global__ void __launch_bounds__(THREADS, 512 / THREADS) icp_small_kernel(IcpDev a) {
-  icp_small_body<THREADS>(a, (int)blockIdx.x, (int)gridDim.x);
-}
 // Frame-spanning launch: every block takes a ticket and looks up (alignment, block-in-alignment) in a host-built map that lists
 // the blocks alignment by alignment. Tickets are handed out in the order blocks START, so when a block spins on its alignment's
 // barrier, every block it waits for either runs already or is next in line for the first free slot — which the alignments ahead
@@ -1916,16 +1911,35 @@ int fitness_device(ope_ctx* ctx, const ope_cloud* src, const ope_cloud* tgt, con
   return OPE_OK;
 }
 
-static int icp_fill(ope_ctx* ctx, const ope_cloud* src, const ope_cloud* tgt, const ope_icp_params& prm, IcpDev* a,
-                    bool allow_smem_target = false) {
-  const bool need_src_normals = prm.estimator == OPE_EST_NORMAL_SHOOTING || prm.n_rejectors > 0;
-  bool need_tgt_normals = false;
-  for (int r = 0; r < prm.n_rejectors; ++r) {
+// The parameter fields of every ICP path's descriptor: iterations, convergence thresholds and the rejector chain (checked)
+static int icp_fill_params(ope_ctx* ctx, const ope_icp_params& prm, IcpDev* a) {
+  if (prm.n_rejectors < 0 || prm.n_rejectors > OPE_MAX_REJECTORS) return fail(ctx, OPE_ERR_INVALID, "bad rejector count");
+  for (int r = 0; r < prm.n_rejectors; ++r)
     if (prm.rejector_kind[r] != OPE_REJ_SURFACE_NORMAL && prm.rejector_kind[r] != OPE_REJ_SELF_OCCLUDED_NORMAL)
       return fail(ctx, OPE_ERR_UNSUPPORTED, "unknown correspondence rejector kind %d", prm.rejector_kind[r]);
+  a->max_iterations = prm.max_iterations; a->min_corr = prm.min_number_correspondences;
+  a->estimator = prm.estimator; a->k_search = prm.k_search; a->n_rej = prm.n_rejectors;
+  a->transformation = prm.transformation; a->variant = prm.variant; a->force_all = prm.force_all_iterations;
+  for (int r = 0; r < OPE_MAX_REJECTORS; ++r) { a->rej_kind[r] = prm.rejector_kind[r]; a->rej_thr[r] = prm.rejector_threshold[r]; }
+  a->max_corr_dist = prm.max_correspondence_distance;
+  const double m2 = prm.max_correspondence_distance * prm.max_correspondence_distance;
+  a->max_d2_f = (m2 >= (double)FLT_MAX || !(m2 == m2)) ? FLT_MAX : (float)m2;
+  a->rot_thr = 1.0 - prm.transformation_epsilon;
+  a->trans_thr = prm.transformation_epsilon;
+  a->rel_mse_thr = prm.euclidean_fitness_epsilon;
+  a->abs_mse_thr = prm.mse_threshold_absolute;
+  a->max_similar = prm.max_iterations_similar_transforms;
+  a->fail_after_max = prm.failure_after_max_iterations;
+  return OPE_OK;
+}
+
+static int icp_fill(ope_ctx* ctx, const ope_cloud* src, const ope_cloud* tgt, const ope_icp_params& prm, IcpDev* a,
+                    bool allow_smem_target = false) {
+  OPE_TRY(icp_fill_params(ctx, prm, a));
+  const bool need_src_normals = prm.estimator == OPE_EST_NORMAL_SHOOTING || prm.n_rejectors > 0;
+  bool need_tgt_normals = false;
+  for (int r = 0; r < prm.n_rejectors; ++r)
     if (prm.rejector_kind[r] == OPE_REJ_SURFACE_NORMAL) need_tgt_normals = true;
-  }
-  if (prm.n_rejectors < 0 || prm.n_rejectors > OPE_MAX_REJECTORS) return fail(ctx, OPE_ERR_INVALID, "bad rejector count");
   if (need_src_normals && !src->normals) return fail(ctx, OPE_ERR_INVALID, "estimator/rejector needs source normals");
   if (need_tgt_normals && !tgt->normals) return fail(ctx, OPE_ERR_INVALID, "rejector needs target normals");
   if (prm.use_reciprocal && prm.estimator != OPE_EST_NEAREST)
@@ -1949,19 +1963,6 @@ static int icp_fill(ope_ctx* ctx, const ope_cloud* src, const ope_cloud* tgt, co
   a->tgt_pts = tgt->pts; a->tgt_nrm = tgt->normals;
   a->src0_pts = src->pts; a->src0_nrm = src->normals;
   a->n_src = (int)src->n;
-  a->max_iterations = prm.max_iterations; a->min_corr = prm.min_number_correspondences;
-  a->estimator = prm.estimator; a->k_search = prm.k_search; a->n_rej = prm.n_rejectors;
-  a->transformation = prm.transformation; a->variant = prm.variant; a->force_all = prm.force_all_iterations;
-  for (int r = 0; r < OPE_MAX_REJECTORS; ++r) { a->rej_kind[r] = prm.rejector_kind[r]; a->rej_thr[r] = prm.rejector_threshold[r]; }
-  a->max_corr_dist = prm.max_correspondence_distance;
-  const double m2 = prm.max_correspondence_distance * prm.max_correspondence_distance;
-  a->max_d2_f = (m2 >= (double)FLT_MAX || !(m2 == m2)) ? FLT_MAX : (float)m2;
-  a->rot_thr = 1.0 - prm.transformation_epsilon;
-  a->trans_thr = prm.transformation_epsilon;
-  a->rel_mse_thr = prm.euclidean_fitness_epsilon;
-  a->abs_mse_thr = prm.mse_threshold_absolute;
-  a->max_similar = prm.max_iterations_similar_transforms;
-  a->fail_after_max = prm.failure_after_max_iterations;
   return OPE_OK;
 }
 
@@ -1976,6 +1977,125 @@ static int icp_stepwise_device(ope_ctx* ctx, const ope_cloud* src, const ope_clo
                                ope_reg_result* res, ope_correspondence* out_corr_host, ope_cloud** out_aligned,
                                ope_correspondence* fixed = nullptr, size_t n_fixed = 0);
 
+// The thread-per-query ICP (icp_small_batch_kernel) takes normal shooting with SVD, k <= 32 and, per alignment, up to 4 096 finite
+// source points against a target of up to 4 096 points in shared memory.
+bool icp_small_applicable(const ope_icp_params& prm, size_t n_src, size_t n_tgt) {
+  return prm.estimator == OPE_EST_NORMAL_SHOOTING && prm.transformation == OPE_TE_SVD && !prm.use_reciprocal && n_tgt > 0 &&
+         n_tgt <= (size_t)kIcpSmemMaxTargets && n_src > 0 && n_src <= (size_t)kIcpSmallMaxBlocks * kIcpSmallThreads &&
+         prm.k_search >= 1 && prm.k_search <= kSlabSlots;
+}
+
+// Runs the alignments descs[0, n) in one launch of icp_small_batch_kernel; the caller fills every descriptor but its partials
+// and barrier, within icp_small_applicable. One alignment is a cooperative launch, so its blocks are co-resident whatever else
+// runs on the device. More are ticketed (see the kernel), which counts on the residency bound checked below.
+static int icp_small_launch(ope_ctx* ctx, IcpDev* descs, int n) {
+  const bool trace = std::getenv("OPE_BATCH_TRACE") != nullptr;
+  auto now = [] { return std::chrono::steady_clock::now(); };
+  auto ms_since = [&](std::chrono::steady_clock::time_point t) { return std::chrono::duration<double, std::milli>(now() - t).count(); };
+  const auto t_enter = now();
+  auto smem_bytes = [](size_t n_tgt) {   // block state, the target in groups of 8 with a box per group, the candidate slab
+    const size_t nt8 = (n_tgt + 7) & ~(size_t)7;
+    return ((sizeof(IcpSmallSmem<kIcpSmallThreads>) + 15) & ~(size_t)15) + nt8 * sizeof(float4) + (nt8 / 8) * 2 * sizeof(float4) +
+           (size_t)kSlabSlots * kIcpSmallThreads * sizeof(float2);
+  };
+  const void* kernel = (const void*)icp_small_batch_kernel<kIcpSmallThreads>;
+  // A ticketed block spins on its alignment's barrier, and up to kMaxLanes lanes launch this kernel at once: each lane can park
+  // all but one block of an alignment, and the device must still hold one more alignment whole. Counted at the largest target
+  // the envelope admits, so the bound holds whatever the other lanes launch.
+  const size_t smem_max = smem_bytes(kIcpSmemMaxTargets);
+  OPE_TRY(dyn_smem(ctx, kernel, smem_max));
+  int per_sm = 0;
+  OPE_CUDA_TRY(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kIcpSmallThreads, smem_max));
+  if (kMaxLanes * (kIcpSmallMaxBlocks - 1) + kIcpSmallMaxBlocks > per_sm * ctx->sm_count)
+    return fail(ctx, OPE_ERR_CUDA, "icp_small_batch_kernel: %d resident blocks cannot hold %d lanes of %d-block alignments",
+                per_sm * ctx->sm_count, kMaxLanes, kIcpSmallMaxBlocks);
+  size_t max_nt = 0, total_blocks = 0;
+  for (int i = 0; i < n; ++i) {
+    max_nt = std::max(max_nt, (size_t)descs[i].n_tgt);
+    total_blocks += div_up((size_t)descs[i].n_work, kIcpSmallThreads);
+  }
+  Scratch<double> partials(ctx);
+  Scratch<unsigned> bars(ctx);
+  Scratch<IcpDev> d_descs(ctx);
+  Scratch<int2> d_map(ctx);
+  OPE_TRY(partials.alloc(2 * total_blocks * kIcpAcc));
+  OPE_TRY(bars.alloc((size_t)n + 1));   // the alignments' barriers, then the ticket counter
+  OPE_TRY(d_descs.alloc((size_t)n)); OPE_TRY(d_map.alloc(total_blocks));
+  OPE_CUDA_TRY(ctx, cudaMemsetAsync(bars.p, 0, ((size_t)n + 1) * sizeof(unsigned), ctx->stream));
+  std::vector<int2> map;
+  map.reserve(total_blocks);
+  for (int i = 0; i < n; ++i) {
+    descs[i].partials = partials.p + 2 * map.size() * kIcpAcc;
+    descs[i].barrier = bars.p + i;
+    for (int b = 0; b * kIcpSmallThreads < descs[i].n_work; ++b) map.push_back(make_int2(i, b));
+  }
+  OPE_CUDA_TRY(ctx, cudaMemcpyAsync(d_descs.p, descs, (size_t)n * sizeof(IcpDev), cudaMemcpyHostToDevice, ctx->stream));
+  OPE_CUDA_TRY(ctx, cudaMemcpyAsync(d_map.p, map.data(), map.size() * sizeof(int2), cudaMemcpyHostToDevice, ctx->stream));
+  const double t_prep = ms_since(t_enter);
+  OPE_CUDA_TRY(ctx, ope::stream_sync(ctx));   // map and the caller's descs are gone or reused after the return
+  if (trace) fprintf(stderr, "[ope batch] icp launch: host preparation %.3f ms, then %.3f ms until the stream had drained\n", t_prep, ms_since(t_enter) - t_prep);
+  unsigned* ticket = bars.p + n;
+  void* args[] = {(void*)&d_descs.p, (void*)&d_map.p, (void*)&ticket};
+  const dim3 grid((unsigned)total_blocks), block(kIcpSmallThreads);
+  const size_t smem = smem_bytes(max_nt);
+  cudaEventRecord(ctx->kev[0][0], ctx->stream);
+  const cudaError_t e = n == 1 ? cudaLaunchCooperativeKernel(kernel, grid, block, args, smem, ctx->stream)
+                               : cudaLaunchKernel(kernel, grid, block, args, smem, ctx->stream);
+  cudaEventRecord(ctx->kev[0][1], ctx->stream);
+  ctx->kev_valid[0] = true;
+  if (e != cudaSuccess) return fail(ctx, OPE_ERR_CUDA, "launch of icp_small_batch_kernel failed: %s", cudaGetErrorString(e));
+  return check_launch(ctx, "icp_small_batch_kernel");
+}
+
+// icp_kernel on descriptor a (filled but for its search scratch, partials and barrier): one persistent cooperative launch, its
+// grid (*blocks) sized by the query count and capped by co-residency and ctx->icp_max_blocks
+static int icp_kernel_launch(ope_ctx* ctx, IcpDev a, int* blocks) {
+  const bool shooting = a.estimator == OPE_EST_NORMAL_SHOOTING;
+  const size_t nw = (size_t)a.n_work;
+  const size_t smem_bytes = ((sizeof(IcpSmem) + 15) & ~(size_t)15) + (a.tgt_in_smem ? (size_t)a.n_tgt * sizeof(float4) : 0);
+  Scratch<int> seed(ctx), dcount(ctx), dhead(ctx);
+  Scratch<float4> defq(ctx), refs(ctx), defres(ctx);
+  Scratch<int4> defm(ctx);
+  Scratch<double> partials(ctx);
+  Scratch<unsigned> bar(ctx);
+  OPE_TRY(seed.alloc(shooting ? nw * (size_t)a.k_search : nw));
+  if (!shooting) {
+    OPE_TRY(defq.alloc(nw)); OPE_TRY(defm.alloc(nw)); OPE_TRY(refs.alloc(nw)); OPE_TRY(defres.alloc(nw));
+  }
+  OPE_TRY(bar.alloc(1));
+  if (cudaMemsetAsync(bar.p, 0, sizeof(unsigned), ctx->stream) != cudaSuccess) return fail(ctx, OPE_ERR_CUDA, "memset failed");
+  OPE_TRY(dyn_smem(ctx, (const void*)icp_kernel, smem_bytes));
+  // cooperative grid: one point per thread (nearest) / per warp (normal shooting), capped by co-residency
+  int per_sm = 0;
+  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, icp_kernel, kIcpThreads, smem_bytes) != cudaSuccess)
+    return fail(ctx, OPE_ERR_CUDA, "occupancy query failed");
+  if (per_sm < 1) return fail(ctx, OPE_ERR_CUDA, "icp_kernel cannot be resident");
+  int max_blocks = std::min(per_sm * ctx->sm_count, kIcpMaxBlocks);
+  if (ctx->icp_max_blocks > 0) max_blocks = std::min(max_blocks, ctx->icp_max_blocks);
+  const size_t want = shooting ? (nw + kIcpWarps - 1) / kIcpWarps : (nw + 127) / 128;
+  *blocks = (int)std::min<size_t>(std::max<size_t>(1, want), (size_t)max_blocks);
+  OPE_TRY(partials.alloc((size_t)2 * *blocks * kIcpAcc));
+  OPE_TRY(dcount.alloc((size_t)2 * *blocks));
+  OPE_TRY(dhead.alloc(4));
+  if (cudaMemsetAsync(dhead.p, 0, 4 * sizeof(int), ctx->stream) != cudaSuccess) return fail(ctx, OPE_ERR_CUDA, "memset failed");
+  a.seed = seed.p; a.def_q = defq.p; a.def_m = defm.p; a.def_count = dcount.p;
+  a.ref = refs.p; a.def_head = dhead.p; a.def_res = defres.p;
+  const char* g = std::getenv("OPE_ICP_CERT_GAP");  // in target-grid cells; 0 disables the certificates (every query searches)
+  a.cert_gap = (g ? (float)std::atof(g) : 0.5f) * a.grid.h;
+  const char* d = std::getenv("OPE_ICP_DFS_MAX");
+  a.dfs_max = d ? std::atoi(d) : 0;   // measured: a single thread's traversal is a long dependent chain; the warp queue wins
+  const char* sp_ = std::getenv("OPE_ICP_SPLIT_MIN");
+  a.split_min = sp_ ? std::atoi(sp_) : kIcpSplitMin;
+  a.partials = partials.p; a.barrier = bar.p;
+  void* args[] = {(void*)&a};
+  cudaEventRecord(ctx->kev[0][0], ctx->stream);
+  cudaError_t e = cudaLaunchCooperativeKernel((const void*)icp_kernel, dim3(*blocks), dim3(kIcpThreads), args, smem_bytes, ctx->stream);
+  cudaEventRecord(ctx->kev[0][1], ctx->stream);
+  ctx->kev_valid[0] = true;
+  if (e != cudaSuccess) return fail(ctx, OPE_ERR_CUDA, "cooperative launch of icp_kernel failed: %s", cudaGetErrorString(e));
+  return check_launch(ctx, "icp_kernel");
+}
+
 int icp_device(ope_ctx* ctx, const ope_cloud* src, const ope_cloud* tgt, const ope_icp_params& prm, const Mat4& guess,
                ope_reg_result* res, ope_correspondence* out_corr_host, ope_cloud** out_aligned) {
   if (prm.transformation != OPE_TE_SVD || prm.use_reciprocal)
@@ -1984,7 +2104,6 @@ int icp_device(ope_ctx* ctx, const ope_cloud* src, const ope_cloud* tgt, const o
   std::memset(&a, 0, sizeof(a));
   OPE_TRY(icp_fill(ctx, src, tgt, prm, &a, /*allow_smem_target=*/true));
   a.guess = guess;
-  size_t smem_bytes = ((sizeof(IcpSmem) + 15) & ~(size_t)15) + (a.tgt_in_smem ? tgt->n * sizeof(float4) : 0);
   const size_t n = src->n;
   // the source in Morton order of its own (cached) grid: spatially coherent work order, finite points only
   GridView gsrc;
@@ -1997,66 +2116,14 @@ int icp_device(ope_ctx* ctx, const ope_cloud* src, const ope_cloud* tgt, const o
   OPE_TRY(cloud_alloc(ctx, std::max<size_t>(n, 1), src->normals != nullptr, &work));
   work->n = n;
   a.cur_pts = work->pts; a.cur_nrm = work->normals;
-  Scratch<int> match(ctx), seed(ctx), dcount(ctx), dhead(ctx);
+  Scratch<int> match(ctx);
   Scratch<float> d2(ctx);
-  Scratch<float4> defq(ctx), refs(ctx), defres(ctx);
-  Scratch<int4> defm(ctx);
-  Scratch<double> partials(ctx);
-  Scratch<unsigned> bar(ctx);
   Scratch<ope_reg_result> dres(ctx);
-  const bool shooting = prm.estimator == OPE_EST_NORMAL_SHOOTING;
   int rc = match.alloc(n);
   if (rc == OPE_OK) rc = d2.alloc(n);
-  if (rc == OPE_OK) rc = seed.alloc(shooting ? nw * (size_t)prm.k_search : nw);
-  if (rc == OPE_OK && !shooting) rc = defq.alloc(nw);
-  if (rc == OPE_OK && !shooting) rc = defm.alloc(nw);
-  if (rc == OPE_OK && !shooting) rc = refs.alloc(nw);
-  if (rc == OPE_OK && !shooting) rc = defres.alloc(nw);
   if (rc == OPE_OK) rc = dres.alloc(1);
-  if (rc == OPE_OK) rc = bar.alloc(1);
-  if (rc == OPE_OK && cudaMemsetAsync(bar.p, 0, sizeof(unsigned), ctx->stream) != cudaSuccess) rc = fail(ctx, OPE_ERR_CUDA, "memset failed");
   if (rc == OPE_OK && n > 0 && cudaMemsetAsync(match.p, 0xff, n * sizeof(int), ctx->stream) != cudaSuccess) rc = fail(ctx, OPE_ERR_CUDA, "memset failed");
   if (rc == OPE_OK && n > 0 && cudaMemsetAsync(d2.p, 0, n * sizeof(float), ctx->stream) != cudaSuccess) rc = fail(ctx, OPE_ERR_CUDA, "memset failed");
-  // small clouds against a shared-memory target: one point per thread, ceil(n / 512) blocks (icp_small_kernel)
-  // It trades the latency of one alignment (the wide kernel spreads it over the whole device) for device time per alignment,
-  // so it is what a batch of concurrent alignments wants (ope_pose_batch sets ctx->icp_prefer_small); OPE_ICP_SMALL=1/0 forces.
-  const char* small_env = std::getenv("OPE_ICP_SMALL");
-  const bool want_small = small_env ? std::atoi(small_env) != 0 : ctx->icp_prefer_small;
-  const bool small = want_small && a.tgt_in_smem && shooting && nw > 0 && nw <= (size_t)kIcpSmallMaxBlocks * kIcpSmallThreads &&
-                     prm.k_search <= kSlabSlots;
-  const void* kernel = small ? (const void*)icp_small_kernel<kIcpSmallThreads> : (const void*)icp_kernel;
-  const int threads = small ? kIcpSmallThreads : kIcpThreads;
-  if (small) {
-    const size_t nt8 = (tgt->n + 7) & ~(size_t)7;
-    smem_bytes = ((sizeof(IcpSmallSmem<kIcpSmallThreads>) + 15) & ~(size_t)15) + nt8 * sizeof(float4) + (nt8 / 8) * 2 * sizeof(float4) +
-                 (size_t)kSlabSlots * kIcpSmallThreads * sizeof(float2);
-    // Persistent blocks of many concurrent alignments must not fill an SM completely: the short kernels of the other stages
-    // (other frames of a batch) need registers and shared memory next to them. Asking for at least this much shared memory
-    // caps the residency at two blocks per SM.
-    const char* pad = std::getenv("OPE_ICP_SMALL_MIN_SMEM_KB");
-    const size_t min_bytes = (size_t)(pad ? std::atoi(pad) : 0) << 10;   // measured: no gain on B200 with 16-48 concurrent frames; off by default
-    if (smem_bytes < min_bytes) smem_bytes = min_bytes;
-  }
-  if (rc == OPE_OK) rc = dyn_smem(ctx, kernel, smem_bytes);
-  // cooperative grid: one point per thread (nearest) / per warp (normal shooting), capped by co-residency
-  int per_sm = 0;
-  if (rc == OPE_OK && cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, smem_bytes) != cudaSuccess)
-    rc = fail(ctx, OPE_ERR_CUDA, "occupancy query failed");
-  int blocks = 1;
-  if (rc == OPE_OK && small) {
-    if (per_sm < 1) rc = fail(ctx, OPE_ERR_CUDA, "icp_small_kernel cannot be resident");
-    blocks = (int)((nw + kIcpSmallThreads - 1) / kIcpSmallThreads);
-  } else if (rc == OPE_OK) {
-    if (per_sm < 1) rc = fail(ctx, OPE_ERR_CUDA, "icp_kernel cannot be resident");
-    int max_blocks = std::min(per_sm * ctx->sm_count, kIcpMaxBlocks);
-    if (ctx->icp_max_blocks > 0) max_blocks = std::min(max_blocks, ctx->icp_max_blocks);
-    const size_t want = shooting ? (nw + kIcpWarps - 1) / kIcpWarps : (nw + 127) / 128;
-    blocks = (int)std::min<size_t>(std::max<size_t>(1, want), (size_t)max_blocks);
-  }
-  if (rc == OPE_OK) rc = partials.alloc((size_t)2 * blocks * kIcpAcc);
-  if (rc == OPE_OK) rc = dcount.alloc((size_t)2 * blocks);
-  if (rc == OPE_OK) rc = dhead.alloc(4);
-  if (rc == OPE_OK && cudaMemsetAsync(dhead.p, 0, 4 * sizeof(int), ctx->stream) != cudaSuccess) rc = fail(ctx, OPE_ERR_CUDA, "memset failed");
   Scratch<long long> phases(ctx);
   const bool profile = std::getenv("OPE_PROFILE") != nullptr;
   const size_t n_prof = 16 + 64 * 8 + 64 + 64 * 4;
@@ -2064,28 +2131,15 @@ int icp_device(ope_ctx* ctx, const ope_cloud* src, const ope_cloud* tgt, const o
     rc = phases.alloc(n_prof); a.phase_cycles = phases.p;
     if (rc == OPE_OK) cudaMemsetAsync(phases.p, 0, n_prof * sizeof(long long), ctx->stream);
   }
-  a.corr_match = match.p; a.corr_d2 = d2.p; a.seed = seed.p; a.def_q = defq.p; a.def_m = defm.p; a.def_count = dcount.p;
-  a.ref = refs.p; a.def_head = dhead.p; a.def_res = defres.p;
-  {
-    const char* g = std::getenv("OPE_ICP_CERT_GAP");  // in target-grid cells; 0 disables the certificates (every query searches)
-    a.cert_gap = (g ? (float)std::atof(g) : 0.5f) * a.grid.h;
-    const char* d = std::getenv("OPE_ICP_DFS_MAX");
-    a.dfs_max = d ? std::atoi(d) : 0;   // measured: a single thread's traversal is a long dependent chain; the warp queue wins
-    const char* sp_ = std::getenv("OPE_ICP_SPLIT_MIN");
-    a.split_min = sp_ ? std::atoi(sp_) : kIcpSplitMin;
-    const char* sm_ = std::getenv("OPE_ICP_SMALL_MAX");
-    a.small_max = sm_ ? std::atoi(sm_) : 0;
-  }
-  a.partials = partials.p; a.barrier = bar.p; a.result = dres.p;
-  if (rc == OPE_OK) {
-    void* args[] = {(void*)&a};
-    cudaEventRecord(ctx->kev[0][0], ctx->stream);
-    cudaError_t e = cudaLaunchCooperativeKernel(kernel, dim3(blocks), dim3(threads), args, smem_bytes, ctx->stream);
-    cudaEventRecord(ctx->kev[0][1], ctx->stream);
-    ctx->kev_valid[0] = true;
-    if (e != cudaSuccess) rc = fail(ctx, OPE_ERR_CUDA, "cooperative launch of icp_kernel failed: %s", cudaGetErrorString(e));
-    else rc = check_launch(ctx, "icp_kernel");
-  }
+  a.corr_match = match.p; a.corr_d2 = d2.p; a.result = dres.p;
+  // Small clouds against a shared-memory target: one point per thread, a one-alignment run of the frame-spanning kernel.
+  // It trades the latency of one alignment (the wide kernel spreads it over the whole device) for device time per alignment,
+  // so it is what a batch of concurrent alignments wants (ope_pose_batch sets ctx->icp_prefer_small); OPE_ICP_SMALL=1/0 forces.
+  const char* small_env = std::getenv("OPE_ICP_SMALL");
+  const bool want_small = small_env ? std::atoi(small_env) != 0 : ctx->icp_prefer_small;
+  const bool small = want_small && a.tgt_in_smem && icp_small_applicable(prm, nw, tgt->n);
+  int blocks = (int)div_up(nw, kIcpSmallThreads);
+  if (rc == OPE_OK) rc = small ? icp_small_launch(ctx, &a, 1) : icp_kernel_launch(ctx, a, &blocks);
   if (rc == OPE_OK) {
     void* h;
     rc = read_back(ctx, dres.p, sizeof(ope_reg_result), &h);
@@ -2108,7 +2162,7 @@ int icp_device(ope_ctx* ctx, const ope_cloud* src, const ope_cloud* tgt, const o
             }
           }
         }
-        fprintf(stderr, "[ope profile] icp_small_kernel blocks=%d, block 0 cycles per iteration: search %.0f | rank+shoot+reject %.0f | moments+barrier %.0f | "
+        fprintf(stderr, "[ope profile] icp_small_batch_kernel blocks=%d, block 0 cycles per iteration: search %.0f | rank+shoot+reject %.0f | moments+barrier %.0f | "
                 "svd+transform %.0f | cooperative re-searches per iteration %.1f | candidates per query %.1f\n", blocks, c[0] / it, c[1] / it,
                 c[2] / it, c[3] / it, c[4] / it, c[5] / it / kIcpSmallThreads);
       }
@@ -2656,100 +2710,37 @@ int fitness_batch_device(ope_ctx* ctx, const float4* tgt, const int* tgt_counts,
 }
 
 // ICP-with-normals (normal shooting, small clouds) for many independent alignments in ONE launch. frames[i]: clouds with normals,
-// source points carrying their index in .w; results[i] on the device. Only alignments icp_small_kernel can run (see below).
-bool icp_small_batch_applicable(const ope_icp_params& prm, size_t n_src, size_t n_tgt) {
-  return prm.estimator == OPE_EST_NORMAL_SHOOTING && prm.transformation == OPE_TE_SVD && !prm.use_reciprocal && n_tgt > 0 &&
-         n_tgt <= (size_t)kIcpSmemMaxTargets && n_src > 0 && n_src <= (size_t)kIcpSmallMaxBlocks * kIcpSmallThreads &&
-         prm.k_search >= 1 && prm.k_search <= kSlabSlots;
-}
-template <int THREADS>
-static int icp_small_batch_launch(ope_ctx* ctx, const ope_icp_params& prm, const IcpBatchFrame* frames, int n_frames, ope_reg_result* d_results) {
+// source points carrying their index in .w; results[i] on the device. Only alignments icp_small_applicable admits.
+int icp_small_batch_device(ope_ctx* ctx, const ope_icp_params& prm, const IcpBatchFrame* frames, int n_frames, ope_reg_result* d_results) {
   if (n_frames <= 0) return OPE_OK;
-  const bool trace = std::getenv("OPE_BATCH_TRACE") != nullptr;
-  auto now = [] { return std::chrono::steady_clock::now(); };
-  auto ms_since = [&](std::chrono::steady_clock::time_point t) { return std::chrono::duration<double, std::milli>(now() - t).count(); };
-  const auto t_enter = now();
-  std::vector<IcpDev> descs((size_t)n_frames);
-  std::vector<int2> map;
-  size_t max_nt = 0, total_src = 0, total_blocks = 0;
+  size_t total_src = 0;
   for (int i = 0; i < n_frames; ++i) {
-    if (!icp_small_batch_applicable(prm, (size_t)frames[i].n_src, (size_t)frames[i].n_tgt)) return fail(ctx, OPE_ERR_UNSUPPORTED, "alignment %d does not fit the small-cloud ICP kernel", i);
-    max_nt = std::max(max_nt, (size_t)frames[i].n_tgt);
+    if (!icp_small_applicable(prm, (size_t)frames[i].n_src, (size_t)frames[i].n_tgt)) return fail(ctx, OPE_ERR_UNSUPPORTED, "alignment %d does not fit the small-cloud ICP kernel", i);
     total_src += (size_t)frames[i].n_src;
-    total_blocks += ((size_t)frames[i].n_src + THREADS - 1) / THREADS;
   }
+  IcpDev common;
+  std::memset(&common, 0, sizeof(common));
+  OPE_TRY(icp_fill_params(ctx, prm, &common));
+  common.tgt_in_smem = 1;
+  common.guess = mat4_identity();
   Scratch<int> match(ctx);
   Scratch<float> d2(ctx);
-  Scratch<double> partials(ctx);
-  Scratch<unsigned> bars(ctx);
-  Scratch<IcpDev> d_descs(ctx);
-  Scratch<int2> d_map(ctx);
   OPE_TRY(match.alloc(total_src)); OPE_TRY(d2.alloc(total_src));
-  OPE_TRY(partials.alloc(2 * total_blocks * kIcpAcc));
-  OPE_TRY(bars.alloc((size_t)n_frames + 1));
-  OPE_TRY(d_descs.alloc((size_t)n_frames)); OPE_TRY(d_map.alloc(total_blocks));
-  OPE_CUDA_TRY(ctx, cudaMemsetAsync(bars.p, 0, ((size_t)n_frames + 1) * sizeof(unsigned), ctx->stream));
-  size_t so = 0, bo = 0;
-  map.reserve(total_blocks);
+  std::vector<IcpDev> descs((size_t)n_frames, common);
+  size_t so = 0;
   for (int i = 0; i < n_frames; ++i) {
     IcpDev& a = descs[(size_t)i];
-    std::memset(&a, 0, sizeof(a));
     const IcpBatchFrame& f = frames[i];
     a.grid.n = f.n_tgt;      // every target point is finite (it survived the sampling and the NaN-normal filter)
-    a.tgt_in_smem = 1; a.n_tgt = f.n_tgt;
+    a.n_tgt = f.n_tgt;
     a.tgt_pts = f.tgt_pts; a.tgt_nrm = f.tgt_nrm;
     a.src0_pts = f.src_pts; a.src0_nrm = f.src_nrm; a.src_sorted = f.src_pts;
     a.n_src = f.n_src; a.n_work = f.n_src;
-    a.max_iterations = prm.max_iterations; a.min_corr = prm.min_number_correspondences;
-    a.estimator = prm.estimator; a.k_search = prm.k_search; a.n_rej = prm.n_rejectors;
-    a.transformation = prm.transformation; a.variant = prm.variant; a.force_all = prm.force_all_iterations;
-    for (int r = 0; r < OPE_MAX_REJECTORS; ++r) { a.rej_kind[r] = prm.rejector_kind[r]; a.rej_thr[r] = prm.rejector_threshold[r]; }
-    a.max_corr_dist = prm.max_correspondence_distance;
-    const double m2 = prm.max_correspondence_distance * prm.max_correspondence_distance;
-    a.max_d2_f = (m2 >= (double)FLT_MAX || !(m2 == m2)) ? FLT_MAX : (float)m2;
-    a.rot_thr = 1.0 - prm.transformation_epsilon; a.trans_thr = prm.transformation_epsilon;
-    a.rel_mse_thr = prm.euclidean_fitness_epsilon; a.abs_mse_thr = prm.mse_threshold_absolute;
-    a.max_similar = prm.max_iterations_similar_transforms; a.fail_after_max = prm.failure_after_max_iterations;
-    a.guess = mat4_identity();
-    const int nblk = (f.n_src + THREADS - 1) / THREADS;
     a.corr_match = match.p + so; a.corr_d2 = d2.p + so;
-    a.partials = partials.p + 2 * bo * kIcpAcc;
-    a.barrier = bars.p + i;
     a.result = d_results + i;
-    for (int b = 0; b < nblk; ++b) map.push_back(make_int2(i, b));
-    so += (size_t)f.n_src; bo += (size_t)nblk;
+    so += (size_t)f.n_src;
   }
-  for (int r = 0; r < prm.n_rejectors; ++r)
-    if (prm.rejector_kind[r] != OPE_REJ_SURFACE_NORMAL && prm.rejector_kind[r] != OPE_REJ_SELF_OCCLUDED_NORMAL)
-      return fail(ctx, OPE_ERR_UNSUPPORTED, "unknown correspondence rejector kind %d", prm.rejector_kind[r]);
-  OPE_CUDA_TRY(ctx, cudaMemcpyAsync(d_descs.p, descs.data(), descs.size() * sizeof(IcpDev), cudaMemcpyHostToDevice, ctx->stream));
-  OPE_CUDA_TRY(ctx, cudaMemcpyAsync(d_map.p, map.data(), map.size() * sizeof(int2), cudaMemcpyHostToDevice, ctx->stream));
-  const double t_prep = ms_since(t_enter);
-  OPE_CUDA_TRY(ctx, ope::stream_sync(ctx));   // descs / map live on this stack frame
-  if (trace) fprintf(stderr, "[ope batch] icp launch: host preparation %.3f ms, then %.3f ms until the stream had drained\n", t_prep, ms_since(t_enter) - t_prep);
-  const size_t nt8 = (max_nt + 7) & ~(size_t)7;
-  const size_t smem_bytes = ((sizeof(IcpSmallSmem<THREADS>) + 15) & ~(size_t)15) + nt8 * sizeof(float4) + (nt8 / 8) * 2 * sizeof(float4) +
-                            (size_t)kSlabSlots * THREADS * sizeof(float2);
-  const void* kernel = (const void*)icp_small_batch_kernel<THREADS>;
-  OPE_TRY(dyn_smem(ctx, kernel, smem_bytes));
-  int per_sm = 0;
-  OPE_CUDA_TRY(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, THREADS, smem_bytes));
-  if ((size_t)per_sm * ctx->sm_count < (size_t)kIcpSmallMaxBlocks) return fail(ctx, OPE_ERR_CUDA, "icp_small_batch_kernel: one alignment's blocks cannot be co-resident");
-  cudaEventRecord(ctx->kev[0][0], ctx->stream);
-  icp_small_batch_kernel<THREADS><<<(unsigned)total_blocks, THREADS, smem_bytes, ctx->stream>>>(d_descs.p, d_map.p, bars.p + n_frames);
-  cudaEventRecord(ctx->kev[0][1], ctx->stream);
-  ctx->kev_valid[0] = true;
-  return check_launch(ctx, "icp_small_batch_kernel");
-}
-
-// Threads per block of the frame-spanning ICP launch: a block keeps its alignment's target (points + group boxes) in shared memory
-// next to 256 bytes of candidate slots per thread, so wider blocks share one target copy among more warps: 2 x 256 threads fit an
-// SM where 3 x 128 do (16 resident warps instead of 12 of this latency-bound kernel). OPE_ICP_BATCH_THREADS=128 selects the narrow form.
-int icp_small_batch_device(ope_ctx* ctx, const ope_icp_params& prm, const IcpBatchFrame* frames, int n_frames, ope_reg_result* d_results) {
-  const char* e = std::getenv("OPE_ICP_BATCH_THREADS");
-  const int t = e ? std::atoi(e) : 256;
-  if (t == 128) return icp_small_batch_launch<128>(ctx, prm, frames, n_frames, d_results);
-  return icp_small_batch_launch<256>(ctx, prm, frames, n_frames, d_results);
+  return icp_small_launch(ctx, descs.data(), n_frames);
 }
 
 }  // namespace ope

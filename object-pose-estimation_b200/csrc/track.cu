@@ -219,7 +219,7 @@ int tracker_step_batch(ope_ctx* ctx, ope_pose_tracker* const* trackers, ope_clou
       }
     }
   } release{ctx, steps};
-  const bool config_ok = icp_small_batch_applicable(P.icp, 1, 1) && P.icp.n_rejectors >= 0 && P.sacia.nr_samples >= 1 &&
+  const bool config_ok = icp_small_applicable(P.icp, 1, 1) && P.icp.n_rejectors >= 0 && P.sacia.nr_samples >= 1 &&
                          P.sacia.max_iterations >= 1 && P.sacia.k_correspondences >= 1 && P.normal_k <= 32;
   for (size_t i = 0; i < n; ++i) {
     Step& s = steps[i];

@@ -270,13 +270,22 @@ def _shooting_cases():
         "tgt4097": (cs[:1500], ct[:4097]),             # the smallest one that is not
         "src4096": (ct[:4096] + np.float32(0.3 * H), ct[:4000]),   # the largest source of the thread-per-query kernel
         "src4097": (ct[:4097] + np.float32(0.3 * H), ct[:4000]),
+        "nonfinite": (with_nonfinite(src)[0], with_nonfinite(tgt)[0]),   # NaN / inf rows in both clouds
+        "guess": (src, tgt),                                             # started from SHOOT_GUESS
     }
 
 
-@pytest.mark.parametrize("name", ["lattice", "crossing", "sphere", "offset-100m", "tgt3", "tgt4096", "tgt4097", "src4096", "src4097"])
+SHOOT_GUESS = np.eye(4, dtype=np.float32)
+SHOOT_GUESS[:3, :3] = _rot((2, -1, 1), 2.0)
+SHOOT_GUESS[:3, 3] = np.array([-0.3, 0.2, 0.25]) * H
+
+
+@pytest.mark.parametrize("name", ["lattice", "crossing", "sphere", "offset-100m", "tgt3", "tgt4096", "tgt4097", "src4096", "src4097",
+                                  "nonfinite", "guess"])
 def test_normal_shooting_every_path(ctx, orc, synth, cuda_lib, name, monkeypatch):
     T = cuda_lib.T
     src, tgt = _shooting_cases()[name]
+    guess = SHOOT_GUESS if name == "guess" else None
     sn, tn = orc.normals_knn(src, 12), orc.normals_knn(tgt, 12)
     cs, ct = ctx.upload(src, sn), ctx.upload(tgt, tn)
     for k in (1, 20, 32):
@@ -284,10 +293,10 @@ def test_normal_shooting_every_path(ctx, orc, synth, cuda_lib, name, monkeypatch
             for variant in (T.ICP_VARIANT_MOD, T.ICP_VARIANT_MODCORR):
                 prm = dict(max_iterations=8, transformation_epsilon=1e-10, euclidean_fitness_epsilon=1e-12, estimator=T.EST_NORMAL_SHOOTING,
                            k_search=k, rejectors=_chain(T, chain), with_normals=1, variant=variant)
-                o, oc = orc.icp(src, tgt, orc.icp_params(**prm), src_normals=sn, tgt_normals=tn, want_corr=True)
+                o, oc = orc.icp(src, tgt, orc.icp_params(**prm), guess=guess, src_normals=sn, tgt_normals=tn, want_corr=True)
                 for env in SHOOT_PATHS:
                     _set_env(monkeypatch, env)
-                    g, gc = ctx.icp(cs, ct, cuda_lib.icp_params(**prm), want_corr=True)
+                    g, gc = ctx.icp(cs, ct, cuda_lib.icp_params(**prm), guess=guess, want_corr=True)
                     _same_as_oracle(synth, T, g, gc, o, oc, (name, k, chain, variant, env))
                 _set_env(monkeypatch, {})
 

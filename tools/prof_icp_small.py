@@ -1,6 +1,7 @@
 import os, sys
 os.environ["OPE_ICP_SMALL"]="1"; os.environ["OPE_PROFILE"]="1"
-sys.path.insert(0,'/root/repo'); sys.path.insert(0,'/root/repo/oracle')
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, 'oracle'))
 import numpy as np, ope_pkg; ope_pkg.load()
 from ope_b200 import cuda_lib, synth
 import ctypes
